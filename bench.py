@@ -9,6 +9,10 @@ One "step" = one full render of the 800x800 frame at 1000 spp (961 effective, de
 8x8 pixel tiles, rank r renders tiles with tile_index % N == r, and one NCCL reduce(sum) of the
 float framebuffer reassembles it on rank 0: total work is fixed, so scaling is "strong".
 
+--dump-outputs DIR writes the image the last timed step computed to DIR/image.npy, (H, W, 3) after the timed region: the float
+framebuffer (on rank 0 the reduced frame), the RgbImage bytes with --single-process, the oracle's partial frame with --impl reference.
+Scene and render seeds are fixed, so two builds run with the same arguments can be compared image for image.
+
 Keys beyond the base contract: `roofline` (dominant kernel = extend), `cpu_baseline` (the oracle on
 this box's host cores, bounded sample), `e2e` (flatten + upload + render + read-back + 8-bit encode
 per step, i.e. what Camera::render does), `clocks`, `gpu_launches`.
@@ -41,6 +45,14 @@ EXTEND_BYTES_PER_SEGMENT = 64 + 16 + 16 + 1
 # SURVEY.md §8(d), whole step: 2 x 64 (path state read + written once) + 2 x 16 (hit record written by extend, read by shade)
 # per segment, + 12 per path for the framebuffer add
 STEP_BYTES_PER_SEGMENT, STEP_BYTES_PER_PATH = 160, 12
+
+
+def dump_outputs(out_dir, image):
+    """--dump-outputs: the image the last timed step computed, as out_dir/image.npy (float32, or float64 when it was rendered so)."""
+    import numpy as np
+    image = np.asarray(image)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "image.npy"), image if image.dtype == np.float64 else image.astype(np.float32))
 
 
 def partition_for_rank(rank, world):
@@ -158,9 +170,11 @@ def run_reference(args, rank):
     t0 = time.perf_counter()
     paths = 0
     for k in range(args.steps):
-        _, st = osc.render(seed=RENDER_SEED, sample_begin=(k * strata) % 960, sample_end=(k * strata) % 960 + strata)
+        img, st = osc.render(seed=RENDER_SEED, sample_begin=(k * strata) % 960, sample_end=(k * strata) % 960 + strata)
         paths += st.paths
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, img)
     v = paths / dt
     sample = f"{strata} strata of 961 per step over the full 800x800 frame ({paths // max(1, args.steps)} paths/step)"
     print(json.dumps({
@@ -204,6 +218,8 @@ def run_single_process(args):
         launches += st.kernel_launches
     dt = time.perf_counter() - t0
     sampler.stop_flag = True
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, img)
     for sc in scenes:
         sc.close()
     t0 = time.perf_counter()
@@ -246,7 +262,10 @@ def main():
     ap.add_argument("--partition", default="tiles", choices=["tiles", "strata"],
                     help="how N > 1 ranks share the frame: interleaved 8x8 pixel tiles (default) or contiguous stratum ranges of every pixel")
     ap.add_argument("--rank-times", action="store_true", help="print every rank's device time per step to stderr (load-balance diagnosis)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the image the last timed step computed to DIR/image.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -322,6 +341,8 @@ def main():
     e1.record()
     barrier()
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fb.cpu().numpy())
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     extra = torch.tensor([segs, launches], dtype=torch.float64, device=dev)
     if world > 1:

@@ -22,6 +22,18 @@ def final_reduced_scene(rt, width=96, spp=4, depth=12):
     return hs
 
 
+def table_digests(hs):
+    """{table: [record count, SHA-256 of its bytes]} for the flat tables of a host scene that do not depend on image
+    resolution (the texel pool does)."""
+    import ctypes as C
+    import hashlib
+    d = hs.desc.contents
+    return {field: [n, hashlib.sha256(C.string_at(getattr(d, field), n * size)).hexdigest()]
+            for field, n, size in (("objects", d.n_objects, 72), ("children", d.n_children, 4), ("planars", d.n_planars, 144),
+                                   ("materials", d.n_materials, 176), ("remaps", d.n_remaps, 200), ("transforms", d.n_transforms, 80),
+                                   ("textures", d.n_textures, 80))}
+
+
 def random_graph_scene(rt, seed, n_prims=60, with_transforms=True, with_media=False, with_lights=True, width=24, spp=4, depth=6):
     """A random object graph mixing every container the reference has."""
     rng = np.random.default_rng(seed)

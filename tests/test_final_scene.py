@@ -4,15 +4,16 @@ image-backed equirect environment (shapes/environment.rs:14-24 over ImageTexture
 CPU tests cover the asset pack, the loader output and the oracle; `-m gpu` tests are the parity tests proper
 (ids and t bit-exact, same-seed images, the environment lookup against an independent numpy restatement).
 """
+import json
 import os
 
 import numpy as np
 import pytest
 
-from scenes_util import _pkg_module, compare_hits, final_reduced_scene
+from scenes_util import _pkg_module, compare_hits, final_reduced_scene, table_digests
 
 KIND = dict(sphere=1, quad=2, tri=3, list=4, bvh=5, transform=6, medium=7)
-REF_ASSETS = "/root/reference/assets"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def image_close(img, ref, frac_bad=5e-3, rel=1e-6):
@@ -59,23 +60,13 @@ def test_final_scene_structure(rt):
     assert (cam.image_width, cam.image_height) == (96, 54) and cam.background_tex != rt.RT_NONE
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ASSETS), reason="reference assets only exist in the build container")
 def test_pack_equals_reference_files(rt):
-    """The committed pack is the parse of the reference's files: geometry, remap frames and material records of the scene
-    built from the pack and from /root/reference/assets are byte-identical (only the texel pools differ: reduced images)."""
-    import ctypes as C
-    scenes, objload = _pkg_module(rt, "scenes"), _pkg_module(rt, "objload")
-    a = final_reduced_scene(rt)
-    b, missing = scenes.obj_scene(rt, REF_ASSETS, width=96, spp=4, depth=12)
-    assert missing == ["初音未来.obj", "卒.obj"]
-    da, db = a.desc.contents, b.desc.contents
-    assert np.array_equal(a.objects(), b.objects()) and np.array_equal(a.children(), b.children())
-    for field, n, size in (("planars", da.n_planars, 144), ("materials", da.n_materials, 176), ("remaps", da.n_remaps, 200),
-                           ("transforms", da.n_transforms, 80), ("textures", da.n_textures, 80)):
-        ba = C.string_at(getattr(da, field), n * size)
-        bb = C.string_at(getattr(db, field), n * size)
-        assert ba == bb, field
-    assert db.n_texels > da.n_texels
+    """The committed pack is the parse of the reference's files: object graph, geometry, remap frames and material records
+    of the scene built from the pack are byte-identical to those of obj_scene() on the reference's assets/ directory, stored
+    as digests in final_assets_tables.json by make_final_pack.py (only the texel pools differ: reduced images)."""
+    with open(os.path.join(GOLDEN, "final_assets_tables.json")) as f:
+        want = json.load(f)
+    assert table_digests(final_reduced_scene(rt)) == want
 
 
 def test_environment_lookup_oracle(rt, orc):
