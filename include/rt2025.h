@@ -285,7 +285,9 @@ typedef struct rt_stats {
     double ms_raygen, ms_extend, ms_shade, ms_other; /* filled when RT_OPT_STAGE_TIMES is set */
     uint64_t iterations;   /* wavefront iterations                                          */
     uint64_t reserved[4];  /* reserved[0]: of `segments`, those evaluated inside the random-walk kernel of an optically
-                              thick ConstantMedium (they never passed through extend)               */
+                              thick ConstantMedium (they never passed through extend);
+                              reserved[1]: of reserved[0], those evaluated by its lean variant (scenes whose walk needs
+                              no Transform, texture lookup or light-tree code)                      */
 } rt_stats;
 
 /* Closest surface hit for a batch of rays over `world` (media excluded: they are stochastic,

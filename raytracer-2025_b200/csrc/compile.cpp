@@ -1089,7 +1089,53 @@ struct Compiler {
             if (overlapping_leaves(b, plain ? ball : nullptr, out.world_root, med.entry, n)) med.n_entry = n;
             if (timer.on) fprintf(stderr, "[rt2025 compile] medium %zu is optically thick: %d entry leaves\n", m, (int)med.n_entry);
         }
+        walk_lean();
+        if (timer.on) fprintf(stderr, "[rt2025 compile] random walk: %s\n", out.walk_lean.empty() ? "generic" : (out.walk_lean[0].shell != RT_NONE ? "lean, shell" : "lean"));
         return RT_OK;
+    }
+
+    // scene_types.h, WalkLean: the record of the lean random walk when the scene qualifies, otherwise nothing
+    void walk_lean() {
+        out.walk_lean.clear();
+        const size_t n_media = out.media.size(), n_lights = out.lights.size();
+        if (n_media > WALK_LEAN_MEDIA || n_lights > WALK_LEAN_LIGHTS) return;
+        WalkLean L;
+        std::memset(&L, 0, sizeof(L));
+        L.n_media = (uint32_t)n_media, L.n_lights = (uint32_t)n_lights, L.thick = RT_NONE, L.shell = RT_NONE;
+        for (size_t m = 0; m < n_media; m++) {
+            const Medium& med = out.media[m];
+            if (med.single_sphere == RT_NONE || med.xform != RT_NONE || out.meta[med.single_sphere].xform != RT_NONE) return;
+            if (med.flags & MEDIUM_THICK) {
+                if (L.thick != RT_NONE || med.n_entry == MEDIUM_NO_ENTRIES) return;
+                L.thick = (uint32_t)m;
+            }
+            std::memcpy(L.sphere[m], out.geom[med.single_sphere].d, 7 * sizeof(double));
+            L.neg_inv_density[m] = med.neg_inv_density;
+            L.rank[m] = med.rank, L.medium_index[m] = med.medium_index;
+        }
+        if (L.thick == RT_NONE) return;
+        const Medium& thick = out.media[L.thick];
+        const Material& iso = out.materials[thick.material];
+        if (iso.kind != RT_MAT_ISOTROPIC || iso.tex >= out.textures.size() || out.textures[iso.tex].kind != RT_TEX_SOLID) return;
+        for (int k = 0; k < 3; k++) L.axp[k] = (1.0 / (4.0 * 3.14159265358979323846264338327950288)) * out.textures[iso.tex].color[k];  // D3 / double
+        for (size_t i = 0; i < n_lights; i++) {  // flat: every leaf weighs 1/n (rt_scene_create's test)
+            const Light& l = out.lights[i];
+            if (l.xform != RT_NONE || l.weight != 1.0 / (double)n_lights) return;
+            L.lights[i] = l;
+        }
+        for (uint32_t e = 0; e < thick.n_entry; e++) {
+            const uint32_t first = (thick.entry[e] & ~LEAF_FLAG) >> 3, count = (thick.entry[e] & 7u) + 1;
+            for (uint32_t pi = first; pi < first + count; pi++) {
+                const PrimMeta& pm = out.meta[pi];
+                if (L.n_prims == WALK_LEAN_PRIMS || pm.xform != RT_NONE) return;
+                const uint32_t k = L.n_prims++;
+                L.prim[k] = out.geom[pi];
+                L.prim_kind[k] = pm.kind_mat >> 30, L.prim_rank[k] = pm.rank;
+                // bit-identical (memcmp, not ==: -0.0 and NaN must not pass) centre, centre_vec and radius
+                if (L.shell == RT_NONE && L.prim_kind[k] == PRIM_SPHERE && std::memcmp(out.geom[pi].d, L.sphere[L.thick], 7 * sizeof(double)) == 0) L.shell = k;
+            }
+        }
+        out.walk_lean.push_back(L);
     }
 };
 

@@ -53,6 +53,7 @@ struct CompiledScene {
     std::vector<Light> lights;
     std::vector<Remap> remaps;
     std::vector<uint32_t> ranks;  // per desc object, RT_NONE for containers
+    std::vector<WalkLean> walk_lean;  // one record when the scene qualifies for the lean random walk, else empty
     uint32_t world_root = INVALID_REF;
     uint32_t bvh_depth = 0;        // world group (binary tree)
     uint32_t media_bvh_depth = 0;  // deepest ConstantMedium boundary group

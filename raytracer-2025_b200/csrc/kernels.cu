@@ -244,6 +244,34 @@ struct MediumDraws {
 
 constexpr uint32_t MEDIUM_INCUMBENT = 0x80000000u;  // `prim` of a traversal whose incumbent is a medium scatter point: flag | medium index
 
+// ConstantMedium::hit after the two boundary hits t1 < t2 (volume.rs:46-73) on the caller's interval [1e-8, inf): true and the
+// scatter distance when the path scatters inside.  lr: the ray in the medium's space.
+__device__ __forceinline__ bool medium_free_flight(double t1, double t2, const RayD& lr, double neg_inv_density, double xi, double& tm) {
+    if (t1 < 1e-8) t1 = 1e-8;  // clamp to the caller's interval [1e-8, inf)
+    if (t1 >= t2) return false;
+    if (t1 < 0.0) t1 = 0.0;
+    const double ray_length = length(lr.d);
+    const double distance_inside_boundary = (t2 - t1) * ray_length;
+    // binary32 screen: when even a pessimistic free-flight estimate clears the segment inside the boundary by a wide
+    // margin the path does not scatter here and the binary64 ln is not needed (the exact comparison below is unchanged)
+    const float hf = (float)neg_inv_density * logf((float)xi);
+    const float hf_err = 4e-7f * fabsf((float)neg_inv_density);
+    if (hf > (float)distance_inside_boundary * 1.001f + hf_err) return false;
+    const double hit_distance = neg_inv_density * log(xi);
+    if (hit_distance > distance_inside_boundary) return false;
+    tm = t1 + hit_distance / ray_length;
+    return true;
+}
+
+// binary32 screen of a medium against a known hit at t: the scatter point lies at t1 + dist/len with t1 >= 0, so a free flight
+// that clearly overshoots the known hit cannot win whatever the boundary does
+__device__ __forceinline__ bool free_flight_overshoots(double neg_inv_density, double xi, double t, const D3& ld) {
+    const float hf = (float)neg_inv_density * logf((float)xi);
+    const float hf_err = 4e-7f * fabsf((float)neg_inv_density);
+    const float len_f = sqrtf((float)ld.x * (float)ld.x + (float)ld.y * (float)ld.y + (float)ld.z * (float)ld.z);
+    return hf > (float)t * len_f * 1.001f + hf_err;
+}
+
 // ConstantMedium::hit (volume.rs:37-73) for a medium whose boundary is a single Sphere, on the caller's interval
 // [1e-8, inf): true and the scatter distance when the path scatters inside.  XF: the medium or its sphere may sit
 // under a Transform.
@@ -259,20 +287,7 @@ __device__ __forceinline__ bool sample_sphere_medium(const SceneView& sv, const 
     double t1, t2;
     if (COUNT) cnt->prims += 2;
     if (!sphere_entry_exit(sv.geom[med.single_sphere].d, br, t1, t2)) return false;
-    if (t1 < 1e-8) t1 = 1e-8;  // clamp to the caller's interval [1e-8, inf)
-    if (t1 >= t2) return false;
-    if (t1 < 0.0) t1 = 0.0;
-    const double ray_length = length(lr.d);
-    const double distance_inside_boundary = (t2 - t1) * ray_length;
-    // binary32 screen: when even a pessimistic free-flight estimate clears the segment inside the boundary by a wide
-    // margin the path does not scatter here and the binary64 ln is not needed (the exact comparison below is unchanged)
-    const float hf = (float)med.neg_inv_density * logf((float)xi);
-    const float hf_err = 4e-7f * fabsf((float)med.neg_inv_density);
-    if (hf > (float)distance_inside_boundary * 1.001f + hf_err) return false;
-    const double hit_distance = med.neg_inv_density * log(xi);
-    if (hit_distance > distance_inside_boundary) return false;
-    tm = t1 + hit_distance / ray_length;
-    return true;
+    return medium_free_flight(t1, t2, lr, med.neg_inv_density, xi, tm);
 }
 
 // MEDIA: 0 = the ray load does not look at media (none, or they are sampled by k_media after extend);
@@ -390,14 +405,8 @@ __device__ __forceinline__ bool sample_media(const SceneView& sv, uint64_t seed,
             double tm;
             RayD lr = r;
             if (XF && med.xform != RT_NONE) lr = ray_to_local(sv, med.xform, r);
-            // binary32 screen: the scatter point lies at t1 + dist/len with t1 >= 0, so a free flight that clearly
-            // overshoots the known hit cannot win whatever the boundary does: skip the boundary test
-            if (RT_MEDIA_EARLY_SCREEN && kind != HIT_MISS) {
-                const float hf = (float)med.neg_inv_density * logf((float)xi);
-                const float hf_err = 4e-7f * fabsf((float)med.neg_inv_density);
-                const float len_f = sqrtf((float)lr.d.x * (float)lr.d.x + (float)lr.d.y * (float)lr.d.y + (float)lr.d.z * (float)lr.d.z);
-                if (hf > (float)t * len_f * 1.001f + hf_err) continue;
-            }
+            // skip the boundary test of a medium that cannot beat the known hit
+            if (RT_MEDIA_EARLY_SCREEN && kind != HIT_MISS && free_flight_overshoots(med.neg_inv_density, xi, t, lr.d)) continue;
             if (med.single_sphere != RT_NONE) {
                 if (!sample_sphere_medium<COUNT, XF>(sv, med, r, xi, tm, cntp)) continue;
             } else if (GENERIC) {
@@ -924,12 +933,117 @@ constexpr int WALK_BLOCK = RT_WALK_BLOCK;
 #ifndef RT_WALK_MIN_BLOCKS
 #define RT_WALK_MIN_BLOCKS 4
 #endif
+#ifndef RT_WALK_LEAN_MIN_BLOCKS
+#define RT_WALK_LEAN_MIN_BLOCKS 4
+#endif
+
+// One segment of the lean walk (scene_types.h, WalkLean) from a scatter point at t inside the thick medium: the SC_ISOTROPIC part
+// of shade_one with the same operations in the same order, then the look-ahead of k_walk - the thick medium, the thin ones when it
+// scattered, the entry primitives - against the staged constants.  Returns whether the path goes on (nr, nbeta); `stay`: the
+// next scatter point (at tn) is again inside the thick medium and nothing beats it.
+__device__ __forceinline__ bool walk_lean_segment(const SceneView& sv, const WalkLean& L, const RenderParams& P, const WavefrontState& W, const RayD& r,
+                                                  D3 beta, uint32_t pixel, uint32_t sidx, uint32_t segment, double t, uint32_t max_steps,
+                                                  uint32_t& steps, RayD& nr, D3& nbeta, double& tn, bool& stay) {
+    stay = false;
+    nr.o = r.o + t * r.d;  // volume.rs:66-72 (h.p); the normal, uv and texture lookup are unused by a solid Isotropic
+    nr.time = r.time;
+    const Rand2 pick = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_MIXTURE);
+    const Rand2 dx = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_DIRECTION);
+    const uint32_t n_lights = L.n_lights;
+    D3 gen = D3{0.0, 0.0, 0.0};
+    bool panic = false;  // shade_one's stop == 1 (None cannot occur here)
+    if (n_lights > 0 && !(pick.a < 0.5)) {  // lights_random over the flat list
+        uint32_t leaf = n_lights - 1;
+        for (uint32_t i = 0; i < n_lights; i++)
+            if (pick.b < L.lights[i].cdf) {
+                leaf = i;
+                break;
+            }
+        panic = !light_leaf_random(L.lights[leaf], nr.o, dx.a, dx.b, gen);
+    } else {
+        gen = random_unit_vector(dx.a, dx.b);
+    }
+    const double value0 = 1.0 / (4.0 * RT_PI);
+    double pdf_val = value0;
+    if (!panic && n_lights > 0) {  // lights_pdf_value of a flat list: sum / len (x / 1.0 == x: no division for one light)
+        double sum = 0.0;
+        for (uint32_t i = 0; i < n_lights; i++) sum += light_leaf_pdf<true>(sv, L.lights[i], nr.o, gen);
+        const double value1 = n_lights == 1 ? sum : sum / (double)n_lights;
+        if (isnan(value1) || (value0 == 0.0 && value1 == 0.0))
+            panic = true;
+        else
+            pdf_val = value0 * 0.5 + value1 * 0.5;
+    }
+    if (panic || pdf_val == 0.0) {
+        atomicAdd(&W.counters->errors, 1ull);
+        return false;
+    }
+    nr.d = gen;
+    nbeta = beta * (ld3(L.axp) / pdf_val);
+    if (segment + 1 >= P.cam.max_depth || (nbeta.x == 0.0 && nbeta.y == 0.0 && nbeta.z == 0.0)) return false;
+
+    // world.hit of the next segment, as sample_media<.., 1> then <.., 2> and leaf_beats_scatter
+    const uint32_t seg1 = segment + 1u, thick = L.thick;
+    MediumDraws draws;
+    double near_root, far_root;  // the thick boundary's roots: the shell's Sphere::hit on this ray has the same
+    {
+        const double* s = L.sphere[thick];
+        double t1, t2;
+        const double xi = draws.get(P.seed, pixel, sidx, seg1, L.medium_index[thick]);
+        const bool inside = sphere_entry_exit_at(ld3(s), ld3(s + 3), s[6], nr, t1, t2, near_root, far_root);
+        if (!inside || !medium_free_flight(t1, t2, nr, L.neg_inv_density[thick], xi, tn)) return true;
+    }
+    if (!(++steps < max_steps)) return true;
+    const uint32_t med_rank = L.rank[thick];
+    for (uint32_t m = 0; m < L.n_media; m++) {
+        if (m == thick) continue;
+        const double xi = draws.get(P.seed, pixel, sidx, seg1, L.medium_index[m]);
+        if (RT_MEDIA_EARLY_SCREEN && free_flight_overshoots(L.neg_inv_density[m], xi, tn, nr.d)) continue;
+        const double* s = L.sphere[m];
+        double t1, t2, nroot, froot, tm;
+        if (!sphere_entry_exit_at(ld3(s), ld3(s + 3), s[6], nr, t1, t2, nroot, froot) || !medium_free_flight(t1, t2, nr, L.neg_inv_density[m], xi, tm)) continue;
+        if (tm < tn || (tm == tn && L.rank[m] < med_rank)) return true;  // a thin medium wins: the walk ends whatever else does
+    }
+    bool beaten = false;
+    for (uint32_t i = 0; i < L.n_prims && !beaten; i++) {
+        const double* g = L.prim[i].d;
+        double th;
+        bool hit;
+        if (i == L.shell) {  // sphere_hit's choice: the near root if it lies in [1e-8, tn], else the far one
+            th = near_root;
+            hit = contains(1e-8, tn, th);
+            if (!hit) {
+                th = far_root;
+                hit = contains(1e-8, tn, th);
+            }
+        } else if (L.prim_kind[i] == PRIM_SPHERE) {
+            hit = sphere_hit_at(ld3(g), ld3(g + 3), g[6], nr, 1e-8, tn, th);
+        } else {
+            Planar pl;
+            load_planar_plain(g, pl);
+            double a, b;
+            hit = planar_hit_loaded(pl, L.prim_kind[i] == PRIM_TRIANGLE, nr, 1e-8, tn, th, a, b);
+        }
+        beaten = hit && (th < tn || L.prim_rank[i] < med_rank);
+    }
+    stay = !beaten;
+    return true;
+}
+
 // ENTRIES: every thick medium of the scene has its entry leaves and there is only one of them, so the traversal from the world
 // root (another medium's scatter point, more leaves than slots) is never needed and is compiled out.
-template <bool XF, bool ENTRIES>
-__global__ void __launch_bounds__(WALK_BLOCK, RT_WALK_MIN_BLOCKS) k_walk(SceneView sv, RenderParams P, WavefrontState W) {
-    extern __shared__ float4 s_mem[];  // traversal stacks (global-memory nodes only)
+// LEAN: the scene's walk constants are staged (SceneView::walk_lean, implies ENTRIES and !XF): walk_lean_segment.
+template <bool XF, bool ENTRIES, bool LEAN = false>
+__global__ void __launch_bounds__(WALK_BLOCK, LEAN ? RT_WALK_LEAN_MIN_BLOCKS : RT_WALK_MIN_BLOCKS) k_walk(SceneView sv, RenderParams P, WavefrontState W) {
+    extern __shared__ float4 s_mem[];  // traversal stacks (global-memory nodes only) | LEAN: the WalkLean record
     uint32_t* stack = reinterpret_cast<uint32_t*>(s_mem) + threadIdx.x;
+    const WalkLean& L = *reinterpret_cast<const WalkLean*>(s_mem);
+    if (LEAN) {
+        unsigned long long* dst = reinterpret_cast<unsigned long long*>(s_mem);
+        const unsigned long long* src = reinterpret_cast<const unsigned long long*>(sv.walk_lean);
+        for (uint32_t k = threadIdx.x; k < sizeof(WalkLean) / 8; k += WALK_BLOCK) dst[k] = src[k];
+        __syncthreads();
+    }
     const uint32_t n = W.counters->n_shade[SC_WALK];
     const RayRec* __restrict__ rays = W.ray_q[W.parity];
     const BetaRec* __restrict__ betas = W.beta_q[W.parity];
@@ -994,16 +1108,19 @@ __global__ void __launch_bounds__(WALK_BLOCK, RT_WALK_MIN_BLOCKS) k_walk(SceneVi
         if (have) {
             RayD nr;
             D3 nbeta;
-            if (!shade_one<SC_ISOTROPIC>(sv, P, W, r, beta, pixel, sidx, segment, t, medium, HIT_MEDIUM, nr, nbeta)) {
-                have = false;
-            } else {
+            double tn = INFINITY;
+            uint32_t pn = medium;
+            bool alive, stay = false;
+            if constexpr (LEAN) {
+                alive = walk_lean_segment(sv, L, P, W, r, beta, pixel, sidx, segment, t, max_steps, steps, nr, nbeta, tn, stay);
+            } else if ((alive = shade_one<SC_ISOTROPIC>(sv, P, W, r, beta, pixel, sidx, segment, t, medium, HIT_MEDIUM, nr, nbeta))) {
                 // world.hit of the next segment: the thick media first (the one the path is in leads); when none of them scatters
                 // the walk is over whatever the thin ones do, otherwise they are screened by the scatter point found
-                double tn = INFINITY;
-                uint32_t pn = 0xFFFFFFFFu, kn = HIT_MISS;
+                uint32_t kn = HIT_MISS;
+                pn = 0xFFFFFFFFu;
                 MediumDraws draws;
                 sample_media<false, false, XF, 1>(sv, P.seed, nr, pixel, sidx, segment + 1u, tn, pn, kn, s_mem, stack, WALK_BLOCK, &cnt, medium, draws);
-                bool stay = kn == HIT_MEDIUM && ++steps < max_steps;
+                stay = kn == HIT_MEDIUM && ++steps < max_steps;
                 if (stay) {
                     sample_media<false, false, XF, 2>(sv, P.seed, nr, pixel, sidx, segment + 1u, tn, pn, kn, s_mem, stack, WALK_BLOCK, &cnt, 0u, draws);
                     stay = (sv.media[pn].flags & MEDIUM_THICK) != 0u;
@@ -1020,26 +1137,33 @@ __global__ void __launch_bounds__(WALK_BLOCK, RT_WALK_MIN_BLOCKS) k_walk(SceneVi
                         stay = !(ts < tn || sv.meta[ps].rank < med_rank);
                     }
                 }
-                if (stay) {
-                    r = nr, beta = nbeta, segment++, t = tn, medium = pn;
-                    walked++;
-                } else {
-                    const uint32_t npos = queue_reserve(&W.counters->n_extend[W.parity ^ 1u], 0);
-                    store_ray(W.ray_q[W.parity ^ 1u] + npos, nr, pack_ids(pixel, sidx, segment + 1u));
-                    store_beta(W.beta_q[W.parity ^ 1u] + npos, nbeta);
-                    have = false;
-                }
+            }
+            if (!alive) {
+                have = false;
+            } else if (stay) {
+                r = nr, beta = nbeta, segment++, t = tn, medium = pn;
+                walked++;
+            } else {
+                const uint32_t npos = queue_reserve(&W.counters->n_extend[W.parity ^ 1u], 0);
+                store_ray(W.ray_q[W.parity ^ 1u] + npos, nr, pack_ids(pixel, sidx, segment + 1u));
+                store_beta(W.beta_q[W.parity ^ 1u] + npos, nbeta);
+                have = false;
             }
         }
     }
     if (walked) {
         atomicAdd(&W.counters->segments, walked);
         atomicAdd(&W.counters->walk_segments, walked);
+        if (LEAN) atomicAdd(&W.counters->walk_lean_segments, walked);
     }
 }
 static void launch_walk(const SceneView& sv, const RenderParams& P, const WavefrontState& W, int grid, cudaStream_t s) {
     SceneView wv = sv;
     wv.n_cached_nodes = 0;  // the non-persistent closest_hit() reads the binary tree from global memory
+    if (sv.walk_lean) {  // no traversal: the dynamic shared memory holds the staged constants
+        k_walk<false, true, true><<<grid / RT_WALK_MIN_BLOCKS * RT_WALK_LEAN_MIN_BLOCKS, WALK_BLOCK, sizeof(WalkLean), s>>>(wv, P, W);
+        return;
+    }
     const size_t smem = (size_t)std::max(sv.tail_stack_entries, 4u) * WALK_BLOCK * sizeof(uint32_t);
     auto k = sv.media_xform ? (sv.walk_entries_only ? k_walk<true, true> : k_walk<true, false>) : (sv.walk_entries_only ? k_walk<false, true> : k_walk<false, false>);
     k<<<grid, WALK_BLOCK, smem, s>>>(wv, P, W);

@@ -107,6 +107,7 @@ struct Counters {
     uint32_t gen_done, walk_cursor;  // arrival counter of k_generate's CTAs; next entry of the SC_WALK queue to be claimed (k_walk)
     unsigned long long next_path, segments, iterations, errors, node_visits, prim_tests;
     unsigned long long walk_segments;  // of `segments`: evaluated inside k_walk (they never went through the streams)
+    unsigned long long walk_lean_segments;  // of `walk_segments`: evaluated by the lean variant of k_walk (SceneView::walk_lean)
 };
 
 struct WavefrontState {

@@ -132,6 +132,28 @@ struct Light {
     double weight, cdf, area;
 };
 
+// The constants of the lean random walk (k_walk<.., LEAN>), gathered by the scene compiler for a scene whose walk needs none of
+// the generic machinery: one MEDIUM_THICK medium with its entry leaves, every medium bounded by one untransformed Sphere, an
+// Isotropic over a solid texture in the thick one, a flat list of at most WALK_LEAN_LIGHTS untransformed lights and at most
+// WALK_LEAN_PRIMS untransformed primitives in the entry leaves.  The kernel copies the record to shared memory once per CTA, so a
+// segment makes no dependent loads through media[], materials[], textures[], meta[] or lights[].
+constexpr uint32_t WALK_LEAN_MEDIA = 4, WALK_LEAN_LIGHTS = 4, WALK_LEAN_PRIMS = 8;
+struct WalkLean {
+    Light lights[WALK_LEAN_LIGHTS];      // the flat light list, as in lights[]
+    PrimGeom prim[WALK_LEAN_PRIMS];      // the primitives of the thick medium's entry leaves, in leaf order
+    double sphere[WALK_LEAN_MEDIA][8];   // boundary Sphere of every medium: centre(3) centre_vec(3) radius
+    double neg_inv_density[WALK_LEAN_MEDIA];
+    double axp[3];                       // albedo / (4 pi) of the thick medium's Isotropic (shade_one's expression)
+    double pad0;
+    uint32_t rank[WALK_LEAN_MEDIA], medium_index[WALK_LEAN_MEDIA];
+    uint32_t prim_kind[WALK_LEAN_PRIMS], prim_rank[WALK_LEAN_PRIMS];
+    uint32_t n_media, thick, n_lights, n_prims;
+    // entry primitive whose geometry is bit-identical to the thick boundary sphere (the glass shell around book2's subsurface
+    // ball), or RT_NONE: its hit on a segment is decided from the roots the boundary test has already computed
+    uint32_t shell;
+    uint32_t pad1[3];
+};
+
 // shade work classes used to bin hits (extend -> shade queues)
 enum ShadeClass : uint32_t {
     SC_MISS = 0,      // background lookup, path ends
@@ -177,6 +199,7 @@ struct SceneView {
     uint32_t n_xforms;           // Transforms in the scene (0: the traversal needs no local-space rays)
     uint32_t walk_entries_only;  // exactly one MEDIUM_THICK medium and it has its entry leaves: k_walk never traverses from the world root
     uint32_t fifo_slots;      // prepared-ray FIFO slots per warp of the persistent traversal: 32 or 64; 0 = no FIFO (traverse.cuh)
+    const WalkLean* walk_lean;  // the scene qualifies for the lean random walk (one record), or nullptr: the generic k_walk
 };
 
 }  // namespace rt

@@ -195,8 +195,10 @@ __device__ inline bool remap_record(const SceneView& sv, const Remap& rm, HitInf
 }
 
 // ---- lights: Hittables::pdf_value / random over the flattened leaves (hits.rs:52-75) -----------
+// STAGED: `l` is an untransformed light copied out of global memory (k_walk's lean variant)
+template <bool STAGED = false>
 __device__ inline double light_leaf_pdf(const SceneView& sv, const Light& l, D3 origin, D3 direction) {
-    if (l.xform != RT_NONE) {  // Transform::pdf_value, shapes.rs:117-123, outermost Transform first
+    if (!STAGED && l.xform != RT_NONE) {  // Transform::pdf_value, shapes.rs:117-123, outermost Transform first
         const Xform* x = sv.xforms + l.xform;
         for (uint32_t k = 0; k < x->n_chain; k++) {
             XformParams p = load_xform(sv.xforms + x->chain[k]);
@@ -211,7 +213,7 @@ __device__ inline double light_leaf_pdf(const SceneView& sv, const Light& l, D3 
     if (l.kind == PRIM_SPHERE) {  // sphere.rs:114-132
         double t;
         // own hit test on [1e-8, inf); the light record lives in global memory like any primitive
-        if (!sphere_hit(g, r, 1e-8, INFINITY, t)) return 0.0;
+        if (!(STAGED ? sphere_hit_at(ld3(g), ld3(g + 3), g[6], r, 1e-8, INFINITY, t) : sphere_hit(g, r, 1e-8, INFINITY, t))) return 0.0;
         D3 center = ld3(g);
         double radius = g[6];
         double dist_squared = length_squared((center + 0.0 * ld3(g + 3)) - origin);
@@ -222,7 +224,10 @@ __device__ inline double light_leaf_pdf(const SceneView& sv, const Light& l, D3 
     }
     // quad.rs:108-120, triangle.rs:104-113
     Planar pl;
-    load_planar(g, pl);
+    if (STAGED)
+        load_planar_plain(g, pl);
+    else
+        load_planar(g, pl);
     double t, a, b2;
     if (!planar_hit_loaded(pl, l.kind == PRIM_TRIANGLE, r, 1e-8, INFINITY, t, a, b2)) return 0.0;
     double distance_squared = t * t * length_squared(direction);

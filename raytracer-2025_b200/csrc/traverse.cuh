@@ -163,12 +163,7 @@ __device__ __forceinline__ void ldg256(const void* p, double2& a, double2& b) {
 }
 
 // Sphere::hit, sphere.rs:77-108 (geometry only)
-__device__ __forceinline__ bool sphere_hit(const double* __restrict__ g, const RayD& r, double tmin, double tmax, double& t_out) {
-    double2 a0, a1, a2, a3;
-    ldg256(g, a0, a1);
-    ldg256(g + 4, a2, a3);
-    D3 center = D3{a0.x, a0.y, a1.x}, cvec = D3{a1.y, a2.x, a2.y};
-    double radius = a3.x;
+__device__ __forceinline__ bool sphere_hit_at(D3 center, D3 cvec, double radius, const RayD& r, double tmin, double tmax, double& t_out) {
     D3 current_center = center + r.time * cvec;
     D3 oc = current_center - r.o;
     double a = length_squared(r.d);
@@ -185,6 +180,12 @@ __device__ __forceinline__ bool sphere_hit(const double* __restrict__ g, const R
     t_out = root;
     return true;
 }
+__device__ __forceinline__ bool sphere_hit(const double* __restrict__ g, const RayD& r, double tmin, double tmax, double& t_out) {
+    double2 a0, a1, a2, a3;
+    ldg256(g, a0, a1);
+    ldg256(g + 4, a2, a3);
+    return sphere_hit_at(D3{a0.x, a0.y, a1.x}, D3{a1.y, a2.x, a2.y}, a3.x, r, tmin, tmax, t_out);
+}
 
 struct Planar {
     D3 q, u, v, n, w;
@@ -200,6 +201,12 @@ __device__ __forceinline__ void load_planar(const double* __restrict__ g, Planar
     p.n = D3{a4.y, a5.x, a5.y};
     p.D = a6.x;
     p.w = D3{a6.y, a7.x, a7.y};
+}
+// the same from a record that is not in global memory (k_walk's shared-memory copy)
+__device__ __forceinline__ void load_planar_plain(const double* g, Planar& p) {
+    p.q = ld3(g), p.u = ld3(g + 3), p.v = ld3(g + 6), p.n = ld3(g + 9);
+    p.D = g[12];
+    p.w = ld3(g + 13);
 }
 // Quad::hit / Triangle::hit, quad.rs:71-102, triangle.rs:56-98 (geometry only)
 __device__ __forceinline__ bool planar_hit_loaded(const Planar& p, bool triangle, const RayD& r, double tmin, double tmax,
@@ -800,23 +807,20 @@ __device__ __forceinline__ void trace_persistent(const SceneView& sv, IO& io, ui
 
 // ConstantMedium boundary that is one untransformed-or-transformed Sphere: both boundary hits of
 // volume.rs:42-45 share a, h, c and the square root.  Same operations, same order, same results as
-// two Sphere::hit calls on (-inf, inf) and [t1 + 1e-4, inf).
-__device__ __forceinline__ bool sphere_entry_exit(const double* __restrict__ g, const RayD& r, double& t1, double& t2) {
-    const double2 a0 = __ldg(reinterpret_cast<const double2*>(g));
-    const double2 a1 = __ldg(reinterpret_cast<const double2*>(g) + 1);
-    const double2 a2 = __ldg(reinterpret_cast<const double2*>(g) + 2);
-    const double2 a3 = __ldg(reinterpret_cast<const double2*>(g) + 3);
-    D3 center = D3{a0.x, a0.y, a1.x}, cvec = D3{a1.y, a2.x, a2.y};
-    double radius = a3.x;
+// two Sphere::hit calls on (-inf, inf) and [t1 + 1e-4, inf).  near_root / far_root are the two roots Sphere::hit would compute
+// for the same sphere and ray whatever the interval (NaN when the discriminant is negative: no interval contains them).
+__device__ __forceinline__ bool sphere_entry_exit_at(D3 center, D3 cvec, double radius, const RayD& r, double& t1, double& t2, double& near_root,
+                                                     double& far_root) {
     D3 current_center = center + r.time * cvec;
     D3 oc = current_center - r.o;
     double a = length_squared(r.d);
     double h = dot(r.d, oc);
     double c = length_squared(oc) - radius * radius;
     double discriminant = h * h - a * c;
+    near_root = far_root = __longlong_as_double(0x7FF8000000000000ll);
     if (discriminant < 0.0) return false;
     double sqrtd = sqrt(discriminant);
-    const double near_root = (h - sqrtd) / a, far_root = (h + sqrtd) / a;
+    near_root = (h - sqrtd) / a, far_root = (h + sqrtd) / a;
     // first hit on Interval::UNIVERSE: only a NaN root is rejected
     double first = near_root;
     if (!contains(-INFINITY, INFINITY, first)) {
@@ -833,6 +837,14 @@ __device__ __forceinline__ bool sphere_entry_exit(const double* __restrict__ g, 
     t1 = first;
     t2 = second;
     return true;
+}
+__device__ __forceinline__ bool sphere_entry_exit(const double* __restrict__ g, const RayD& r, double& t1, double& t2) {
+    const double2 a0 = __ldg(reinterpret_cast<const double2*>(g));
+    const double2 a1 = __ldg(reinterpret_cast<const double2*>(g) + 1);
+    const double2 a2 = __ldg(reinterpret_cast<const double2*>(g) + 2);
+    const double2 a3 = __ldg(reinterpret_cast<const double2*>(g) + 3);
+    double near_root, far_root;
+    return sphere_entry_exit_at(D3{a0.x, a0.y, a1.x}, D3{a1.y, a2.x, a2.y}, a3.x, r, t1, t2, near_root, far_root);
 }
 
 }  // namespace rt

@@ -75,6 +75,11 @@ class rt_stats(C.Structure):
         """of `segments`: evaluated inside the random-walk kernel of an optically thick medium (rt2025.h, reserved[0])"""
         return int(self.reserved[0])
 
+    @property
+    def walk_lean_segments(self):
+        """of `walk_segments`: evaluated by the lean variant of the random-walk kernel (rt2025.h, reserved[1])"""
+        return int(self.reserved[1])
+
 
 class rt_scene_info(C.Structure):
     _fields_ = [
