@@ -287,7 +287,10 @@ typedef struct rt_stats {
     uint64_t reserved[4];  /* reserved[0]: of `segments`, those evaluated inside the random-walk kernel of an optically
                               thick ConstantMedium (they never passed through extend);
                               reserved[1]: of reserved[0], those evaluated by its lean variant (scenes whose walk needs
-                              no Transform, texture lookup or light-tree code)                      */
+                              no Transform, texture lookup or light-tree code);
+                              reserved[2]: hits shaded by the lean variant of a shade-class kernel (diffuse, textured,
+                              isotropic or emissive hits of scenes whose class needs no Transform, texture lookup or
+                              light-tree code)                                                      */
 } rt_stats;
 
 /* Closest surface hit for a batch of rays over `world` (media excluded: they are stochastic,

@@ -310,7 +310,7 @@ int rt_scene_create(const rt_scene_desc* desc, const rt_build_opts* opts, rt_sce
             cudaStream_t st = cudaStreamPerThread;
             Arena a;
             a.reserve(cs.nodes4), a.reserve(cs.nodes), a.reserve(cs.geom), a.reserve(cs.meta), a.reserve(cs.xforms), a.reserve(cs.materials), a.reserve(cs.textures);
-            a.reserve(cs.images), a.reserve(cs.texels), a.reserve(cs.perlins), a.reserve(cs.media), a.reserve(cs.lights), a.reserve(cs.remaps), a.reserve(cs.walk_lean);
+            a.reserve(cs.images), a.reserve(cs.texels), a.reserve(cs.perlins), a.reserve(cs.media), a.reserve(cs.lights), a.reserve(cs.remaps), a.reserve(cs.walk_lean), a.reserve(cs.shade_lean);
             a.allocate(st);
             s->arena = a.base;
             v.nodes4 = a.put(cs.nodes4, st), v.world_root4 = cs.world_root4;
@@ -318,6 +318,7 @@ int rt_scene_create(const rt_scene_desc* desc, const rt_build_opts* opts, rt_sce
             v.materials = a.put(cs.materials, st), v.textures = a.put(cs.textures, st), v.images = a.put(cs.images, st);
             v.texels = a.put(cs.texels, st), v.perlins = a.put(cs.perlins, st), v.media = a.put(cs.media, st);
             v.lights = a.put(cs.lights, st), v.remaps = a.put(cs.remaps, st), v.walk_lean = a.put(cs.walk_lean, st);
+            v.shade_lean = a.put(cs.shade_lean, st), v.shade_lean_mask = cs.shade_lean_mask;
             CU(cudaStreamSynchronize(st));  // the host vectors die with this call
         }
         v.world_root = cs.world_root;
@@ -785,6 +786,7 @@ int rt_render_device(const rt_scene* cs, const rt_camera* cam, const rt_render_o
             stats->iterations = total_paths ? c.iterations : 0;
             stats->reserved[0] = total_paths ? c.walk_segments : 0;  // rt_stats.walk_segments
             stats->reserved[1] = total_paths ? c.walk_lean_segments : 0;  // rt_stats.walk_lean_segments
+            stats->reserved[2] = total_paths ? c.shade_lean_hits : 0;  // rt_stats.shade_lean_hits
             stats->kernel_launches = launches;
             stats->ms_total = ms;
             stats->ms_raygen = ms_gen, stats->ms_extend = ms_ext, stats->ms_shade = ms_shd;

@@ -1091,17 +1091,49 @@ struct Compiler {
         }
         walk_lean();
         if (timer.on) fprintf(stderr, "[rt2025 compile] random walk: %s\n", out.walk_lean.empty() ? "generic" : (out.walk_lean[0].shell != RT_NONE ? "lean, shell" : "lean"));
+        shade_lean();
+        if (timer.on) {
+            std::string classes;
+            const std::pair<uint32_t, const char*> names[] = {{SC_DIFFUSE, " diffuse"}, {SC_TEXTURED, " textured"}, {SC_ISOTROPIC, " isotropic"}, {SC_EMISSIVE, " emissive"}};
+            for (const auto& c : names)
+                if (out.shade_lean_mask & (1u << c.first)) classes += c.second;
+            fprintf(stderr, "[rt2025 compile] shade lean:%s\n", classes.empty() ? " generic" : classes.c_str());
+        }
         return RT_OK;
+    }
+
+    // scene_types.h, LeanLights: the staged light list, or false when the scene's list is not flat, is longer than LEAN_LIGHTS or
+    // has a leaf below a Transform
+    bool lean_lights(LeanLights& L) const {
+        std::memset(&L, 0, sizeof(L));
+        const size_t n = out.lights.size();
+        if (n > LEAN_LIGHTS) return false;
+        for (size_t i = 0; i < n; i++) {  // flat: every leaf weighs 1/n (rt_scene_create's test)
+            const Light& l = out.lights[i];
+            if (l.xform != RT_NONE || l.weight != 1.0 / (double)n) return false;
+            L.lights[i] = l;
+        }
+        L.n = (uint32_t)n;
+        return true;
+    }
+
+    // albedo / (4 pi) of an Isotropic over a solid texture, as shade_one computes it (D3 / double), or false for any other material
+    bool isotropic_axp(uint32_t material, double* axp) const {
+        const Material& iso = out.materials[material];
+        if (iso.kind != RT_MAT_ISOTROPIC || iso.tex >= out.textures.size() || out.textures[iso.tex].kind != RT_TEX_SOLID) return false;
+        for (int k = 0; k < 3; k++) axp[k] = (1.0 / (4.0 * 3.14159265358979323846264338327950288)) * out.textures[iso.tex].color[k];
+        return true;
     }
 
     // scene_types.h, WalkLean: the record of the lean random walk when the scene qualifies, otherwise nothing
     void walk_lean() {
         out.walk_lean.clear();
-        const size_t n_media = out.media.size(), n_lights = out.lights.size();
-        if (n_media > WALK_LEAN_MEDIA || n_lights > WALK_LEAN_LIGHTS) return;
+        const size_t n_media = out.media.size();
+        if (n_media > WALK_LEAN_MEDIA) return;
         WalkLean L;
         std::memset(&L, 0, sizeof(L));
-        L.n_media = (uint32_t)n_media, L.n_lights = (uint32_t)n_lights, L.thick = RT_NONE, L.shell = RT_NONE;
+        if (!lean_lights(L.lights)) return;
+        L.n_media = (uint32_t)n_media, L.thick = RT_NONE, L.shell = RT_NONE;
         for (size_t m = 0; m < n_media; m++) {
             const Medium& med = out.media[m];
             if (med.single_sphere == RT_NONE || med.xform != RT_NONE || out.meta[med.single_sphere].xform != RT_NONE) return;
@@ -1115,14 +1147,7 @@ struct Compiler {
         }
         if (L.thick == RT_NONE) return;
         const Medium& thick = out.media[L.thick];
-        const Material& iso = out.materials[thick.material];
-        if (iso.kind != RT_MAT_ISOTROPIC || iso.tex >= out.textures.size() || out.textures[iso.tex].kind != RT_TEX_SOLID) return;
-        for (int k = 0; k < 3; k++) L.axp[k] = (1.0 / (4.0 * 3.14159265358979323846264338327950288)) * out.textures[iso.tex].color[k];  // D3 / double
-        for (size_t i = 0; i < n_lights; i++) {  // flat: every leaf weighs 1/n (rt_scene_create's test)
-            const Light& l = out.lights[i];
-            if (l.xform != RT_NONE || l.weight != 1.0 / (double)n_lights) return;
-            L.lights[i] = l;
-        }
+        if (!isotropic_axp(thick.material, L.axp)) return;
         for (uint32_t e = 0; e < thick.n_entry; e++) {
             const uint32_t first = (thick.entry[e] & ~LEAF_FLAG) >> 3, count = (thick.entry[e] & 7u) + 1;
             for (uint32_t pi = first; pi < first + count; pi++) {
@@ -1136,6 +1161,39 @@ struct Compiler {
             }
         }
         out.walk_lean.push_back(L);
+    }
+
+    // scene_types.h, ShadeLean: which shade classes may run their lean kernel, and the record they stage
+    void shade_lean() {
+        out.shade_lean.clear();
+        out.shade_lean_mask = 0;
+        ShadeLean S;
+        std::memset(&S, 0, sizeof(S));
+        const bool lights = lean_lights(S.lights);
+        // SC_ISOTROPIC: the scatter points of every medium that is not MEDIUM_THICK (those go to k_walk) land there
+        bool iso = lights && out.media.size() <= SHADE_LEAN_MEDIA;
+        for (size_t m = 0; iso && m < out.media.size(); m++) {
+            const Medium& med = out.media[m];
+            if (med.flags & MEDIUM_THICK) continue;
+            iso = med.xform == RT_NONE && isotropic_axp(med.material, S.axp[m]);
+        }
+        // the classes of the surfaces: one with an Isotropic material would land in SC_ISOTROPIC as well
+        bool emissive = true;
+        for (size_t p = 0; p < out.meta.size() && (iso || emissive); p++) {
+            const PrimMeta& pm = out.meta[p];
+            const uint32_t cls = (pm.kind_mat >> META_CLASS_SHIFT) & 15u;
+            if (cls == SC_ISOTROPIC) iso = false;
+            if (cls == SC_EMISSIVE) {
+                const Material& M = out.materials[pm.kind_mat & META_MAT_MASK];
+                if (pm.xform != RT_NONE || M.kind != RT_MAT_DIFFUSE_LIGHT || M.inner != RT_NONE || M.tex >= out.textures.size() ||
+                    out.textures[M.tex].kind != RT_TEX_SOLID)
+                    emissive = false;
+            }
+        }
+        if (lights) out.shade_lean_mask |= 1u << SC_DIFFUSE | 1u << SC_TEXTURED;
+        if (iso) out.shade_lean_mask |= 1u << SC_ISOTROPIC;
+        if (emissive) out.shade_lean_mask |= 1u << SC_EMISSIVE;
+        if (out.shade_lean_mask) out.shade_lean.push_back(S);
     }
 };
 

@@ -54,6 +54,8 @@ struct CompiledScene {
     std::vector<Remap> remaps;
     std::vector<uint32_t> ranks;  // per desc object, RT_NONE for containers
     std::vector<WalkLean> walk_lean;  // one record when the scene qualifies for the lean random walk, else empty
+    std::vector<ShadeLean> shade_lean;  // one record when some shade class qualifies for its lean kernel, else empty
+    uint32_t shade_lean_mask = 0;       // bit c: shade class c runs its lean kernel (scene_types.h, ShadeLean)
     uint32_t world_root = INVALID_REF;
     uint32_t bvh_depth = 0;        // world group (binary tree)
     uint32_t media_bvh_depth = 0;  // deepest ConstantMedium boundary group

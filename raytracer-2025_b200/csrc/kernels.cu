@@ -611,9 +611,13 @@ __device__ __forceinline__ void contribute(const RenderParams& P, const Wavefron
 // emitted + scatter + mixture-pdf light sampling for ONE hit (camera.rs:288-321).  Returns whether the path goes on, with the
 // next ray and throughput in nr / nbeta.  One instantiation per shade class: everything another class would need is compiled
 // out; CLS == SC_OTHER is the fully general version (Mix, Portal, Transparent, lights that wrap a material, misses, media).
-template <uint32_t CLS>
+// LEAN (SC_DIFFUSE, SC_TEXTURED; scene_types.h, ShadeLean): the light list is the staged flat list `LL`, and a SC_DIFFUSE albedo
+// is read straight from its solid texture.
+template <uint32_t CLS, bool LEAN = false>
 __device__ __forceinline__ bool shade_one(const SceneView& sv, const RenderParams& P, const WavefrontState& W, const RayD& r, D3 beta, uint32_t pixel,
-                                          uint32_t sidx, uint32_t segment, double t, uint32_t prim, uint32_t kind, RayD& nr, D3& nbeta) {
+                                          uint32_t sidx, uint32_t segment, double t, uint32_t prim, uint32_t kind, RayD& nr, D3& nbeta,
+                                          const LeanLights* LL = nullptr) {
+    static_assert(!LEAN || CLS == SC_DIFFUSE || CLS == SC_TEXTURED, "the other lean classes have their own code");
     constexpr bool GENERIC = CLS == SC_OTHER;
     constexpr bool DO_MISS = CLS == SC_MISS;
     constexpr bool DO_MEDIUM = GENERIC || CLS == SC_ISOTROPIC;
@@ -748,7 +752,9 @@ __device__ __forceinline__ bool shade_one(const SceneView& sv, const RenderParam
                             // ScatterRecord::PDF branch, camera.rs:297-312
                             const bool iso = CLS == SC_ISOTROPIC || (GENERIC && M.kind == RT_MAT_ISOTROPIC);
                             const bool dis = CLS == SC_DISNEY || (GENERIC && M.kind == RT_MAT_DISNEY);
-                            D3 albedo = (M.kind == RT_MAT_EMPTY || dis) ? D3{0.75, 0.75, 0.75} : texture_value(sv, M.tex, h.u, h.v, h.p);
+                            D3 albedo = (M.kind == RT_MAT_EMPTY || dis)  ? D3{0.75, 0.75, 0.75}
+                                        : (LEAN && CLS == SC_DIFFUSE) ? ld3(sv.textures[M.tex].color)  // texture_value of a solid texture
+                                                                      : texture_value(sv, M.tex, h.u, h.v, h.p);
                             ONB uvw;
                             if (!iso && !make_onb(h.normal, uvw)) {
                                 error = true;
@@ -773,13 +779,13 @@ __device__ __forceinline__ bool shade_one(const SceneView& sv, const RenderParam
                             Rand2 pick = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_MIXTURE);
                             Rand2 dx = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_DIRECTION);
                             D3 gen = D3{0.0, 0.0, 0.0};
-                            const bool have_lights = sv.n_lights > 0;
+                            const bool have_lights = LEAN ? LL->n > 0 : sv.n_lights > 0;
                             // No `break` inside the divergent sampling branch below: with an early-exit edge the warp would
                             // only reconverge at the end of the switch and run the whole pdf evaluation once per side
                             // (measured: 16 of 32 lanes active from here on).  stop: 1 = the reference panics, 2 = None (black).
                             int stop = 0;
                             if (have_lights && !(pick.a < 0.5)) {
-                                if (!lights_random(sv, h.p, pick.b, dx.a, dx.b, gen)) stop = 1;
+                                if (!(LEAN ? lean_lights_random(*LL, h.p, pick.b, dx.a, dx.b, gen) : lights_random(sv, h.p, pick.b, dx.a, dx.b, gen))) stop = 1;
                             } else if (dis) {
                                 Rand2 dpick = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_DISNEY);
                                 D3 v_in_l;
@@ -816,7 +822,7 @@ __device__ __forceinline__ bool shade_one(const SceneView& sv, const RenderParam
                             }
                             double pdf_val = value0;
                             if (!stop && have_lights) {
-                                double value1 = lights_pdf_value(sv, P.lights_flat, h.p, gen);
+                                double value1 = LEAN ? lean_lights_pdf(sv, *LL, h.p, gen) : lights_pdf_value(sv, P.lights_flat, h.p, gen);
                                 if (isnan(value1) || (value0 == 0.0 && value1 == 0.0))  // hits.rs:64, pdf.rs:105-109
                                     stop = 1;
                                 else
@@ -844,14 +850,73 @@ __device__ __forceinline__ bool shade_one(const SceneView& sv, const RenderParam
             return alive;
 }
 
+// shade_one<SC_ISOTROPIC> at the scatter point r.at(t) of a medium below no Transform whose Isotropic has a solid albedo
+// (axp = albedo / (4 pi)), over a staged flat light list: the same operations in the same order, without the normal, uv, ONB and
+// texture lookup a solid Isotropic does not use.  Returns whether the path goes on (nr, nbeta).  Used by k_shade<SC_ISOTROPIC, true>
+// and by every segment of the lean k_walk.
+__device__ __forceinline__ bool lean_isotropic_scatter(const SceneView& sv, const LeanLights& L, D3 axp, const RenderParams& P, const WavefrontState& W,
+                                                       const RayD& r, D3 beta, uint32_t pixel, uint32_t sidx, uint32_t segment, double t, RayD& nr,
+                                                       D3& nbeta) {
+    nr.o = r.o + t * r.d;  // volume.rs:66-72 (h.p)
+    nr.time = r.time;
+    const Rand2 pick = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_MIXTURE);
+    const Rand2 dx = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_DIRECTION);
+    D3 gen = D3{0.0, 0.0, 0.0};
+    bool panic = false;  // shade_one's stop == 1 (None cannot occur here)
+    if (L.n > 0 && !(pick.a < 0.5))
+        panic = !lean_lights_random(L, nr.o, pick.b, dx.a, dx.b, gen);
+    else
+        gen = random_unit_vector(dx.a, dx.b);
+    const double value0 = 1.0 / (4.0 * RT_PI);
+    double pdf_val = value0;
+    if (!panic && L.n > 0) {
+        const double value1 = lean_lights_pdf(sv, L, nr.o, gen);
+        if (isnan(value1) || (value0 == 0.0 && value1 == 0.0))
+            panic = true;
+        else
+            pdf_val = value0 * 0.5 + value1 * 0.5;
+    }
+    if (panic || pdf_val == 0.0) {
+        atomicAdd(&W.counters->errors, 1ull);
+        return false;
+    }
+    nr.d = gen;
+    nbeta = beta * (axp / pdf_val);
+    return !(segment + 1 >= P.cam.max_depth || (nbeta.x == 0.0 && nbeta.y == 0.0 && nbeta.z == 0.0));
+}
+
+// CTAs per SM of the lean class kernels, one hex digit per shade class (digit c: class c).  Measured on book2 (torch.profiler, ms
+// per frame at 2 / 3 / 4 CTAs): diffuse 39.1 / 34.0 / 35.9, textured 18.3 / 20.0 / 22.5, isotropic 22.5 / 20.9 / 20.6, emissive
+// 14.5 / 12.7 / 13.0.  Isotropic keeps three: four is within 0.3 ms and spills more.
+#ifndef RT_SHADE_LEAN_BLOCKS
+#define RT_SHADE_LEAN_BLOCKS 0x3003230u
+#endif
+constexpr int shade_lean_blocks(uint32_t cls) { return (int)((RT_SHADE_LEAN_BLOCKS >> (4u * cls)) & 15u); }
+constexpr int shade_blocks(uint32_t cls, bool lean) {
+    return lean ? shade_lean_blocks(cls) : (((RT_SHADE_3BLOCK_MASK >> cls) & 1u) ? 3 : RT_SHADE_MIN_BLOCKS);
+}
+
 // One instantiation per shade class (scene_types.h ShadeClass): the queue it reads only holds hits
 // of that class, so everything another class would need is compiled out and the kernel keeps few
 // registers.  CLS == SC_OTHER is the fully general version (Mix, Portal, Transparent, lights that
 // wrap a material) and is also what runs when binning is switched off.
-template <uint32_t CLS>
-__global__ void __launch_bounds__(SHADE_BLOCK, ((RT_SHADE_3BLOCK_MASK >> CLS) & 1u) ? 3 : RT_SHADE_MIN_BLOCKS) k_shade(SceneView sv, RenderParams P, WavefrontState W, uint32_t queue) {
+// LEAN: the scene lets class CLS skip the code it cannot reach (scene_types.h, ShadeLean; SceneView::shade_lean_mask); each CTA
+// copies the ShadeLean record to shared memory first.  SC_EMISSIVE then only adds beta * the light's colour: it reads the path
+// ids, the throughput and the hit record, and no geometry.
+template <uint32_t CLS, bool LEAN = false>
+__global__ void __launch_bounds__(SHADE_BLOCK, shade_blocks(CLS, LEAN)) k_shade(SceneView sv, RenderParams P, WavefrontState W, uint32_t queue) {
+    constexpr bool EMIT_ONLY = LEAN && CLS == SC_EMISSIVE;
     __shared__ uint32_t s_warp_count[SHADE_BLOCK / 32];
     __shared__ uint32_t s_base;
+    extern __shared__ float4 s_lean[];  // LEAN: the ShadeLean record
+    const ShadeLean& SL = *reinterpret_cast<const ShadeLean*>(s_lean);
+    if (LEAN && !EMIT_ONLY) {
+        unsigned long long* dst = reinterpret_cast<unsigned long long*>(s_lean);
+        const unsigned long long* src = reinterpret_cast<const unsigned long long*>(sv.shade_lean);
+        for (uint32_t k = threadIdx.x; k < sizeof(ShadeLean) / 8; k += SHADE_BLOCK) dst[k] = src[k];
+        __syncthreads();
+    }
+    unsigned long long lean_hits = 0;  // thread 0: the entries this CTA shaded
     const uint32_t n = W.counters->n_shade[queue];
     const RayRec* __restrict__ rays = W.ray_q[W.parity];
     const BetaRec* __restrict__ betas = W.beta_q[W.parity];
@@ -873,21 +938,38 @@ __global__ void __launch_bounds__(SHADE_BLOCK, ((RT_SHADE_3BLOCK_MASK >> CLS) & 
             }
         }
 #endif
+        if (LEAN && threadIdx.x == 0) lean_hits += min(n - j0, (uint32_t)SHADE_BLOCK);
         if (j < n) {
             const uint32_t pos = W.q_shade[queue][j];
-            RayD r;
-            uint64_t ids64;
-            load_ray(rays + pos, r, ids64);
-            unpack_ids(ids64, pixel, sidx, segment);
-            const double2* sp2 = reinterpret_cast<const double2*>(betas + pos);
-            const double2 b0 = sp2[0], b1 = sp2[1];
-            D3 beta = D3{b0.x, b0.y, b1.x};
-            const double2 hw = *reinterpret_cast<const double2*>(W.hit_q + pos);
-            const double t = hw.x;
-            const uint32_t prim = (uint32_t)__double2hiint(hw.y), kind = (uint32_t)__double2loint(hw.y);
-            const bool alive = shade_one<CLS>(sv, P, W, r, beta, pixel, sidx, segment, t, prim, kind, nr, nbeta);
-            q = alive ? 0 : -1;
+            if constexpr (EMIT_ONLY) {  // material_emitted of a DiffuseLight over a solid texture; the path ends
+                unpack_ids((uint64_t)__double_as_longlong(reinterpret_cast<const double2*>(rays + pos)[3].y), pixel, sidx, segment);
+                const double2* sp2 = reinterpret_cast<const double2*>(betas + pos);
+                const double2 b0 = sp2[0], b1 = sp2[1];
+                const D3 beta = D3{b0.x, b0.y, b1.x};
+                const uint32_t prim = (uint32_t)__double2hiint(reinterpret_cast<const double2*>(W.hit_q + pos)->y);
+                const uint32_t mat = sv.meta[prim].kind_mat & META_MAT_MASK;
+                const D3 e = D3{0.0, 0.0, 0.0} + 1.0 * ld3(sv.textures[sv.materials[mat].tex].color);
+                contribute(P, W, pixel, beta * e);
+            } else {
+                RayD r;
+                uint64_t ids64;
+                load_ray(rays + pos, r, ids64);
+                unpack_ids(ids64, pixel, sidx, segment);
+                const double2* sp2 = reinterpret_cast<const double2*>(betas + pos);
+                const double2 b0 = sp2[0], b1 = sp2[1];
+                D3 beta = D3{b0.x, b0.y, b1.x};
+                const double2 hw = *reinterpret_cast<const double2*>(W.hit_q + pos);
+                const double t = hw.x;
+                const uint32_t prim = (uint32_t)__double2hiint(hw.y), kind = (uint32_t)__double2loint(hw.y);
+                bool alive;
+                if constexpr (LEAN && CLS == SC_ISOTROPIC)  // only media scatter here (ShadeLean): prim is the medium index
+                    alive = lean_isotropic_scatter(sv, SL.lights, ld3(SL.axp[prim]), P, W, r, beta, pixel, sidx, segment, t, nr, nbeta);
+                else
+                    alive = shade_one<CLS, LEAN>(sv, P, W, r, beta, pixel, sidx, segment, t, prim, kind, nr, nbeta, &SL.lights);
+                q = alive ? 0 : -1;
+            }
         }
+        if constexpr (EMIT_ONLY) continue;  // no survivors
         // survivors are appended to the other copy of the streams: one atomic per block
         const unsigned alive_mask = __ballot_sync(0xFFFFFFFFu, q == 0);
         const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
@@ -903,11 +985,14 @@ __global__ void __launch_bounds__(SHADE_BLOCK, ((RT_SHADE_3BLOCK_MASK >> CLS) & 
         uint32_t npos = s_base + __popc(alive_mask & ((1u << lane) - 1u));
         for (uint32_t w = 0; w < warp; w++) npos += s_warp_count[w];
         __syncthreads();  // s_warp_count / s_base are reused by the next iteration
-        if (q == 0) {
-            store_ray(W.ray_q[W.parity ^ 1u] + npos, nr, pack_ids(pixel, sidx, segment + 1));
-            store_beta(W.beta_q[W.parity ^ 1u] + npos, nbeta);
+        if constexpr (!EMIT_ONLY) {
+            if (q == 0) {
+                store_ray(W.ray_q[W.parity ^ 1u] + npos, nr, pack_ids(pixel, sidx, segment + 1));
+                store_beta(W.beta_q[W.parity ^ 1u] + npos, nbeta);
+            }
         }
     }
+    if (LEAN && lean_hits) atomicAdd(&W.counters->shade_lean_hits, lean_hits);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -937,50 +1022,15 @@ constexpr int WALK_BLOCK = RT_WALK_BLOCK;
 #define RT_WALK_LEAN_MIN_BLOCKS 4
 #endif
 
-// One segment of the lean walk (scene_types.h, WalkLean) from a scatter point at t inside the thick medium: the SC_ISOTROPIC part
-// of shade_one with the same operations in the same order, then the look-ahead of k_walk - the thick medium, the thin ones when it
+// One segment of the lean walk (scene_types.h, WalkLean) from a scatter point at t inside the thick medium: lean_isotropic_scatter,
+// then the look-ahead of k_walk - the thick medium, the thin ones when it
 // scattered, the entry primitives - against the staged constants.  Returns whether the path goes on (nr, nbeta); `stay`: the
 // next scatter point (at tn) is again inside the thick medium and nothing beats it.
 __device__ __forceinline__ bool walk_lean_segment(const SceneView& sv, const WalkLean& L, const RenderParams& P, const WavefrontState& W, const RayD& r,
                                                   D3 beta, uint32_t pixel, uint32_t sidx, uint32_t segment, double t, uint32_t max_steps,
                                                   uint32_t& steps, RayD& nr, D3& nbeta, double& tn, bool& stay) {
     stay = false;
-    nr.o = r.o + t * r.d;  // volume.rs:66-72 (h.p); the normal, uv and texture lookup are unused by a solid Isotropic
-    nr.time = r.time;
-    const Rand2 pick = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_MIXTURE);
-    const Rand2 dx = philox_pair(P.seed, pixel, sidx, segment, RT_SLOT_DIRECTION);
-    const uint32_t n_lights = L.n_lights;
-    D3 gen = D3{0.0, 0.0, 0.0};
-    bool panic = false;  // shade_one's stop == 1 (None cannot occur here)
-    if (n_lights > 0 && !(pick.a < 0.5)) {  // lights_random over the flat list
-        uint32_t leaf = n_lights - 1;
-        for (uint32_t i = 0; i < n_lights; i++)
-            if (pick.b < L.lights[i].cdf) {
-                leaf = i;
-                break;
-            }
-        panic = !light_leaf_random(L.lights[leaf], nr.o, dx.a, dx.b, gen);
-    } else {
-        gen = random_unit_vector(dx.a, dx.b);
-    }
-    const double value0 = 1.0 / (4.0 * RT_PI);
-    double pdf_val = value0;
-    if (!panic && n_lights > 0) {  // lights_pdf_value of a flat list: sum / len (x / 1.0 == x: no division for one light)
-        double sum = 0.0;
-        for (uint32_t i = 0; i < n_lights; i++) sum += light_leaf_pdf<true>(sv, L.lights[i], nr.o, gen);
-        const double value1 = n_lights == 1 ? sum : sum / (double)n_lights;
-        if (isnan(value1) || (value0 == 0.0 && value1 == 0.0))
-            panic = true;
-        else
-            pdf_val = value0 * 0.5 + value1 * 0.5;
-    }
-    if (panic || pdf_val == 0.0) {
-        atomicAdd(&W.counters->errors, 1ull);
-        return false;
-    }
-    nr.d = gen;
-    nbeta = beta * (ld3(L.axp) / pdf_val);
-    if (segment + 1 >= P.cam.max_depth || (nbeta.x == 0.0 && nbeta.y == 0.0 && nbeta.z == 0.0)) return false;
+    if (!lean_isotropic_scatter(sv, L.lights, ld3(L.axp), P, W, r, beta, pixel, sidx, segment, t, nr, nbeta)) return false;
 
     // world.hit of the next segment, as sample_media<.., 1> then <.., 2> and leaf_beats_scatter
     const uint32_t seg1 = segment + 1u, thick = L.thick;
@@ -1356,7 +1406,14 @@ int launch_media_bin(const SceneView& sv, const RenderParams& P, const Wavefront
 }
 template <uint32_t CLS>
 static void launch_shade_cls(const SceneView& sv, const RenderParams& P, const WavefrontState& W, uint32_t queue, int grid, cudaStream_t s) {
-    // `grid` is sized for RT_SHADE_MIN_BLOCKS resident CTAs per SM; classes compiled for three get the matching grid
+    // `grid` is sized for RT_SHADE_MIN_BLOCKS resident CTAs per SM; classes compiled for another count get the matching grid
+    if constexpr (CLS == SC_DIFFUSE || CLS == SC_TEXTURED || CLS == SC_ISOTROPIC || CLS == SC_EMISSIVE) {
+        if (queue == CLS && (sv.shade_lean_mask >> CLS) & 1u) {  // the scene compiler's choice (scene_types.h, ShadeLean)
+            static_assert(shade_lean_blocks(CLS) >= 1, "RT_SHADE_LEAN_BLOCKS: no CTA count for a lean class");
+            k_shade<CLS, true><<<grid / RT_SHADE_MIN_BLOCKS * shade_lean_blocks(CLS), SHADE_BLOCK, CLS == SC_EMISSIVE ? 0 : sizeof(ShadeLean), s>>>(sv, P, W, queue);
+            return;
+        }
+    }
     if ((RT_SHADE_3BLOCK_MASK >> CLS) & 1u) grid = grid / RT_SHADE_MIN_BLOCKS * 3;
     k_shade<CLS><<<grid, SHADE_BLOCK, 0, s>>>(sv, P, W, queue);
 }

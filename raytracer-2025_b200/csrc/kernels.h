@@ -108,6 +108,7 @@ struct Counters {
     unsigned long long next_path, segments, iterations, errors, node_visits, prim_tests;
     unsigned long long walk_segments;  // of `segments`: evaluated inside k_walk (they never went through the streams)
     unsigned long long walk_lean_segments;  // of `walk_segments`: evaluated by the lean variant of k_walk (SceneView::walk_lean)
+    unsigned long long shade_lean_hits;     // hits shaded by a lean class kernel (k_shade<CLS, true>, SceneView::shade_lean_mask)
 };
 
 struct WavefrontState {

@@ -132,14 +132,24 @@ struct Light {
     double weight, cdf, area;
 };
 
+// The light list as the lean kernels stage it (WalkLean, ShadeLean): flat - every leaf weighs 1/n - with at most LEAN_LIGHTS
+// leaves, none of them below a Transform, so the mixture pdf needs no light-tree or Transform code (kernels.cu, lean_lights_*).
+// The scene compiler fills it (compile.cpp, lean_lights) or finds that the scene's list does not qualify.
+constexpr uint32_t LEAN_LIGHTS = 4;
+struct LeanLights {
+    Light lights[LEAN_LIGHTS];  // as in lights[]
+    uint32_t n;
+    uint32_t pad[7];
+};
+
 // The constants of the lean random walk (k_walk<.., LEAN>), gathered by the scene compiler for a scene whose walk needs none of
 // the generic machinery: one MEDIUM_THICK medium with its entry leaves, every medium bounded by one untransformed Sphere, an
-// Isotropic over a solid texture in the thick one, a flat list of at most WALK_LEAN_LIGHTS untransformed lights and at most
-// WALK_LEAN_PRIMS untransformed primitives in the entry leaves.  The kernel copies the record to shared memory once per CTA, so a
-// segment makes no dependent loads through media[], materials[], textures[], meta[] or lights[].
-constexpr uint32_t WALK_LEAN_MEDIA = 4, WALK_LEAN_LIGHTS = 4, WALK_LEAN_PRIMS = 8;
+// Isotropic over a solid texture in the thick one, a LeanLights list and at most WALK_LEAN_PRIMS untransformed primitives in the
+// entry leaves.  The kernel copies the record to shared memory once per CTA, so a segment makes no dependent loads through
+// media[], materials[], textures[], meta[] or lights[].
+constexpr uint32_t WALK_LEAN_MEDIA = 4, WALK_LEAN_PRIMS = 8;
 struct WalkLean {
-    Light lights[WALK_LEAN_LIGHTS];      // the flat light list, as in lights[]
+    LeanLights lights;
     PrimGeom prim[WALK_LEAN_PRIMS];      // the primitives of the thick medium's entry leaves, in leaf order
     double sphere[WALK_LEAN_MEDIA][8];   // boundary Sphere of every medium: centre(3) centre_vec(3) radius
     double neg_inv_density[WALK_LEAN_MEDIA];
@@ -147,11 +157,24 @@ struct WalkLean {
     double pad0;
     uint32_t rank[WALK_LEAN_MEDIA], medium_index[WALK_LEAN_MEDIA];
     uint32_t prim_kind[WALK_LEAN_PRIMS], prim_rank[WALK_LEAN_PRIMS];
-    uint32_t n_media, thick, n_lights, n_prims;
+    uint32_t n_media, thick, n_prims;
     // entry primitive whose geometry is bit-identical to the thick boundary sphere (the glass shell around book2's subsurface
     // ball), or RT_NONE: its hit on a segment is decided from the roots the boundary test has already computed
     uint32_t shell;
-    uint32_t pad1[3];
+};
+
+// The constants of the lean shade-class kernels (k_shade<CLS, true>), gathered by the scene compiler; SceneView::shade_lean_mask
+// says which classes may use them (bit c: class c):
+//   SC_DIFFUSE, SC_TEXTURED - the light list is a LeanLights list;
+//   SC_ISOTROPIC            - the same, no surface has an Isotropic material, and every medium that is not MEDIUM_THICK sits below
+//                             no Transform and scatters with an Isotropic over a solid texture (its albedo / (4 pi) is in axp);
+//   SC_EMISSIVE             - every primitive of the class sits below no Transform and its DiffuseLight (no inner material) has a
+//                             solid texture.
+// Each CTA copies the record to shared memory, as k_walk does with WalkLean.
+constexpr uint32_t SHADE_LEAN_MEDIA = 4;
+struct ShadeLean {
+    LeanLights lights;
+    double axp[SHADE_LEAN_MEDIA][4];  // per medium index: albedo / (4 pi) of its Isotropic (shade_one's expression), w unused
 };
 
 // shade work classes used to bin hits (extend -> shade queues)
@@ -200,6 +223,8 @@ struct SceneView {
     uint32_t walk_entries_only;  // exactly one MEDIUM_THICK medium and it has its entry leaves: k_walk never traverses from the world root
     uint32_t fifo_slots;      // prepared-ray FIFO slots per warp of the persistent traversal: 32 or 64; 0 = no FIFO (traverse.cuh)
     const WalkLean* walk_lean;  // the scene qualifies for the lean random walk (one record), or nullptr: the generic k_walk
+    const ShadeLean* shade_lean;  // the constants of the lean shade-class kernels (one record), or nullptr: every class generic
+    uint32_t shade_lean_mask;     // bit c: shade class c runs its lean kernel (ShadeLean)
 };
 
 }  // namespace rt

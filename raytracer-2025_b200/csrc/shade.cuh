@@ -195,7 +195,7 @@ __device__ inline bool remap_record(const SceneView& sv, const Remap& rm, HitInf
 }
 
 // ---- lights: Hittables::pdf_value / random over the flattened leaves (hits.rs:52-75) -----------
-// STAGED: `l` is an untransformed light copied out of global memory (k_walk's lean variant)
+// STAGED: `l` is an untransformed light copied out of global memory (LeanLights)
 template <bool STAGED = false>
 __device__ inline double light_leaf_pdf(const SceneView& sv, const Light& l, D3 origin, D3 direction) {
     if (!STAGED && l.xform != RT_NONE) {  // Transform::pdf_value, shapes.rs:117-123, outermost Transform first
@@ -301,6 +301,23 @@ __device__ inline bool lights_random(const SceneView& sv, D3 origin, double pick
     }
     out = dir;
     return ok;
+}
+
+// The same two over a staged flat list (scene_types.h, LeanLights): no Transform chain, every leaf weighs 1/n.
+__device__ __forceinline__ bool lean_lights_random(const LeanLights& L, D3 origin, double pick, double r1, double r2, D3& out) {
+    uint32_t leaf = L.n - 1;
+    for (uint32_t i = 0; i < L.n; i++)
+        if (pick < L.lights[i].cdf) {
+            leaf = i;
+            break;
+        }
+    return light_leaf_random(L.lights[leaf], origin, r1, r2, out);
+}
+// sum / len as lights_pdf_value (x / 1.0 == x: no division for one light)
+__device__ __forceinline__ double lean_lights_pdf(const SceneView& sv, const LeanLights& L, D3 origin, D3 direction) {
+    double sum = 0.0;
+    for (uint32_t i = 0; i < L.n; i++) sum += light_leaf_pdf<true>(sv, L.lights[i], origin, direction);
+    return L.n == 1 ? sum : sum / (double)L.n;
 }
 
 // shapes/environment.rs:14-24

@@ -80,6 +80,11 @@ class rt_stats(C.Structure):
         """of `walk_segments`: evaluated by the lean variant of the random-walk kernel (rt2025.h, reserved[1])"""
         return int(self.reserved[1])
 
+    @property
+    def shade_lean_hits(self):
+        """hits shaded by the lean variant of a shade-class kernel (rt2025.h, reserved[2])"""
+        return int(self.reserved[2])
+
 
 class rt_scene_info(C.Structure):
     _fields_ = [
