@@ -305,6 +305,25 @@ int rt_closest_hit_device(const rt_scene* scene, const rt_ray* d_rays, uint64_t 
                           double t_max, uint32_t flags, rt_hit* d_out, void* stream,
                           rt_stats* stats);
 
+/* Occlusion (any-hit) query for a batch of rays over `world`.  With
+ * t_max_i = t_max_per_ray ? t_max_per_ray[i] : t_max,
+ *     out[i] = 1 iff some surface primitive has a hit t with Interval::contains(t_min, t_max_i, t)
+ *              (inclusive at both ends, utils/interval.rs:65-67), else 0.
+ * This is geometric visibility: every surface occludes whatever its material (Dielectric,
+ * Transparent, Portal and emitters alike); media are excluded as in rt_closest_hit and no
+ * transmittance is computed.  An empty interval (t_max_i < t_min, or a NaN bound) gives 0.
+ * With the same primitive arithmetic as rt_closest_hit, bit for bit:
+ *     out[i] == (closest_hit(ray, t_min, +inf).prim_id != RT_NONE && .t <= t_max_i)
+ * A ray's traversal ends at the first hit found, so it visits at most the nodes and primitives
+ * closest hit would.  `stats` gets segments = n, ms_total and kernel_launches, and node_visits /
+ * prim_tests with RT_OPT_COUNT.  Host-pointer version copies in and out; the _device version
+ * takes device pointers (t_max_per_ray may be NULL) and enqueues on `stream`. */
+int rt_occluded(const rt_scene* scene, const rt_ray* rays, const double* t_max_per_ray /* n values or NULL */,
+                uint64_t n, double t_min, double t_max, uint32_t flags, uint8_t* out, rt_stats* stats);
+int rt_occluded_device(const rt_scene* scene, const rt_ray* d_rays, const double* d_t_max_per_ray,
+                       uint64_t n, double t_min, double t_max, uint32_t flags, uint8_t* d_out,
+                       void* stream, rt_stats* stats);
+
 typedef enum rt_accum_type { RT_ACCUM_F32 = 0, RT_ACCUM_F64 = 1 } rt_accum_type;
 
 typedef struct rt_render_opts {

@@ -253,6 +253,62 @@ int check_device(int requested, int& device, int& sm_count) {
     return RT_OK;
 }
 
+// The body of the _device batch queries: the batch size check, RT_OPT_COUNT counters, event timing and `stats`.
+// launch(count, d_counters, grid, stream) enqueues the kernel.
+template <class Launch>
+int run_batch(const rt_scene* s, uint64_t n, uint32_t flags, void* stream, rt_stats* stats, Launch launch) {
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    if (n == 0) return RT_OK;
+    if (n > 0xFFFFFFF0ull) return set_err(RT_ERR_INVALID, "more than 2^32 rays in one batch");
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned long long* d_cnt = nullptr;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    int rc = RT_OK;
+    DeviceGuard guard;
+    try {
+        CU(cudaSetDevice(s->device));
+        // counters are only read back through `stats`: without it the kernel runs the uncounted instantiation.
+        // The buffer is allocated and freed in stream order on the caller's stream, like the kernel that writes it.
+        const bool count = (flags & RT_OPT_COUNT) != 0 && stats != nullptr;
+        if (count) {
+            CU(cudaMallocAsync((void**)&d_cnt, 2 * sizeof(unsigned long long), st));
+            CU(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(unsigned long long), st));
+        }
+        int grid = s->sm_count * s->extend_blocks_per_sm;
+        uint64_t need = (n + EXTEND_BLOCK - 1) / EXTEND_BLOCK;
+        if ((uint64_t)grid > need) grid = (int)need;
+        if (stats) {
+            CU(cudaEventCreate(&e0));
+            CU(cudaEventCreate(&e1));
+            CU(cudaEventRecord(e0, st));
+        }
+        launch(count, d_cnt, grid, st);
+        CU(cudaGetLastError());
+        if (stats) {
+            CU(cudaEventRecord(e1, st));
+            CU(cudaEventSynchronize(e1));
+            float ms = 0;
+            CU(cudaEventElapsedTime(&ms, e0, e1));
+            stats->ms_total = ms;
+            stats->ms_extend = ms;
+            stats->segments = n;
+            stats->kernel_launches = 1;
+            if (count) {
+                unsigned long long h[2];
+                CU(cudaMemcpyAsync(h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
+                CU(cudaStreamSynchronize(st));
+                stats->node_visits = h[0], stats->prim_tests = h[1];
+            }
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    if (e0) cudaEventDestroy(e0);
+    if (e1) cudaEventDestroy(e1);
+    if (d_cnt) cudaFreeAsync(d_cnt, st);
+    return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -481,56 +537,9 @@ int rt_scene_get_ranks(const rt_scene* s, uint32_t* ranks, uint32_t n) {
 int rt_closest_hit_device(const rt_scene* s, const rt_ray* d_rays, uint64_t n, double t_min, double t_max, uint32_t flags,
                           rt_hit* d_out, void* stream, rt_stats* stats) {
     if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
-    if (stats) std::memset(stats, 0, sizeof(*stats));
-    if (n == 0) return RT_OK;
-    if (n > 0xFFFFFFF0ull) return set_err(RT_ERR_INVALID, "more than 2^32 rays in one batch");
-    cudaStream_t st = (cudaStream_t)stream;
-    unsigned long long* d_cnt = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    int rc = RT_OK;
-    DeviceGuard guard;
-    try {
-        CU(cudaSetDevice(s->device));
-        // counters are only read back through `stats`: without it the kernel runs the uncounted instantiation.
-        // The buffer is allocated and freed in stream order on the caller's stream, like the kernel that writes it.
-        const bool count = (flags & RT_OPT_COUNT) != 0 && stats != nullptr;
-        if (count) {
-            CU(cudaMallocAsync((void**)&d_cnt, 2 * sizeof(unsigned long long), st));
-            CU(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(unsigned long long), st));
-        }
-        int grid = s->sm_count * s->extend_blocks_per_sm;
-        uint64_t need = (n + EXTEND_BLOCK - 1) / EXTEND_BLOCK;
-        if ((uint64_t)grid > need) grid = (int)need;
-        if (stats) {
-            CU(cudaEventCreate(&e0));
-            CU(cudaEventCreate(&e1));
-            CU(cudaEventRecord(e0, st));
-        }
+    return run_batch(s, n, flags, stream, stats, [&](bool count, unsigned long long* d_cnt, int grid, cudaStream_t st) {
         launch_closest_hit(s->view, d_rays, (uint32_t)n, t_min, t_max, count, d_out, d_cnt, grid, s->stack_bytes, st);
-        CU(cudaGetLastError());
-        if (stats) {
-            CU(cudaEventRecord(e1, st));
-            CU(cudaEventSynchronize(e1));
-            float ms = 0;
-            CU(cudaEventElapsedTime(&ms, e0, e1));
-            stats->ms_total = ms;
-            stats->ms_extend = ms;
-            stats->segments = n;
-            stats->kernel_launches = 1;
-            if (count) {
-                unsigned long long h[2];
-                CU(cudaMemcpyAsync(h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
-                CU(cudaStreamSynchronize(st));
-                stats->node_visits = h[0], stats->prim_tests = h[1];
-            }
-        }
-    } catch (const CudaFail& f) {
-        rc = set_err(RT_ERR_CUDA, f.what);
-    }
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    if (d_cnt) cudaFreeAsync(d_cnt, st);
-    return rc;
+    });
 }
 
 int rt_closest_hit(const rt_scene* s, const rt_ray* rays, uint64_t n, double t_min, double t_max, uint32_t flags, rt_hit* out,
@@ -558,6 +567,49 @@ int rt_closest_hit(const rt_scene* s, const rt_ray* rays, uint64_t n, double t_m
         rc = set_err(RT_ERR_CUDA, f.what);
     }
     scratch_free(d_rays);
+    scratch_free(d_out);
+    return rc;
+}
+
+int rt_occluded_device(const rt_scene* s, const rt_ray* d_rays, const double* d_t_max_per_ray, uint64_t n, double t_min, double t_max,
+                       uint32_t flags, uint8_t* d_out, void* stream, rt_stats* stats) {
+    if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
+    return run_batch(s, n, flags, stream, stats, [&](bool count, unsigned long long* d_cnt, int grid, cudaStream_t st) {
+        launch_occluded(s->view, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, count, d_out, d_cnt, grid, s->stack_bytes, st);
+    });
+}
+
+int rt_occluded(const rt_scene* s, const rt_ray* rays, const double* t_max_per_ray, uint64_t n, double t_min, double t_max, uint32_t flags,
+                uint8_t* out, rt_stats* stats) {
+    if (!s || (n && (!rays || !out))) return set_err(RT_ERR_INVALID, "null argument");
+    if (n == 0) {
+        if (stats) std::memset(stats, 0, sizeof(*stats));
+        return RT_OK;
+    }
+    rt_ray* d_rays = nullptr;
+    double* d_tmax = nullptr;
+    uint8_t* d_out = nullptr;
+    int rc = RT_OK;
+    DeviceGuard guard;
+    try {
+        CU(cudaSetDevice(s->device));
+        scratch_alloc(&d_rays, n * sizeof(rt_ray));
+        scratch_alloc(&d_out, n);
+        CU(cudaMemcpy(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice));
+        if (t_max_per_ray) {
+            scratch_alloc(&d_tmax, n * sizeof(double));
+            CU(cudaMemcpy(d_tmax, t_max_per_ray, n * sizeof(double), cudaMemcpyHostToDevice));
+        }
+        rc = rt_occluded_device(s, d_rays, d_tmax, n, t_min, t_max, flags, d_out, nullptr, stats);
+        if (rc == RT_OK) {
+            CU(cudaDeviceSynchronize());
+            CU(cudaMemcpy(out, d_out, n, cudaMemcpyDeviceToHost));
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    scratch_free(d_rays);
+    scratch_free(d_tmax);
     scratch_free(d_out);
     return rc;
 }

@@ -1,4 +1,4 @@
-// kernels.cu — the wavefront path tracer and the closest-hit batch kernel (sm_100a).
+// kernels.cu — the wavefront path tracer and the closest-hit and occlusion batch kernels (sm_100a).
 //
 // Pipeline per iteration (all queues and counters live in HBM; no host round trip is needed to
 // size a launch — kernels are persistent grid-stride loops that read the counts themselves):
@@ -27,7 +27,7 @@
 namespace rt {
 
 // ------------------------------------------------------------------------------------------
-// closest-hit batch kernel (rt_closest_hit)
+// closest-hit and occlusion batch kernels (rt_closest_hit, rt_occluded)
 // ------------------------------------------------------------------------------------------
 struct RayArrayIO {  // rt_closest_hit batches: rays in, rt_hit out
     const SceneView& sv;
@@ -68,9 +68,32 @@ struct RayArrayIO {  // rt_closest_hit batches: rays in, rt_hit out
     }
 };
 
-template <bool COUNT, bool PARK, int WIDE, bool XF = true, int KINDS = 0>
-__global__ void __launch_bounds__(EXTEND_BLOCK, EXTEND_MIN_BLOCKS) k_closest_hit(SceneView sv, const rt_ray* __restrict__ rays, uint32_t n, double tmin,
-                                                                 double tmax, rt_hit* __restrict__ out, unsigned long long* counters) {
+struct OcclusionIO {  // rt_occluded batches: rays and per-ray t_max in, one byte out
+    const rt_ray* __restrict__ rays;
+    const double* __restrict__ tmax_per_ray;  // nullptr: `tmax` for every ray
+    uint8_t* __restrict__ out;
+    double tmin, tmax;
+    __device__ __forceinline__ double t_min() const { return tmin; }
+    __device__ __forceinline__ bool load(uint32_t i, RayD& r, double& t1, uint32_t& prim0, uint32_t& rank0) const {
+        const double* rp = reinterpret_cast<const double*>(rays + i);
+        r.o = D3{rp[0], rp[1], rp[2]};
+        r.d = D3{rp[3], rp[4], rp[5]};
+        r.time = rp[6];
+        t1 = tmax_per_ray ? tmax_per_ray[i] : tmax;
+        prim0 = 0xFFFFFFFFu, rank0 = 0xFFFFFFFFu;
+        if (!(tmin <= t1)) {  // an empty interval (t_max_i < t_min, or a NaN bound) contains no t: answered here, never traced
+            out[i] = 0;
+            return false;
+        }
+        return true;
+    }
+    __device__ __forceinline__ void prefetch(uint32_t i) const { asm volatile("prefetch.global.L2 [%0];" ::"l"(rays + i)); }
+    __device__ __forceinline__ void store(uint32_t i, bool hit, double, uint32_t, uint32_t) const { out[i] = hit ? 1 : 0; }
+};
+
+// The persistent traversal of a ray batch, shared by k_closest_hit (ANY = false) and k_occluded (ANY = true).
+template <bool COUNT, bool USE_RANK, bool PARK, int WIDE, bool XF, int KINDS, bool ANY, class IO>
+__device__ __forceinline__ void trace_batch(const SceneView& sv, IO& io, uint32_t n, unsigned long long* counters) {
     extern __shared__ float4 s_mem[];  // [cached nodes | traversal stacks | per-warp ray FIFOs]
     __shared__ uint32_t s_cursor;
     uint32_t* stack_base = reinterpret_cast<uint32_t*>(s_mem + cached_tree_float4(sv));
@@ -79,14 +102,36 @@ __global__ void __launch_bounds__(EXTEND_BLOCK, EXTEND_MIN_BLOCKS) k_closest_hit
     if (threadIdx.x == 0) s_cursor = 0;
     stage_nodes(sv, s_mem);
     TraceCounters cnt{0, 0};
-    RayArrayIO io{sv, rays, out, tmin, tmax};
     double* ray_s = reinterpret_cast<double*>(stack_base + sv.stack_entries * EXTEND_BLOCK + (EXTEND_BLOCK / 32) * sv.fifo_slots * FIFO_SLOT_WORDS) + threadIdx.x;
-    trace_persistent<COUNT, true, PARK, WIDE, XF, KINDS>(sv, io, n, &s_cursor, s_mem, stack, EXTEND_BLOCK, fifo, sv.fifo_slots, &cnt, ray_s);
+    trace_persistent<COUNT, USE_RANK, PARK, WIDE, XF, KINDS, ANY>(sv, io, n, &s_cursor, s_mem, stack, EXTEND_BLOCK, fifo, sv.fifo_slots, &cnt, ray_s);
     if (COUNT) {
         atomicAdd(&counters[0], (unsigned long long)cnt.nodes);
         atomicAdd(&counters[1], (unsigned long long)cnt.prims);
     }
 }
+
+template <bool COUNT, bool PARK, int WIDE, bool XF = true, int KINDS = 0>
+__global__ void __launch_bounds__(EXTEND_BLOCK, EXTEND_MIN_BLOCKS) k_closest_hit(SceneView sv, const rt_ray* __restrict__ rays, uint32_t n, double tmin,
+                                                                 double tmax, rt_hit* __restrict__ out, unsigned long long* counters) {
+    RayArrayIO io{sv, rays, out, tmin, tmax};
+    trace_batch<COUNT, true, PARK, WIDE, XF, KINDS, false>(sv, io, n, counters);
+}
+
+// any hit: the ray's traversal ends at the first primitive hit, whatever it is (no rank: any hit is the answer)
+template <bool COUNT, bool PARK, int WIDE, bool XF = true, int KINDS = 0>
+__global__ void __launch_bounds__(EXTEND_BLOCK, EXTEND_MIN_BLOCKS) k_occluded(SceneView sv, const rt_ray* __restrict__ rays, const double* __restrict__ tmax_per_ray,
+                                                              uint32_t n, double tmin, double tmax, uint8_t* __restrict__ out, unsigned long long* counters) {
+    OcclusionIO io{rays, tmax_per_ray, out, tmin, tmax};
+    trace_batch<COUNT, false, PARK, WIDE, XF, KINDS, true>(sv, io, n, counters);
+}
+
+// Every instantiation of a batch kernel family that batch_variant() can pick (kernel_setup opts them into the big shared memory).
+#define RT_BATCH_VARIANTS(K)                                                                                                            \
+    (const void*)K<false, false, 0>, (const void*)K<false, true, 0>, (const void*)K<false, true, 1>, (const void*)K<false, true, 2>,     \
+        (const void*)K<true, false, 0>, (const void*)K<true, true, 0>, (const void*)K<true, true, 1>, (const void*)K<true, true, 2>,     \
+        (const void*)K<false, false, 3>, (const void*)K<true, false, 3>, (const void*)K<false, true, 1, false, 0>,                      \
+        (const void*)K<true, true, 1, false, 0>, (const void*)K<false, true, 1, false, 1>, (const void*)K<true, true, 1, false, 1>,     \
+        (const void*)K<false, true, 1, false, 2>, (const void*)K<true, true, 1, false, 2>
 
 // Launch with the top of the BVH pinned in L2.  A scene whose nodes + primitives exceed the L2 makes almost every
 // warp-wide node visit wait for at least one lane's DRAM miss; nodes are stored breadth first, so a persisting
@@ -111,22 +156,43 @@ static void launch_with_l2_window(K kernel, const SceneView& sv, int grid, int b
     cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
-void launch_closest_hit(const SceneView& sv, const rt_ray* d_rays, uint32_t n, double tmin, double tmax, bool count, rt_hit* d_out,
-                        unsigned long long* d_counters, int grid, size_t stack_bytes, cudaStream_t stream) {  // stack_bytes = whole dynamic smem
+// The variant of a batch kernel family a scene runs: one choice for k_closest_hit and k_occluded.  F::get<COUNT, PARK, WIDE, XF,
+// KINDS>() names an instantiation of the family.
+template <class F>
+static auto batch_variant(const SceneView& sv, bool count) {
     // scenes without any Transform that hold one kind of primitive (a mesh, the soups) have variants without the detransform and
     // without the other primitive test
     auto soup = [&]() {
-        if (sv.kinds == 1) return count ? k_closest_hit<true, true, 1, false, 1> : k_closest_hit<false, true, 1, false, 1>;
-        if (sv.kinds == 2) return count ? k_closest_hit<true, true, 1, false, 2> : k_closest_hit<false, true, 1, false, 2>;
-        return count ? k_closest_hit<true, true, 1, false, 0> : k_closest_hit<false, true, 1, false, 0>;
+        if (sv.kinds == 1) return count ? F::template get<true, true, 1, false, 1>() : F::template get<false, true, 1, false, 1>();
+        if (sv.kinds == 2) return count ? F::template get<true, true, 1, false, 2>() : F::template get<false, true, 1, false, 2>();
+        return count ? F::template get<true, true, 1, false, 0>() : F::template get<false, true, 1, false, 0>();
     };
-    auto k = (sv.nodes4 && !sv.n_cached_nodes && !sv.n_xforms) ? soup()
-             : sv.nodes4 ? (sv.n_cached_nodes && !sv.fifo_slots ? (count ? k_closest_hit<true, true, 2> : k_closest_hit<false, true, 2>)
-                                            : (count ? k_closest_hit<true, true, 1> : k_closest_hit<false, true, 1>))
-             : (!sv.park_leaves && !sv.fifo_slots && sv.n_cached_nodes == sv.n_nodes) ? (count ? k_closest_hit<true, false, 3> : k_closest_hit<false, false, 3>)
-             : count   ? (sv.park_leaves ? k_closest_hit<true, true, 0> : k_closest_hit<true, false, 0>)
-                       : (sv.park_leaves ? k_closest_hit<false, true, 0> : k_closest_hit<false, false, 0>);
-    launch_with_l2_window(k, sv, grid, EXTEND_BLOCK, stack_bytes, stream, sv, d_rays, n, tmin, tmax, d_out, d_counters);
+    return (sv.nodes4 && !sv.n_cached_nodes && !sv.n_xforms) ? soup()
+           : sv.nodes4 ? (sv.n_cached_nodes && !sv.fifo_slots ? (count ? F::template get<true, true, 2>() : F::template get<false, true, 2>())
+                                                              : (count ? F::template get<true, true, 1>() : F::template get<false, true, 1>()))
+           : (!sv.park_leaves && !sv.fifo_slots && sv.n_cached_nodes == sv.n_nodes) ? (count ? F::template get<true, false, 3>() : F::template get<false, false, 3>())
+           : count ? (sv.park_leaves ? F::template get<true, true, 0>() : F::template get<true, false, 0>())
+                   : (sv.park_leaves ? F::template get<false, true, 0>() : F::template get<false, false, 0>());
+}
+struct ClosestHitKernels {
+    template <bool COUNT, bool PARK, int WIDE, bool XF = true, int KINDS = 0>
+    static auto get() { return k_closest_hit<COUNT, PARK, WIDE, XF, KINDS>; }
+};
+struct OccludedKernels {
+    template <bool COUNT, bool PARK, int WIDE, bool XF = true, int KINDS = 0>
+    static auto get() { return k_occluded<COUNT, PARK, WIDE, XF, KINDS>; }
+};
+
+void launch_closest_hit(const SceneView& sv, const rt_ray* d_rays, uint32_t n, double tmin, double tmax, bool count, rt_hit* d_out,
+                        unsigned long long* d_counters, int grid, size_t stack_bytes, cudaStream_t stream) {  // stack_bytes = whole dynamic smem
+    launch_with_l2_window(batch_variant<ClosestHitKernels>(sv, count), sv, grid, EXTEND_BLOCK, stack_bytes, stream, sv, d_rays, n, tmin, tmax, d_out,
+                          d_counters);
+}
+
+void launch_occluded(const SceneView& sv, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax, bool count,
+                     uint8_t* d_out, unsigned long long* d_counters, int grid, size_t stack_bytes, cudaStream_t stream) {
+    launch_with_l2_window(batch_variant<OccludedKernels>(sv, count), sv, grid, EXTEND_BLOCK, stack_bytes, stream, sv, d_rays, d_tmax_per_ray, n, tmin,
+                          tmax, d_out, d_counters);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1473,12 +1539,7 @@ int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks
         (const void*)k_extend<true, false, 3, M>
         RT_EXTEND_VARIANTS(0), RT_EXTEND_VARIANTS(1), RT_EXTEND_VARIANTS(2), RT_EXTEND_VARIANTS(3),
 #undef RT_EXTEND_VARIANTS
-        (const void*)k_closest_hit<false, false, 0>, (const void*)k_closest_hit<false, true, 0>, (const void*)k_closest_hit<false, true, 1>,
-        (const void*)k_closest_hit<false, true, 2>,  (const void*)k_closest_hit<true, false, 0>, (const void*)k_closest_hit<true, true, 0>,
-        (const void*)k_closest_hit<true, true, 1>,   (const void*)k_closest_hit<true, true, 2>,  (const void*)k_closest_hit<false, false, 3>,
-        (const void*)k_closest_hit<true, false, 3>,  (const void*)k_closest_hit<false, true, 1, false, 0>,  (const void*)k_closest_hit<true, true, 1, false, 0>,
-        (const void*)k_closest_hit<false, true, 1, false, 1>,  (const void*)k_closest_hit<true, true, 1, false, 1>,
-        (const void*)k_closest_hit<false, true, 1, false, 2>,  (const void*)k_closest_hit<true, true, 1, false, 2>};
+        RT_BATCH_VARIANTS(k_closest_hit), RT_BATCH_VARIANTS(k_occluded)};
     for (const void* f : big_smem)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(EXTEND_SMEM_MAX - 1024))) != cudaSuccess) return (int)e;
     // the general-boundary media pass: TRAVERSAL_STACK entries per thread is 64 KB

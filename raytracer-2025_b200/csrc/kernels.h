@@ -139,6 +139,9 @@ struct RenderParams {
 
 void launch_closest_hit(const SceneView& sv, const rt_ray* d_rays, uint32_t n, double tmin, double tmax, bool count, rt_hit* d_out,
                         unsigned long long* d_counters, int grid, size_t smem_bytes, cudaStream_t stream);
+// d_out[i] = 1 when a surface hit lies in [tmin, d_tmax_per_ray ? d_tmax_per_ray[i] : tmax]; the same variant as launch_closest_hit
+void launch_occluded(const SceneView& sv, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax, bool count,
+                     uint8_t* d_out, unsigned long long* d_counters, int grid, size_t smem_bytes, cudaStream_t stream);
 void launch_init(const WavefrontState& W, const RenderParams& P, int grid, cudaStream_t s);
 void launch_generate(const SceneView& sv, const RenderParams& P, const WavefrontState& W, int grid, cudaStream_t s);
 void launch_extend(const SceneView& sv, const RenderParams& P, const WavefrontState& W, bool count, int grid, size_t smem_bytes, cudaStream_t s);

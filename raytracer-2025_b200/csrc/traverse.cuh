@@ -465,7 +465,8 @@ __device__ __forceinline__ bool leaf_beats_scatter(const SceneView& sv, uint32_t
 // than they save, so rt_scene_create picks per scene (SceneView::park_leaves).
 //
 // IO::load(item, ray, tmax, prim0, rank0) -> bool, IO::t_min() and IO::store(item, hit, t, prim) bind the routine
-// to the path streams (k_extend) or to a plain ray array (k_closest_hit).
+// to the path streams (k_extend) or to a plain ray array (k_closest_hit, k_occluded).  An item whose load returns false is
+// dropped without a store.
 // ------------------------------------------------------------------------------------------------
 constexpr uint32_t FIFO_SLOT_WORDS = 28;
 constexpr uint32_t FIFO_INVALID_ITEM = 0xFFFFFFFFu;  // a slot of the ragged last group: popped and dropped
@@ -478,7 +479,10 @@ constexpr uint32_t FIFO_INVALID_ITEM = 0xFFFFFFFFu;  // a slot of the ragged las
 // shared memory, likewise without the global-memory path)
 // XF = false: the scene has no Transform at all (the soups): no local-space copy of the ray, no detransform code.
 // KINDS: 0 = any primitives, 1 = the scene holds spheres only, 2 = quads / triangles only (a mesh, the soups): the other test is compiled out.
-template <bool COUNT, bool USE_RANK, bool PARK, int WIDE, bool XF, int KINDS, class IO>
+// ANY = any-hit (occlusion): the first primitive test that hits within [tmin, tmax] ends the lane's traversal - its parked leaf,
+// the rest of the current leaf and its stack are dropped - and store() is called with hit = true.  The interval never shrinks, so
+// no rank, kind or binary32 bound is kept.
+template <bool COUNT, bool USE_RANK, bool PARK, int WIDE, bool XF, int KINDS, bool ANY = false, class IO>
 __device__ __forceinline__ void trace_persistent(const SceneView& sv, IO& io, uint32_t n, uint32_t* s_cursor,
                                                  const float4* __restrict__ smem_nodes, uint32_t* __restrict__ stack, int stride,
                                                  uint32_t* __restrict__ fifo, uint32_t fifo_slots_arg, TraceCounters* cnt, double* __restrict__ ray_s = nullptr) {
@@ -783,7 +787,13 @@ __device__ __forceinline__ void trace_persistent(const SceneView& sv, IO& io, ui
                                : KINDS == 2 ? planar_hit(g, kind == PRIM_TRIANGLE, tr, tmin, tbest, t)
                                : kind == PRIM_SPHERE ? sphere_hit(g, tr, tmin, tbest, t) : planar_hit(g, kind == PRIM_TRIANGLE, tr, tmin, tbest, t);
                     if (COUNT) cnt->prims++;
-                    if (hit && (prim == 0xFFFFFFFFu || t < tbest || (USE_RANK && km.y < prim_rank))) {
+                    if (ANY) {
+                        if (hit) {
+                            prim = pi;
+                            cur = INVALID_REF;  // with parked = INVALID_REF below: the traversal is finished
+                            break;
+                        }
+                    } else if (hit && (prim == 0xFFFFFFFFu || t < tbest || (USE_RANK && km.y < prim_rank))) {
                         tbest = t;
                         prim = pi;
                         prim_rank = km.y;
