@@ -311,7 +311,7 @@ int rt_closest_hit_device(const rt_scene* scene, const rt_ray* d_rays, uint64_t 
  *              (inclusive at both ends, utils/interval.rs:65-67), else 0.
  * This is geometric visibility: every surface occludes whatever its material (Dielectric,
  * Transparent, Portal and emitters alike); media are excluded as in rt_closest_hit and no
- * transmittance is computed.  An empty interval (t_max_i < t_min, or a NaN bound) gives 0.
+ * transmittance is computed (rt_transmittance below does).  An empty interval (t_max_i < t_min, or a NaN bound) gives 0.
  * With the same primitive arithmetic as rt_closest_hit, bit for bit:
  *     out[i] == (closest_hit(ray, t_min, +inf).prim_id != RT_NONE && .t <= t_max_i)
  * A ray's traversal ends at the first hit found, so it visits at most the nodes and primitives
@@ -323,6 +323,30 @@ int rt_occluded(const rt_scene* scene, const rt_ray* rays, const double* t_max_p
 int rt_occluded_device(const rt_scene* scene, const rt_ray* d_rays, const double* d_t_max_per_ray,
                        uint64_t n, double t_min, double t_max, uint32_t flags, uint8_t* d_out,
                        void* stream, rt_stats* stats);
+
+/* Transmittance (visibility through media) for a batch of rays over `world`: out[i] (binary64) is
+ * the probability that world.hit(ray, [t_min, t_max_i]) returns None when every ConstantMedium
+ * draws its own uniform number, with t_max_i as in rt_occluded:
+ *   - an empty interval (t_max_i < t_min, or a NaN bound) gives 1.0 (the ray is not traced);
+ *   - where rt_occluded with the same arguments gives 1 the result is 0.0 exactly (every surface
+ *     blocks whatever its material);
+ *   - otherwise the product, in ascending medium order, of exp(L_m / neg_inv_density_m) over all
+ *     media, where L_m is the distance_inside_boundary of ConstantMedium::hit (volume.rs:42-58) on
+ *     [t_min, t_max_i]: t1 = boundary.hit(r, UNIVERSE), t2 = boundary.hit(r, [t1 + 1e-4, inf))
+ *     (factor 1 if either misses), t1 clamped up to t_min and t2 down to t_max_i (factor 1 if
+ *     t1 >= t2), t1 = max(t1, 0), L = (t2 - t1) * |d| with d the direction in the medium's space.
+ * Density 0 gives a factor 1, an infinite density a factor 0 wherever L > 0; neither is special-
+ * cased.  T == 0 with rt_occluded == 0 happens only by underflow or through an infinite density.
+ * Two launches: the occlusion pass of rt_occluded into a stream-ordered scratch buffer, then one
+ * media pass.  `stats` gets segments = n, kernel_launches = 2 and ms_total over both, and with
+ * RT_OPT_COUNT node_visits / prim_tests summed over both passes (a sphere boundary counts 2
+ * primitive tests).  Host-pointer version copies in and out; the _device version takes device
+ * pointers (t_max_per_ray may be NULL) and enqueues on `stream`. */
+int rt_transmittance(const rt_scene* scene, const rt_ray* rays, const double* t_max_per_ray /* n values or NULL */,
+                     uint64_t n, double t_min, double t_max, uint32_t flags, double* out, rt_stats* stats);
+int rt_transmittance_device(const rt_scene* scene, const rt_ray* d_rays, const double* d_t_max_per_ray,
+                            uint64_t n, double t_min, double t_max, uint32_t flags, double* d_out,
+                            void* stream, rt_stats* stats);
 
 typedef enum rt_accum_type { RT_ACCUM_F32 = 0, RT_ACCUM_F64 = 1 } rt_accum_type;
 

@@ -254,7 +254,7 @@ int check_device(int requested, int& device, int& sm_count) {
 }
 
 // The body of the _device batch queries: the batch size check, RT_OPT_COUNT counters, event timing and `stats`.
-// launch(count, d_counters, grid, stream) enqueues the kernel.
+// launch(count, d_counters, grid, stream) enqueues the kernels and returns how many it launched.
 template <class Launch>
 int run_batch(const rt_scene* s, uint64_t n, uint32_t flags, void* stream, rt_stats* stats, Launch launch) {
     if (stats) std::memset(stats, 0, sizeof(*stats));
@@ -282,7 +282,7 @@ int run_batch(const rt_scene* s, uint64_t n, uint32_t flags, void* stream, rt_st
             CU(cudaEventCreate(&e1));
             CU(cudaEventRecord(e0, st));
         }
-        launch(count, d_cnt, grid, st);
+        const int launches = launch(count, d_cnt, grid, st);
         CU(cudaGetLastError());
         if (stats) {
             CU(cudaEventRecord(e1, st));
@@ -292,7 +292,7 @@ int run_batch(const rt_scene* s, uint64_t n, uint32_t flags, void* stream, rt_st
             stats->ms_total = ms;
             stats->ms_extend = ms;
             stats->segments = n;
-            stats->kernel_launches = 1;
+            stats->kernel_launches = launches;
             if (count) {
                 unsigned long long h[2];
                 CU(cudaMemcpyAsync(h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
@@ -539,6 +539,7 @@ int rt_closest_hit_device(const rt_scene* s, const rt_ray* d_rays, uint64_t n, d
     if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
     return run_batch(s, n, flags, stream, stats, [&](bool count, unsigned long long* d_cnt, int grid, cudaStream_t st) {
         launch_closest_hit(s->view, d_rays, (uint32_t)n, t_min, t_max, count, d_out, d_cnt, grid, s->stack_bytes, st);
+        return 1;
     });
 }
 
@@ -576,6 +577,7 @@ int rt_occluded_device(const rt_scene* s, const rt_ray* d_rays, const double* d_
     if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
     return run_batch(s, n, flags, stream, stats, [&](bool count, unsigned long long* d_cnt, int grid, cudaStream_t st) {
         launch_occluded(s->view, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, count, d_out, d_cnt, grid, s->stack_bytes, st);
+        return 1;
     });
 }
 
@@ -604,6 +606,58 @@ int rt_occluded(const rt_scene* s, const rt_ray* rays, const double* t_max_per_r
         if (rc == RT_OK) {
             CU(cudaDeviceSynchronize());
             CU(cudaMemcpy(out, d_out, n, cudaMemcpyDeviceToHost));
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    scratch_free(d_rays);
+    scratch_free(d_tmax);
+    scratch_free(d_out);
+    return rc;
+}
+
+int rt_transmittance_device(const rt_scene* s, const rt_ray* d_rays, const double* d_t_max_per_ray, uint64_t n, double t_min, double t_max,
+                            uint32_t flags, double* d_out, void* stream, rt_stats* stats) {
+    if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
+    return run_batch(s, n, flags, stream, stats, [&](bool count, unsigned long long* d_cnt, int grid, cudaStream_t st) {
+        // the surface pass writes one occlusion byte per ray to a stream-ordered scratch buffer; the media pass reads it
+        uint8_t* d_occ = nullptr;
+        CU(cudaMallocAsync((void**)&d_occ, n, st));
+        launch_occluded(s->view, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, count, d_occ, d_cnt, grid, s->stack_bytes, st);
+        int grid_m = s->sm_count * 8;
+        const uint64_t need = (n + MEDIA_BLOCK - 1) / MEDIA_BLOCK;
+        if ((uint64_t)grid_m > need) grid_m = (int)need;
+        launch_transmittance(s->view, s->generic_media, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, count, d_occ, d_out, d_cnt, grid_m, st);
+        CU(cudaFreeAsync(d_occ, st));
+        return 2;
+    });
+}
+
+int rt_transmittance(const rt_scene* s, const rt_ray* rays, const double* t_max_per_ray, uint64_t n, double t_min, double t_max,
+                     uint32_t flags, double* out, rt_stats* stats) {
+    if (!s || (n && (!rays || !out))) return set_err(RT_ERR_INVALID, "null argument");
+    if (n == 0) {
+        if (stats) std::memset(stats, 0, sizeof(*stats));
+        return RT_OK;
+    }
+    rt_ray* d_rays = nullptr;
+    double* d_tmax = nullptr;
+    double* d_out = nullptr;
+    int rc = RT_OK;
+    DeviceGuard guard;
+    try {
+        CU(cudaSetDevice(s->device));
+        scratch_alloc(&d_rays, n * sizeof(rt_ray));
+        scratch_alloc(&d_out, n * sizeof(double));
+        CU(cudaMemcpy(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice));
+        if (t_max_per_ray) {
+            scratch_alloc(&d_tmax, n * sizeof(double));
+            CU(cudaMemcpy(d_tmax, t_max_per_ray, n * sizeof(double), cudaMemcpyHostToDevice));
+        }
+        rc = rt_transmittance_device(s, d_rays, d_tmax, n, t_min, t_max, flags, d_out, nullptr, stats);
+        if (rc == RT_OK) {
+            CU(cudaDeviceSynchronize());
+            CU(cudaMemcpy(out, d_out, n * sizeof(double), cudaMemcpyDeviceToHost));
         }
     } catch (const CudaFail& f) {
         rc = set_err(RT_ERR_CUDA, f.what);

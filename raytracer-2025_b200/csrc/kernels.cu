@@ -338,21 +338,45 @@ __device__ __forceinline__ bool free_flight_overshoots(double neg_inv_density, d
     return hf > (float)t * len_f * 1.001f + hf_err;
 }
 
+// The ray in a medium's space (Medium::xform): ConstantMedium::hit measures ray_length on it (volume.rs:55).  XF: the
+// medium may sit under a Transform.
+template <bool XF>
+__device__ __forceinline__ void medium_ray(const SceneView& sv, const Medium& med, const RayD& r, RayD& lr) {
+    lr = r;
+    if (XF && med.xform != RT_NONE) lr = ray_to_local(sv, med.xform, r);
+}
+
+// The two boundary hits of ConstantMedium::hit (volume.rs:42-45): t1 = boundary.hit(r, UNIVERSE), then
+// t2 = boundary.hit(r, [t1 + 1e-4, inf)); false when either misses.  lr = medium_ray(r).
+//   SPHERE: the boundary is the single Sphere med.single_sphere; one fused entry/exit test (2 primitive tests) on the
+//   sphere's local ray, which is lr unless the sphere sits under a Transform of its own (XF).
+//   Otherwise two closest-hit traversals of the boundary group, global nodes only, stacks at `stack` (stride apart).
+template <bool COUNT, bool SPHERE, bool XF>
+__device__ __forceinline__ bool medium_boundary_hits(const SceneView& sv, const Medium& med, const RayD& r, const RayD& lr, const float4* s_mem,
+                                                     uint32_t* stack, int stride, double& t1, double& t2, TraceCounters* cnt) {
+    if (SPHERE) {
+        RayD br = lr;
+        if (XF) {
+            const uint32_t bx = sv.meta[med.single_sphere].xform;
+            if (bx != med.xform) br = bx == RT_NONE ? r : ray_to_local(sv, bx, r);
+        }
+        if (COUNT) cnt->prims += 2;
+        return sphere_entry_exit(sv.geom[med.single_sphere].d, br, t1, t2);
+    }
+    uint32_t bp;
+    if (!closest_hit<COUNT, false>(sv, med.root, r, -INFINITY, INFINITY, s_mem, stack, stride, t1, bp, cnt)) return false;
+    return closest_hit<COUNT, false>(sv, med.root, r, t1 + 0.0001, INFINITY, s_mem, stack, stride, t2, bp, cnt);
+}
+
 // ConstantMedium::hit (volume.rs:37-73) for a medium whose boundary is a single Sphere, on the caller's interval
 // [1e-8, inf): true and the scatter distance when the path scatters inside.  XF: the medium or its sphere may sit
 // under a Transform.
 template <bool COUNT, bool XF>
 __device__ __forceinline__ bool sample_sphere_medium(const SceneView& sv, const Medium& med, const RayD& r, double xi, double& tm, TraceCounters* cnt) {
-    RayD lr = r;
-    if (XF && med.xform != RT_NONE) lr = ray_to_local(sv, med.xform, r);
-    RayD br = lr;
-    if (XF) {
-        const uint32_t bx = sv.meta[med.single_sphere].xform;
-        if (bx != med.xform) br = bx == RT_NONE ? r : ray_to_local(sv, bx, r);
-    }
+    RayD lr;
+    medium_ray<XF>(sv, med, r, lr);
     double t1, t2;
-    if (COUNT) cnt->prims += 2;
-    if (!sphere_entry_exit(sv.geom[med.single_sphere].d, br, t1, t2)) return false;
+    if (!medium_boundary_hits<COUNT, true, XF>(sv, med, r, lr, nullptr, nullptr, 0, t1, t2, cnt)) return false;
     return medium_free_flight(t1, t2, lr, med.neg_inv_density, xi, tm);
 }
 
@@ -469,17 +493,15 @@ __device__ __forceinline__ bool sample_media(const SceneView& sv, uint64_t seed,
             const Medium& med = sv.media[m];
             const double xi = draws.get(seed, pixel, sample, segment, med.medium_index);
             double tm;
-            RayD lr = r;
-            if (XF && med.xform != RT_NONE) lr = ray_to_local(sv, med.xform, r);
+            RayD lr;
+            medium_ray<XF>(sv, med, r, lr);
             // skip the boundary test of a medium that cannot beat the known hit
             if (RT_MEDIA_EARLY_SCREEN && kind != HIT_MISS && free_flight_overshoots(med.neg_inv_density, xi, t, lr.d)) continue;
             if (med.single_sphere != RT_NONE) {
                 if (!sample_sphere_medium<COUNT, XF>(sv, med, r, xi, tm, cntp)) continue;
             } else if (GENERIC) {
                 double t1, t2;
-                uint32_t bp;
-                if (!closest_hit<COUNT, false>(sv, med.root, r, -INFINITY, INFINITY, s_mem, stack, stride, t1, bp, cntp)) continue;
-                if (!closest_hit<COUNT, false>(sv, med.root, r, t1 + 0.0001, INFINITY, s_mem, stack, stride, t2, bp, cntp)) continue;
+                if (!medium_boundary_hits<COUNT, false, XF>(sv, med, r, lr, s_mem, stack, stride, t1, t2, cntp)) continue;
                 if (t1 < 1e-8) t1 = 1e-8;  // clamp to the caller's interval [1e-8, inf)
                 if (t1 >= t2) continue;
                 if (t1 < 0.0) t1 = 0.0;
@@ -632,6 +654,60 @@ __global__ void __launch_bounds__(MEDIA_BLOCK, MODE == 2 ? RT_MEDIA_GENERIC_MIN_
     if (COUNT) {
         atomicAdd(&W.counters->node_visits, (unsigned long long)cnt.nodes);
         atomicAdd(&W.counters->prim_tests, (unsigned long long)cnt.prims);
+    }
+}
+
+// rt_transmittance's media pass, after k_occluded left the surface answer of every ray in `occluded`: one ray per thread.
+// An occluded ray gets 0 (its ray record is not read), an empty interval 1, every other ray the product over the media, in
+// medium order, of the probability that ConstantMedium::hit (volume.rs:37-73) returns None on the caller's interval
+// [tmin, t_max_i]: exp(distance_inside_boundary / neg_inv_density).  GENERIC / XF as MODE 2 / XF of k_media.
+template <bool COUNT, bool GENERIC, bool XF>
+__global__ void __launch_bounds__(MEDIA_BLOCK) k_transmittance(SceneView sv, const rt_ray* __restrict__ rays, const double* __restrict__ tmax_per_ray,
+                                                             uint32_t n, double tmin, double tmax, const uint8_t* __restrict__ occluded,
+                                                             double* __restrict__ out, unsigned long long* counters) {
+    extern __shared__ float4 s_mem[];  // traversal stacks for boundaries that are not a single sphere
+    uint32_t* stack = reinterpret_cast<uint32_t*>(s_mem) + threadIdx.x;
+    TraceCounters cnt{0, 0};
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        if (occluded[i]) {
+            out[i] = 0.0;
+            continue;
+        }
+        const double t_max_i = tmax_per_ray ? tmax_per_ray[i] : tmax;
+        if (!(tmin <= t_max_i)) {  // an empty interval (t_max_i < t_min, or a NaN bound): nothing in it can stop the ray
+            out[i] = 1.0;
+            continue;
+        }
+        const double* rp = reinterpret_cast<const double*>(rays + i);
+        RayD r;
+        r.o = D3{rp[0], rp[1], rp[2]};
+        r.d = D3{rp[3], rp[4], rp[5]};
+        r.time = rp[6];
+        double T = 1.0;
+        for (uint32_t m = 0; m < sv.n_media; m++) {
+            const Medium& med = sv.media[m];
+            RayD lr;
+            medium_ray<XF>(sv, med, r, lr);
+            double t1, t2;
+            if (med.single_sphere != RT_NONE) {
+                if (!medium_boundary_hits<COUNT, true, XF>(sv, med, r, lr, s_mem, stack, MEDIA_BLOCK, t1, t2, &cnt)) continue;
+            } else if (GENERIC) {
+                if (!medium_boundary_hits<COUNT, false, XF>(sv, med, r, lr, s_mem, stack, MEDIA_BLOCK, t1, t2, &cnt)) continue;
+            } else {
+                continue;  // unreachable: the host launches the GENERIC instantiation for such scenes
+            }
+            if (t1 < tmin) t1 = tmin;  // clamp_min_assign / clamp_max_assign to the caller's interval
+            if (t2 > t_max_i) t2 = t_max_i;
+            if (t1 >= t2) continue;
+            if (t1 < 0.0) t1 = 0.0;
+            const double distance_inside_boundary = (t2 - t1) * length(lr.d);
+            T *= exp(distance_inside_boundary / med.neg_inv_density);
+        }
+        out[i] = T;
+    }
+    if (COUNT) {
+        atomicAdd(&counters[0], (unsigned long long)cnt.nodes);
+        atomicAdd(&counters[1], (unsigned long long)cnt.prims);
     }
 }
 
@@ -1470,6 +1546,18 @@ int launch_media_bin(const SceneView& sv, const RenderParams& P, const Wavefront
     k_bin<<<grid, MEDIA_BLOCK, 0, s>>>(W);
     return launches;
 }
+void launch_transmittance(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax,
+                          bool count, const uint8_t* d_occluded, double* d_out, unsigned long long* d_counters, int grid, cudaStream_t s) {
+    SceneView mv = sv;  // global-memory nodes only, as the media pass of the render (its shared memory holds just the stacks)
+    mv.n_cached_nodes = 0;
+    const size_t media_smem = generic ? (size_t)sv.media_stack_entries * MEDIA_BLOCK * sizeof(uint32_t) : 0;  // <= 64 KB, opted in by kernel_setup
+    const bool xf = sv.media_xform != 0;
+    auto k = generic ? (count ? (xf ? k_transmittance<true, true, true> : k_transmittance<true, true, false>)
+                              : (xf ? k_transmittance<false, true, true> : k_transmittance<false, true, false>))
+                     : (count ? (xf ? k_transmittance<true, false, true> : k_transmittance<true, false, false>)
+                              : (xf ? k_transmittance<false, false, true> : k_transmittance<false, false, false>));
+    k<<<grid, MEDIA_BLOCK, media_smem, s>>>(mv, d_rays, d_tmax_per_ray, n, tmin, tmax, d_occluded, d_out, d_counters);
+}
 template <uint32_t CLS>
 static void launch_shade_cls(const SceneView& sv, const RenderParams& P, const WavefrontState& W, uint32_t queue, int grid, cudaStream_t s) {
     // `grid` is sized for RT_SHADE_MIN_BLOCKS resident CTAs per SM; classes compiled for another count get the matching grid
@@ -1547,7 +1635,9 @@ int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks
     for (const void* f : {(const void*)k_walk<false, false>, (const void*)k_walk<true, false>, (const void*)k_walk<false, true>, (const void*)k_walk<true, true>})
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, TRAVERSAL_STACK * WALK_BLOCK * (int)sizeof(uint32_t))) != cudaSuccess) return (int)e;
     const void* media_smem[] = {(const void*)k_media<false, 2, false, false>, (const void*)k_media<false, 2, true, false>,
-                                (const void*)k_media<true, 2, false, false>, (const void*)k_media<true, 2, true, false>};
+                                (const void*)k_media<true, 2, false, false>, (const void*)k_media<true, 2, true, false>,
+                                (const void*)k_transmittance<false, true, false>, (const void*)k_transmittance<false, true, true>,
+                                (const void*)k_transmittance<true, true, false>, (const void*)k_transmittance<true, true, true>};
     for (const void* f : media_smem)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, TRAVERSAL_STACK * MEDIA_BLOCK * (int)sizeof(uint32_t))) != cudaSuccess) return (int)e;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(extend_blocks_per_sm, k_extend<false, false, 0, 0>, EXTEND_BLOCK, smem_bytes);

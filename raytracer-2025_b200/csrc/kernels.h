@@ -142,6 +142,11 @@ void launch_closest_hit(const SceneView& sv, const rt_ray* d_rays, uint32_t n, d
 // d_out[i] = 1 when a surface hit lies in [tmin, d_tmax_per_ray ? d_tmax_per_ray[i] : tmax]; the same variant as launch_closest_hit
 void launch_occluded(const SceneView& sv, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax, bool count,
                      uint8_t* d_out, unsigned long long* d_counters, int grid, size_t smem_bytes, cudaStream_t stream);
+// The media pass of rt_transmittance, after launch_occluded wrote d_occluded: d_out[i] = 0 for an occluded ray, else the product
+// of exp(L / neg_inv_density) over the media on [tmin, t_max_i] (1 for an empty interval).  generic: some boundary is not a single
+// Sphere.  `grid` CTAs of MEDIA_BLOCK threads.
+void launch_transmittance(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax,
+                          bool count, const uint8_t* d_occluded, double* d_out, unsigned long long* d_counters, int grid, cudaStream_t s);
 void launch_init(const WavefrontState& W, const RenderParams& P, int grid, cudaStream_t s);
 void launch_generate(const SceneView& sv, const RenderParams& P, const WavefrontState& W, int grid, cudaStream_t s);
 void launch_extend(const SceneView& sv, const RenderParams& P, const WavefrontState& W, bool count, int grid, size_t smem_bytes, cudaStream_t s);

@@ -23,7 +23,8 @@ RT_BUILD_DEVICE_LBVH = 2
 
 # every symbol include/rt2025.h declares (tests check that the library exports them all)
 ABI_SYMBOLS = [
-    "rt_scene_create", "rt_scene_destroy", "rt_closest_hit", "rt_closest_hit_device", "rt_occluded", "rt_occluded_device", "rt_render",
+    "rt_scene_create", "rt_scene_destroy", "rt_closest_hit", "rt_closest_hit_device", "rt_occluded", "rt_occluded_device", "rt_transmittance",
+    "rt_transmittance_device", "rt_render",
     "rt_render_device", "rt_render_rgb8", "rt_render_multi", "rt_render_multi_rgb8", "rt_tonemap", "rt_tonemap_device", "rt_scene_get_info", "rt_scene_get_ranks", "rt_last_error",
     "rt_abi_version", "rt_device_count",
 ]
@@ -219,6 +220,11 @@ def product_lib(required=True):
                                       C.c_void_p, C.POINTER(rt_stats)]
             L.rt_occluded_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint32,
                                              C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+        if hasattr(L, "rt_transmittance"):  # absent from older builds selected with RT2025_LIB for A/B runs
+            L.rt_transmittance.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint32,
+                                           C.c_void_p, C.POINTER(rt_stats)]
+            L.rt_transmittance_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint32,
+                                                  C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
         L.rt_render.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
                                 C.POINTER(rt_stats)]
         L.rt_render_device.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
@@ -463,6 +469,29 @@ class Scene:
         """rt_occluded_device: n bytes at d_out_ptr; d_t_max_ptr (n doubles) overrides the scalar t_max."""
         st = rt_stats()
         _check(self.L.rt_occluded_device(self.h, d_rays_ptr, d_t_max_ptr, n, t_min, t_max, flags, d_out_ptr, stream, C.byref(st)), self.L)
+        return st
+
+    def transmittance(self, rays, t_min=1e-8, t_max=float("inf"), flags=0):
+        """rt_transmittance: for each ray, the probability that nothing in [t_min, t_max] stops it - 0 behind a surface, else the
+        product of the media's exp(L / neg_inv_density).  `t_max` is a scalar or one value per ray.  Returns (float64 array, stats)."""
+        rays = np.ascontiguousarray(rays, dtype=rt_ray_dtype)
+        out = np.empty(len(rays), dtype=np.float64)
+        per_ray = None
+        if np.ndim(t_max) != 0:
+            per_ray = np.ascontiguousarray(t_max, dtype=np.float64)
+            if per_ray.shape != (len(rays),):
+                raise ValueError(f"t_max has shape {per_ray.shape}; a scalar or {len(rays)} values expected")
+            t_max = float("inf")
+        st = rt_stats()
+        _check(self.L.rt_transmittance(self.h, rays.ctypes.data, None if per_ray is None else per_ray.ctypes.data, len(rays), t_min, t_max,
+                                       flags, out.ctypes.data, C.byref(st)), self.L)
+        return out, st
+
+    def transmittance_device(self, d_rays_ptr, n, d_out_ptr, d_t_max_ptr=None, t_min=1e-8, t_max=float("inf"), flags=0, stream=None):
+        """rt_transmittance_device: n doubles at d_out_ptr; d_t_max_ptr (n doubles) overrides the scalar t_max."""
+        st = rt_stats()
+        _check(self.L.rt_transmittance_device(self.h, d_rays_ptr, d_t_max_ptr, n, t_min, t_max, flags, d_out_ptr, stream, C.byref(st)),
+               self.L)
         return st
 
     def render_opts(self, seed=1, accum_type=RT_ACCUM_F64, part_index=0, part_count=1, sample_begin=0, sample_end=0,

@@ -114,6 +114,8 @@ extern "C" {
     pub fn rt_closest_hit(scene: *const rt_scene, rays: *const rt_ray, n: u64, t_min: f64, t_max: f64, flags: u32, out: *mut rt_hit, stats: *mut rt_stats) -> i32;
     pub fn rt_occluded(scene: *const rt_scene, rays: *const rt_ray, t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, out: *mut u8, stats: *mut rt_stats) -> i32;
     pub fn rt_occluded_device(scene: *const rt_scene, d_rays: *const rt_ray, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, d_out: *mut u8, stream: *mut c_void, stats: *mut rt_stats) -> i32;
+    pub fn rt_transmittance(scene: *const rt_scene, rays: *const rt_ray, t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, out: *mut f64, stats: *mut rt_stats) -> i32;
+    pub fn rt_transmittance_device(scene: *const rt_scene, d_rays: *const rt_ray, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, d_out: *mut f64, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, accum: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_device(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, d_accum: *mut c_void, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_rgb8(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, rgb: *mut u8, stats: *mut rt_stats) -> i32;
