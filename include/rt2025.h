@@ -348,6 +348,53 @@ int rt_transmittance_device(const rt_scene* scene, const rt_ray* d_rays, const d
                             uint64_t n, double t_min, double t_max, uint32_t flags, double* d_out,
                             void* stream, rt_stats* stats);
 
+/* World hit: the HitRecord world.hit(ray, Interval(t_min, t_max_i)) returns (camera.rs:286, hit.rs:9-60),
+ * media included, for a batch of rays over `world`, with t_max_i as in rt_occluded.
+ *   - Draws: the ConstantMedium of media[m] draws philox(seed; pixel = i, sample = 0, segment,
+ *     RT_MEDIUM_SLOT(m)), component a for even m and b for odd m, as the renderer does.  The same
+ *     (seed, segment) reproduces a batch bit for bit; a client path loop passes its bounce number as
+ *     `segment`.
+ *   - Interval: surfaces use Interval::contains (inclusive at both ends).  A medium runs
+ *     ConstantMedium::hit (volume.rs:37-73) on [t_min, t_max_i]: t1 = boundary.hit(r, UNIVERSE),
+ *     t2 = boundary.hit(r, [t1 + 1e-4, inf)), t1 clamped up to t_min and t2 down to t_max_i (no hit
+ *     if t1 >= t2), t1 = max(t1, 0), then t = t1 + hit_distance / |d| with d the direction in the
+ *     medium's space, when hit_distance = neg_inv_density * ln(xi) <= (t2 - t1) * |d|.
+ *   - Winner: the smallest t; an exact tie goes to the lower tie rank (rt_scene_get_ranks).
+ *   - Medium record: p = r.at(t) and normal (1, 0, 0) flipped by front_face, in the medium's space,
+ *     then taken through its Transform chain like a surface's; u = v = 0.
+ *   - An empty interval (t_max_i < t_min, or a NaN bound) gives a miss record; it is not traced and
+ *     takes no draws.  Miss record: t = +inf, p and normal zero, ids and material RT_NONE,
+ *     kind RT_HIT_MISS.
+ * Two launches: a closest-hit surface pass into a stream-ordered scratch buffer (16 bytes per ray),
+ * then the record pass.  `stats` gets segments = n, kernel_launches = 2 and ms_total over both,
+ * and with RT_OPT_COUNT node_visits / prim_tests summed over both passes.  Host-pointer version
+ * copies in and out; the _device version takes device pointers (t_max_per_ray may be NULL) and
+ * enqueues on `stream`. */
+#define RT_HIT_MISS 0u
+#define RT_HIT_SURFACE 1u
+#define RT_HIT_MEDIUM 2u
+
+typedef struct rt_hit_record { /* HitRecord, hit.rs:9-20, in world space */
+    double t;
+    double p[3];
+    double normal[3];     /* faces the ray (set_face_normal, hit.rs:33-36), after the Transform chain */
+    double u, v;          /* binary64; 0, 0 for a medium */
+    uint32_t kind;        /* RT_HIT_* */
+    uint32_t front_face;  /* 0 / 1 */
+    uint32_t prim_id;     /* object index of the leaf shape, or of the RT_OBJ_MEDIUM object; RT_NONE on a miss */
+    uint32_t inst_id;     /* innermost enclosing Transform's object index, RT_NONE if none */
+    uint32_t material;    /* materials[] index: the shape's material (a RemappedMaterial stays as it is, the
+                             remap belongs to scatter) or the medium's phase function; RT_NONE on a miss */
+    uint32_t reserved;
+} rt_hit_record;          /* 96 bytes */
+
+int rt_world_hit(const rt_scene* scene, const rt_ray* rays, const double* t_max_per_ray /* n values or NULL */,
+                 uint64_t n, double t_min, double t_max, uint64_t seed, uint32_t segment, uint32_t flags,
+                 rt_hit_record* out, rt_stats* stats);
+int rt_world_hit_device(const rt_scene* scene, const rt_ray* d_rays, const double* d_t_max_per_ray,
+                        uint64_t n, double t_min, double t_max, uint64_t seed, uint32_t segment,
+                        uint32_t flags, rt_hit_record* d_out, void* stream, rt_stats* stats);
+
 typedef enum rt_accum_type { RT_ACCUM_F32 = 0, RT_ACCUM_F64 = 1 } rt_accum_type;
 
 typedef struct rt_render_opts {

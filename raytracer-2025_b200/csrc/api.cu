@@ -668,6 +668,59 @@ int rt_transmittance(const rt_scene* s, const rt_ray* rays, const double* t_max_
     return rc;
 }
 
+int rt_world_hit_device(const rt_scene* s, const rt_ray* d_rays, const double* d_t_max_per_ray, uint64_t n, double t_min, double t_max,
+                        uint64_t seed, uint32_t segment, uint32_t flags, rt_hit_record* d_out, void* stream, rt_stats* stats) {
+    if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
+    return run_batch(s, n, flags, stream, stats, [&](bool count, unsigned long long* d_cnt, int grid, cudaStream_t st) {
+        // the surface pass writes the surface winner of every ray (16 bytes) to a stream-ordered scratch buffer; the record pass reads it
+        HitRec* d_surface = nullptr;
+        CU(cudaMallocAsync((void**)&d_surface, n * sizeof(HitRec), st));
+        launch_world_hit_surface(s->view, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, count, d_surface, d_cnt, grid, s->stack_bytes, st);
+        int grid_m = s->sm_count * 8;
+        const uint64_t need = (n + MEDIA_BLOCK - 1) / MEDIA_BLOCK;
+        if ((uint64_t)grid_m > need) grid_m = (int)need;
+        launch_world_hit_record(s->view, s->generic_media, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, seed, segment, count, d_surface, d_out,
+                                d_cnt, grid_m, st);
+        CU(cudaFreeAsync(d_surface, st));
+        return 2;
+    });
+}
+
+int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_ray, uint64_t n, double t_min, double t_max, uint64_t seed,
+                 uint32_t segment, uint32_t flags, rt_hit_record* out, rt_stats* stats) {
+    if (!s || (n && (!rays || !out))) return set_err(RT_ERR_INVALID, "null argument");
+    if (n == 0) {
+        if (stats) std::memset(stats, 0, sizeof(*stats));
+        return RT_OK;
+    }
+    rt_ray* d_rays = nullptr;
+    double* d_tmax = nullptr;
+    rt_hit_record* d_out = nullptr;
+    int rc = RT_OK;
+    DeviceGuard guard;
+    try {
+        CU(cudaSetDevice(s->device));
+        scratch_alloc(&d_rays, n * sizeof(rt_ray));
+        scratch_alloc(&d_out, n * sizeof(rt_hit_record));
+        CU(cudaMemcpy(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice));
+        if (t_max_per_ray) {
+            scratch_alloc(&d_tmax, n * sizeof(double));
+            CU(cudaMemcpy(d_tmax, t_max_per_ray, n * sizeof(double), cudaMemcpyHostToDevice));
+        }
+        rc = rt_world_hit_device(s, d_rays, d_tmax, n, t_min, t_max, seed, segment, flags, d_out, nullptr, stats);
+        if (rc == RT_OK) {
+            CU(cudaDeviceSynchronize());
+            CU(cudaMemcpy(out, d_out, n * sizeof(rt_hit_record), cudaMemcpyDeviceToHost));
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    scratch_free(d_rays);
+    scratch_free(d_tmax);
+    scratch_free(d_out);
+    return rc;
+}
+
 static uint64_t count_partition_pixels(uint32_t W, uint32_t H, uint32_t part_index, uint32_t part_count) {
     uint32_t tiles_x = (W + 7) / 8, tiles_y = (H + 7) / 8;
     uint64_t n = 0;

@@ -1,4 +1,4 @@
-// kernels.cu — the wavefront path tracer and the closest-hit and occlusion batch kernels (sm_100a).
+// kernels.cu — the wavefront path tracer and the closest-hit, occlusion, transmittance and world-hit batch kernels (sm_100a).
 //
 // Pipeline per iteration (all queues and counters live in HBM; no host round trip is needed to
 // size a launch — kernels are persistent grid-stride loops that read the counts themselves):
@@ -27,7 +27,7 @@
 namespace rt {
 
 // ------------------------------------------------------------------------------------------
-// closest-hit and occlusion batch kernels (rt_closest_hit, rt_occluded)
+// closest-hit, occlusion and world-hit surface batch kernels (rt_closest_hit, rt_occluded, rt_world_hit)
 // ------------------------------------------------------------------------------------------
 struct RayArrayIO {  // rt_closest_hit batches: rays in, rt_hit out
     const SceneView& sv;
@@ -91,7 +91,32 @@ struct OcclusionIO {  // rt_occluded batches: rays and per-ray t_max in, one byt
     __device__ __forceinline__ void store(uint32_t i, bool hit, double, uint32_t, uint32_t) const { out[i] = hit ? 1 : 0; }
 };
 
-// The persistent traversal of a ray batch, shared by k_closest_hit (ANY = false) and k_occluded (ANY = true).
+struct WorldHitIO {  // rt_world_hit's surface pass: rays and per-ray t_max in, the winner (t, kind, internal primitive) out
+    const rt_ray* __restrict__ rays;
+    const double* __restrict__ tmax_per_ray;  // nullptr: `tmax` for every ray
+    HitRec* __restrict__ out;
+    double tmin, tmax;
+    __device__ __forceinline__ double t_min() const { return tmin; }
+    __device__ __forceinline__ bool load(uint32_t i, RayD& r, double& t1, uint32_t& prim0, uint32_t& rank0) const {
+        const double* rp = reinterpret_cast<const double*>(rays + i);
+        r.o = D3{rp[0], rp[1], rp[2]};
+        r.d = D3{rp[3], rp[4], rp[5]};
+        r.time = rp[6];
+        t1 = tmax_per_ray ? tmax_per_ray[i] : tmax;
+        prim0 = 0xFFFFFFFFu, rank0 = 0xFFFFFFFFu;
+        if (!(tmin <= t1)) {  // an empty interval (t_max_i < t_min, or a NaN bound) contains no t: answered here, never traced
+            store(i, false, 0.0, 0xFFFFFFFFu, 0u);
+            return false;
+        }
+        return true;
+    }
+    __device__ __forceinline__ void prefetch(uint32_t i) const { asm volatile("prefetch.global.L2 [%0];" ::"l"(rays + i)); }
+    __device__ __forceinline__ void store(uint32_t i, bool hit, double t, uint32_t prim, uint32_t) const {
+        *reinterpret_cast<double2*>(out + i) = make_double2(hit ? t : INFINITY, __hiloint2double((int)prim, (int)(hit ? HIT_SURFACE : HIT_MISS)));
+    }
+};
+
+// The persistent traversal of a ray batch, shared by k_closest_hit and k_world_hit_surface (ANY = false) and k_occluded (ANY = true).
 template <bool COUNT, bool USE_RANK, bool PARK, int WIDE, bool XF, int KINDS, bool ANY, class IO>
 __device__ __forceinline__ void trace_batch(const SceneView& sv, IO& io, uint32_t n, unsigned long long* counters) {
     extern __shared__ float4 s_mem[];  // [cached nodes | traversal stacks | per-warp ray FIFOs]
@@ -156,7 +181,7 @@ static void launch_with_l2_window(K kernel, const SceneView& sv, int grid, int b
     cudaLaunchKernelEx(&cfg, kernel, args...);
 }
 
-// The variant of a batch kernel family a scene runs: one choice for k_closest_hit and k_occluded.  F::get<COUNT, PARK, WIDE, XF,
+// The variant of a batch kernel family a scene runs: one choice for k_closest_hit, k_occluded and k_world_hit_surface.  F::get<COUNT, PARK, WIDE, XF,
 // KINDS>() names an instantiation of the family.
 template <class F>
 static auto batch_variant(const SceneView& sv, bool count) {
@@ -704,6 +729,111 @@ __global__ void __launch_bounds__(MEDIA_BLOCK) k_transmittance(SceneView sv, con
             T *= exp(distance_inside_boundary / med.neg_inv_density);
         }
         out[i] = T;
+    }
+    if (COUNT) {
+        atomicAdd(&counters[0], (unsigned long long)cnt.nodes);
+        atomicAdd(&counters[1], (unsigned long long)cnt.prims);
+    }
+}
+
+// rt_world_hit's record pass, after k_world_hit_surface left the surface winner of every ray in `surface`: one ray per thread.
+// Every medium competes on the caller's interval [tmin, t_max_i] as ConstantMedium::hit (volume.rs:37-73) does there, with the
+// free-flight draw philox(seed; pixel = i, sample = 0, segment, RT_MEDIUM_SLOT(medium_index)); the nearest t wins, an exact tie
+// goes to the lower rank.  The winner's HitRecord is rebuilt in world space.  GENERIC / XF as in k_transmittance.
+template <bool COUNT, bool GENERIC, bool XF>
+__global__ void __launch_bounds__(MEDIA_BLOCK) k_world_hit_record(SceneView sv, const rt_ray* __restrict__ rays, const double* __restrict__ tmax_per_ray,
+                                                                uint32_t n, double tmin, double tmax, uint64_t seed, uint32_t segment,
+                                                                const HitRec* __restrict__ surface, rt_hit_record* __restrict__ out,
+                                                                unsigned long long* counters) {
+    extern __shared__ float4 s_mem[];  // traversal stacks for boundaries that are not a single sphere
+    uint32_t* stack = reinterpret_cast<uint32_t*>(s_mem) + threadIdx.x;
+    TraceCounters cnt{0, 0};
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const double2 hw = *reinterpret_cast<const double2*>(surface + i);
+        double t = hw.x;
+        uint32_t kind = (uint32_t)__double2loint(hw.y), prim = (uint32_t)__double2hiint(hw.y);
+        const double t_max_i = tmax_per_ray ? tmax_per_ray[i] : tmax;
+        // an empty interval (t_max_i < t_min, or a NaN bound) is a miss of the surface pass and takes no draws; a surface miss
+        // in a scene without media needs no ray
+        const bool media = tmin <= t_max_i && sv.n_media != 0;
+        RayD r;
+        if (media || kind != HIT_MISS) {
+            const double* rp = reinterpret_cast<const double*>(rays + i);
+            r.o = D3{rp[0], rp[1], rp[2]};
+            r.d = D3{rp[3], rp[4], rp[5]};
+            r.time = rp[6];
+        }
+        uint32_t rank = kind == HIT_SURFACE ? sv.meta[prim].rank : 0xFFFFFFFFu;
+        MediumDraws draws;
+        for (uint32_t m = 0; media && m < sv.n_media; m++) {
+            const Medium& med = sv.media[m];
+            RayD lr;
+            medium_ray<XF>(sv, med, r, lr);
+            double t1, t2;
+            if (med.single_sphere != RT_NONE) {
+                if (!medium_boundary_hits<COUNT, true, XF>(sv, med, r, lr, s_mem, stack, MEDIA_BLOCK, t1, t2, &cnt)) continue;
+            } else if (GENERIC) {
+                if (!medium_boundary_hits<COUNT, false, XF>(sv, med, r, lr, s_mem, stack, MEDIA_BLOCK, t1, t2, &cnt)) continue;
+            } else {
+                continue;  // unreachable: the host launches the GENERIC instantiation for such scenes
+            }
+            if (t1 < tmin) t1 = tmin;  // clamp_min_assign / clamp_max_assign to the caller's interval
+            if (t2 > t_max_i) t2 = t_max_i;
+            if (t1 >= t2) continue;
+            if (t1 < 0.0) t1 = 0.0;
+            const double ray_length = length(lr.d);
+            const double distance_inside_boundary = (t2 - t1) * ray_length;
+            const double hit_distance = med.neg_inv_density * log(draws.get(seed, i, 0u, segment, med.medium_index));
+            if (hit_distance > distance_inside_boundary) continue;
+            const double tm = t1 + hit_distance / ray_length;
+            // the medium competes with the other children of its container like any hit
+            if (kind == HIT_MISS || tm < t || (tm == t && med.rank < rank)) {
+                t = tm;
+                prim = m;
+                kind = HIT_MEDIUM;
+                rank = med.rank;
+            }
+        }
+        HitInfo h;
+        uint32_t object = RT_NONE, xform = RT_NONE;
+        if (kind == HIT_MEDIUM) {  // volume.rs:66-72 in the medium's space, as shade_one builds it
+            const Medium& med = sv.media[prim];
+            RayD lr;
+            medium_ray<XF>(sv, med, r, lr);
+            h.p = lr.o + t * lr.d;
+            const D3 nrm = D3{1.0, 0.0, 0.0};
+            h.front_face = dot(lr.d, nrm) < 0.0;
+            h.normal = h.front_face ? nrm : -nrm;
+            h.u = 0.0, h.v = 0.0;
+            h.material = med.material;
+            object = med.object;
+            if (XF && med.xform != RT_NONE) {
+                xform = med.xform;
+                hit_to_world(sv, xform, h);
+            }
+        } else if (kind == HIT_SURFACE) {
+            surface_hit_info(sv, prim, t, r, true, h);
+            const PrimMeta pm = sv.meta[prim];
+            object = pm.object, xform = pm.xform;
+        } else {
+            t = INFINITY;
+            h.p = h.normal = D3{0.0, 0.0, 0.0};
+            h.u = h.v = 0.0;
+            h.front_face = false;
+            h.material = RT_NONE;
+        }
+        rt_hit_record rec;
+        rec.t = t;
+        rec.p[0] = h.p.x, rec.p[1] = h.p.y, rec.p[2] = h.p.z;
+        rec.normal[0] = h.normal.x, rec.normal[1] = h.normal.y, rec.normal[2] = h.normal.z;
+        rec.u = h.u, rec.v = h.v;
+        rec.kind = kind == HIT_MEDIUM ? RT_HIT_MEDIUM : kind == HIT_SURFACE ? RT_HIT_SURFACE : RT_HIT_MISS;
+        rec.front_face = h.front_face ? 1u : 0u;
+        rec.prim_id = object;
+        rec.inst_id = xform == RT_NONE ? RT_NONE : sv.xforms[xform].inst_object;
+        rec.material = h.material;
+        rec.reserved = 0;
+        out[i] = rec;
     }
     if (COUNT) {
         atomicAdd(&counters[0], (unsigned long long)cnt.nodes);
@@ -1558,6 +1688,19 @@ void launch_transmittance(const SceneView& sv, bool generic, const rt_ray* d_ray
                               : (xf ? k_transmittance<false, false, true> : k_transmittance<false, false, false>));
     k<<<grid, MEDIA_BLOCK, media_smem, s>>>(mv, d_rays, d_tmax_per_ray, n, tmin, tmax, d_occluded, d_out, d_counters);
 }
+void launch_world_hit_record(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin,
+                             double tmax, uint64_t seed, uint32_t segment, bool count, const HitRec* d_surface, rt_hit_record* d_out,
+                             unsigned long long* d_counters, int grid, cudaStream_t s) {
+    SceneView mv = sv;  // global-memory nodes only, as launch_transmittance
+    mv.n_cached_nodes = 0;
+    const size_t media_smem = generic ? (size_t)sv.media_stack_entries * MEDIA_BLOCK * sizeof(uint32_t) : 0;  // <= 64 KB, opted in by kernel_setup
+    const bool xf = sv.media_xform != 0;
+    auto k = generic ? (count ? (xf ? k_world_hit_record<true, true, true> : k_world_hit_record<true, true, false>)
+                              : (xf ? k_world_hit_record<false, true, true> : k_world_hit_record<false, true, false>))
+                     : (count ? (xf ? k_world_hit_record<true, false, true> : k_world_hit_record<true, false, false>)
+                              : (xf ? k_world_hit_record<false, false, true> : k_world_hit_record<false, false, false>));
+    k<<<grid, MEDIA_BLOCK, media_smem, s>>>(mv, d_rays, d_tmax_per_ray, n, tmin, tmax, seed, segment, d_surface, d_out, d_counters);
+}
 template <uint32_t CLS>
 static void launch_shade_cls(const SceneView& sv, const RenderParams& P, const WavefrontState& W, uint32_t queue, int grid, cudaStream_t s) {
     // `grid` is sized for RT_SHADE_MIN_BLOCKS resident CTAs per SM; classes compiled for another count get the matching grid
@@ -1616,6 +1759,26 @@ void launch_finalize(const double* accum, uint64_t n, double scale, void* out, b
     k_finalize<<<grid, 256, 0, s>>>(accum, n, scale, out, out_f64 ? 1 : 0);
 }
 
+// The surface pass of rt_world_hit: closest hit on [tmin, t_max_i], the internal primitive kept for the record pass.  Defined
+// after the render kernels: instantiated ahead of them, the family changes the register assignment of four k_shade
+// instantiations (same instructions, permuted registers), and the render's SASS is kept as it was.
+template <bool COUNT, bool PARK, int WIDE, bool XF = true, int KINDS = 0>
+__global__ void __launch_bounds__(EXTEND_BLOCK, EXTEND_MIN_BLOCKS) k_world_hit_surface(SceneView sv, const rt_ray* __restrict__ rays,
+                                                                       const double* __restrict__ tmax_per_ray, uint32_t n, double tmin,
+                                                                       double tmax, HitRec* __restrict__ out, unsigned long long* counters) {
+    WorldHitIO io{rays, tmax_per_ray, out, tmin, tmax};
+    trace_batch<COUNT, true, PARK, WIDE, XF, KINDS, false>(sv, io, n, counters);
+}
+struct WorldHitSurfaceKernels {
+    template <bool COUNT, bool PARK, int WIDE, bool XF = true, int KINDS = 0>
+    static auto get() { return k_world_hit_surface<COUNT, PARK, WIDE, XF, KINDS>; }
+};
+void launch_world_hit_surface(const SceneView& sv, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax, bool count,
+                              HitRec* d_out, unsigned long long* d_counters, int grid, size_t stack_bytes, cudaStream_t stream) {
+    launch_with_l2_window(batch_variant<WorldHitSurfaceKernels>(sv, count), sv, grid, EXTEND_BLOCK, stack_bytes, stream, sv, d_rays, d_tmax_per_ray,
+                          n, tmin, tmax, d_out, d_counters);
+}
+
 int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks_per_sm, int* walk_blocks_per_sm) {
     // dynamic shared memory above 48 KB is opt-in
     cudaError_t e = cudaSuccess;
@@ -1627,7 +1790,7 @@ int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks
         (const void*)k_extend<true, false, 3, M>
         RT_EXTEND_VARIANTS(0), RT_EXTEND_VARIANTS(1), RT_EXTEND_VARIANTS(2), RT_EXTEND_VARIANTS(3),
 #undef RT_EXTEND_VARIANTS
-        RT_BATCH_VARIANTS(k_closest_hit), RT_BATCH_VARIANTS(k_occluded)};
+        RT_BATCH_VARIANTS(k_closest_hit), RT_BATCH_VARIANTS(k_occluded), RT_BATCH_VARIANTS(k_world_hit_surface)};
     for (const void* f : big_smem)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(EXTEND_SMEM_MAX - 1024))) != cudaSuccess) return (int)e;
     // the general-boundary media pass: TRAVERSAL_STACK entries per thread is 64 KB
@@ -1637,7 +1800,9 @@ int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks
     const void* media_smem[] = {(const void*)k_media<false, 2, false, false>, (const void*)k_media<false, 2, true, false>,
                                 (const void*)k_media<true, 2, false, false>, (const void*)k_media<true, 2, true, false>,
                                 (const void*)k_transmittance<false, true, false>, (const void*)k_transmittance<false, true, true>,
-                                (const void*)k_transmittance<true, true, false>, (const void*)k_transmittance<true, true, true>};
+                                (const void*)k_transmittance<true, true, false>, (const void*)k_transmittance<true, true, true>,
+                                (const void*)k_world_hit_record<false, true, false>, (const void*)k_world_hit_record<false, true, true>,
+                                (const void*)k_world_hit_record<true, true, false>, (const void*)k_world_hit_record<true, true, true>};
     for (const void* f : media_smem)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, TRAVERSAL_STACK * MEDIA_BLOCK * (int)sizeof(uint32_t))) != cudaSuccess) return (int)e;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(extend_blocks_per_sm, k_extend<false, false, 0, 0>, EXTEND_BLOCK, smem_bytes);

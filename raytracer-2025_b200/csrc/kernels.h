@@ -147,6 +147,15 @@ void launch_occluded(const SceneView& sv, const rt_ray* d_rays, const double* d_
 // Sphere.  `grid` CTAs of MEDIA_BLOCK threads.
 void launch_transmittance(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax,
                           bool count, const uint8_t* d_occluded, double* d_out, unsigned long long* d_counters, int grid, cudaStream_t s);
+// The two passes of rt_world_hit.  Surface: d_out[i] = the closest surface hit on [tmin, t_max_i] as a HitRec (internal primitive,
+// kind HIT_SURFACE or HIT_MISS; an empty interval is a miss); the same variant as launch_closest_hit.  Record: every medium competes
+// with that hit on the caller's interval, drawing philox(seed; i, 0, segment, RT_MEDIUM_SLOT(m)), and the winner's record goes to
+// d_out; generic as in launch_transmittance, `grid` CTAs of MEDIA_BLOCK threads.
+void launch_world_hit_surface(const SceneView& sv, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin, double tmax, bool count,
+                              HitRec* d_out, unsigned long long* d_counters, int grid, size_t smem_bytes, cudaStream_t stream);
+void launch_world_hit_record(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin,
+                             double tmax, uint64_t seed, uint32_t segment, bool count, const HitRec* d_surface, rt_hit_record* d_out,
+                             unsigned long long* d_counters, int grid, cudaStream_t s);
 void launch_init(const WavefrontState& W, const RenderParams& P, int grid, cudaStream_t s);
 void launch_generate(const SceneView& sv, const RenderParams& P, const WavefrontState& W, int grid, cudaStream_t s);
 void launch_extend(const SceneView& sv, const RenderParams& P, const WavefrontState& W, bool count, int grid, size_t smem_bytes, cudaStream_t s);

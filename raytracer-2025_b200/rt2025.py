@@ -20,11 +20,12 @@ RT_ACCUM_F32 = 0
 RT_ACCUM_F64 = 1
 RT_BUILD_NO_REF_RANKS = 1
 RT_BUILD_DEVICE_LBVH = 2
+RT_HIT_MISS, RT_HIT_SURFACE, RT_HIT_MEDIUM = 0, 1, 2  # rt_hit_record.kind
 
 # every symbol include/rt2025.h declares (tests check that the library exports them all)
 ABI_SYMBOLS = [
     "rt_scene_create", "rt_scene_destroy", "rt_closest_hit", "rt_closest_hit_device", "rt_occluded", "rt_occluded_device", "rt_transmittance",
-    "rt_transmittance_device", "rt_render",
+    "rt_transmittance_device", "rt_world_hit", "rt_world_hit_device", "rt_render",
     "rt_render_device", "rt_render_rgb8", "rt_render_multi", "rt_render_multi_rgb8", "rt_tonemap", "rt_tonemap_device", "rt_scene_get_info", "rt_scene_get_ranks", "rt_last_error",
     "rt_abi_version", "rt_device_count",
 ]
@@ -124,6 +125,9 @@ rt_object_dtype = np.dtype([("kind", "<u4"), ("material", "<u4"), ("first_child"
 rt_ray_dtype = np.dtype([("origin", "<f8", (3,)), ("direction", "<f8", (3,)), ("time", "<f8")])
 rt_hit_dtype = np.dtype([("t", "<f8"), ("prim_id", "<u4"), ("inst_id", "<u4"), ("u", "<f4"), ("v", "<f4")])
 assert rt_ray_dtype.itemsize == 56 and rt_hit_dtype.itemsize == 24 and rt_object_dtype.itemsize == 72
+rt_hit_record_dtype = np.dtype([("t", "<f8"), ("p", "<f8", (3,)), ("normal", "<f8", (3,)), ("u", "<f8"), ("v", "<f8"), ("kind", "<u4"),
+                                ("front_face", "<u4"), ("prim_id", "<u4"), ("inst_id", "<u4"), ("material", "<u4"), ("reserved", "<u4")])
+assert rt_hit_record_dtype.itemsize == 96
 
 
 def build_native(targets=("product", "host")):
@@ -225,6 +229,11 @@ def product_lib(required=True):
                                            C.c_void_p, C.POINTER(rt_stats)]
             L.rt_transmittance_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint32,
                                                   C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+        if hasattr(L, "rt_world_hit"):  # absent from older builds selected with RT2025_LIB for A/B runs
+            L.rt_world_hit.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint64, C.c_uint32,
+                                       C.c_uint32, C.c_void_p, C.POINTER(rt_stats)]
+            L.rt_world_hit_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint64,
+                                              C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
         L.rt_render.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
                                 C.POINTER(rt_stats)]
         L.rt_render_device.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
@@ -492,6 +501,31 @@ class Scene:
         st = rt_stats()
         _check(self.L.rt_transmittance_device(self.h, d_rays_ptr, d_t_max_ptr, n, t_min, t_max, flags, d_out_ptr, stream, C.byref(st)),
                self.L)
+        return st
+
+    def world_hit(self, rays, t_min=1e-8, t_max=float("inf"), seed=0, segment=0, flags=0):
+        """rt_world_hit: for each ray the HitRecord world.hit(ray, [t_min, t_max]) returns, media sampled with the addressed draws
+        of (seed, pixel = ray index, sample 0, segment).  `t_max` is a scalar or one value per ray.  Returns
+        (rt_hit_record_dtype array, stats)."""
+        rays = np.ascontiguousarray(rays, dtype=rt_ray_dtype)
+        out = np.empty(len(rays), dtype=rt_hit_record_dtype)
+        per_ray = None
+        if np.ndim(t_max) != 0:
+            per_ray = np.ascontiguousarray(t_max, dtype=np.float64)
+            if per_ray.shape != (len(rays),):
+                raise ValueError(f"t_max has shape {per_ray.shape}; a scalar or {len(rays)} values expected")
+            t_max = float("inf")
+        st = rt_stats()
+        _check(self.L.rt_world_hit(self.h, rays.ctypes.data, None if per_ray is None else per_ray.ctypes.data, len(rays), t_min, t_max, seed,
+                                   segment, flags, out.ctypes.data, C.byref(st)), self.L)
+        return out, st
+
+    def world_hit_device(self, d_rays_ptr, n, d_out_ptr, d_t_max_ptr=None, t_min=1e-8, t_max=float("inf"), seed=0, segment=0, flags=0,
+                         stream=None):
+        """rt_world_hit_device: n 96-byte rt_hit_record at d_out_ptr; d_t_max_ptr (n doubles) overrides the scalar t_max."""
+        st = rt_stats()
+        _check(self.L.rt_world_hit_device(self.h, d_rays_ptr, d_t_max_ptr, n, t_min, t_max, seed, segment, flags, d_out_ptr, stream,
+                                          C.byref(st)), self.L)
         return st
 
     def render_opts(self, seed=1, accum_type=RT_ACCUM_F64, part_index=0, part_count=1, sample_begin=0, sample_end=0,

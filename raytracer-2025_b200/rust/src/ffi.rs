@@ -106,6 +106,14 @@ pub struct rt_stats {
 pub struct rt_ray { pub origin: [f64; 3], pub direction: [f64; 3], pub time: f64 }
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct rt_hit { pub t: f64, pub prim_id: u32, pub inst_id: u32, pub u: f32, pub v: f32 }
+pub const RT_HIT_MISS: u32 = 0;
+pub const RT_HIT_SURFACE: u32 = 1;
+pub const RT_HIT_MEDIUM: u32 = 2;
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct rt_hit_record {
+    pub t: f64, pub p: [f64; 3], pub normal: [f64; 3], pub u: f64, pub v: f64,
+    pub kind: u32, pub front_face: u32, pub prim_id: u32, pub inst_id: u32, pub material: u32, pub reserved: u32,
+}
 #[repr(C)] pub struct rt_scene { _private: [u8; 0] }
 
 extern "C" {
@@ -116,6 +124,8 @@ extern "C" {
     pub fn rt_occluded_device(scene: *const rt_scene, d_rays: *const rt_ray, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, d_out: *mut u8, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_transmittance(scene: *const rt_scene, rays: *const rt_ray, t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, out: *mut f64, stats: *mut rt_stats) -> i32;
     pub fn rt_transmittance_device(scene: *const rt_scene, d_rays: *const rt_ray, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, d_out: *mut f64, stream: *mut c_void, stats: *mut rt_stats) -> i32;
+    pub fn rt_world_hit(scene: *const rt_scene, rays: *const rt_ray, t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, seed: u64, segment: u32, flags: u32, out: *mut rt_hit_record, stats: *mut rt_stats) -> i32;
+    pub fn rt_world_hit_device(scene: *const rt_scene, d_rays: *const rt_ray, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, seed: u64, segment: u32, flags: u32, d_out: *mut rt_hit_record, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, accum: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_device(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, d_accum: *mut c_void, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_rgb8(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, rgb: *mut u8, stats: *mut rt_stats) -> i32;
