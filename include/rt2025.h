@@ -261,6 +261,10 @@ int rt_scene_create(const rt_scene_desc* desc, const rt_build_opts* opts, rt_sce
 /* Drop of the scene (the reference's Box<dyn Hittable> going out of scope). */
 int rt_scene_destroy(rt_scene* scene);
 
+/* Any time is valid.  A moving sphere is placed at center + time*center_vec whatever the time, as Sphere::hit does, but
+ * its traversal box bounds it over times [0, 1] only (sphere.rs:35-51): in a scene with a moving sphere a ray whose time
+ * lies outside [0, 1] (or is NaN) culls no box and tests every primitive.  Its answer is still exact, at brute-force cost;
+ * Camera::get_ray draws times in [0, 1). */
 typedef struct rt_ray {
     double origin[3];
     double direction[3];
@@ -295,6 +299,9 @@ typedef struct rt_stats {
 
 /* Closest surface hit for a batch of rays over `world` (media excluded: they are stochastic,
  * volume.rs:58).  Interval semantics are Interval::contains (utils/interval.rs:65-67).
+ * The answer is that of a test of every primitive (the oracle's brute-force mode): the box
+ * test never culls a hit, also where the reference's AABB::hit inside a BVH would (rays that
+ * graze a box face, edge or corner).  This holds for every query below.
  * Host-pointer version copies in and out; the _device version takes device pointers and
  * enqueues on `stream` (a cudaStream_t passed as void*; NULL = default stream). */
 #define RT_OPT_COUNT 1u

@@ -383,6 +383,9 @@ int rt_scene_create(const rt_scene_desc* desc, const rt_build_opts* opts, rt_sce
         v.kinds = (cs.n_spheres && !cs.n_planars) ? 1u : ((cs.n_planars && !cs.n_spheres) ? 2u : 0u);
         v.n_lights = (uint32_t)cs.lights.size();
         v.n_prims = (uint32_t)cs.geom.size();
+        v.moving = 0;
+        for (size_t p = 0; p < cs.geom.size(); p++)
+            if ((cs.meta[p].kind_mat >> 30) == PRIM_SPHERE && (cs.geom[p].d[3] != 0.0 || cs.geom[p].d[4] != 0.0 || cs.geom[p].d[5] != 0.0)) v.moving = 1;
         s->ranks = cs.ranks;
         for (auto& m : cs.media) s->generic_media |= m.single_sphere == RT_NONE;
         v.media_xform = 0;

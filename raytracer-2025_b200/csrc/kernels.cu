@@ -30,6 +30,7 @@ namespace rt {
 // closest-hit, occlusion and world-hit surface batch kernels (rt_closest_hit, rt_occluded, rt_world_hit)
 // ------------------------------------------------------------------------------------------
 struct RayArrayIO {  // rt_closest_hit batches: rays in, rt_hit out
+    static constexpr bool any_time = true;  // the caller's rays may carry any time (make_rayf)
     const SceneView& sv;
     const rt_ray* __restrict__ rays;
     rt_hit* __restrict__ out;
@@ -69,6 +70,7 @@ struct RayArrayIO {  // rt_closest_hit batches: rays in, rt_hit out
 };
 
 struct OcclusionIO {  // rt_occluded batches: rays and per-ray t_max in, one byte out
+    static constexpr bool any_time = true;
     const rt_ray* __restrict__ rays;
     const double* __restrict__ tmax_per_ray;  // nullptr: `tmax` for every ray
     uint8_t* __restrict__ out;
@@ -92,6 +94,7 @@ struct OcclusionIO {  // rt_occluded batches: rays and per-ray t_max in, one byt
 };
 
 struct WorldHitIO {  // rt_world_hit's surface pass: rays and per-ray t_max in, the winner (t, kind, internal primitive) out
+    static constexpr bool any_time = true;
     const rt_ray* __restrict__ rays;
     const double* __restrict__ tmax_per_ray;  // nullptr: `tmax` for every ray
     HitRec* __restrict__ out;
@@ -335,34 +338,6 @@ struct MediumDraws {
 
 constexpr uint32_t MEDIUM_INCUMBENT = 0x80000000u;  // `prim` of a traversal whose incumbent is a medium scatter point: flag | medium index
 
-// ConstantMedium::hit after the two boundary hits t1 < t2 (volume.rs:46-73) on the caller's interval [1e-8, inf): true and the
-// scatter distance when the path scatters inside.  lr: the ray in the medium's space.
-__device__ __forceinline__ bool medium_free_flight(double t1, double t2, const RayD& lr, double neg_inv_density, double xi, double& tm) {
-    if (t1 < 1e-8) t1 = 1e-8;  // clamp to the caller's interval [1e-8, inf)
-    if (t1 >= t2) return false;
-    if (t1 < 0.0) t1 = 0.0;
-    const double ray_length = length(lr.d);
-    const double distance_inside_boundary = (t2 - t1) * ray_length;
-    // binary32 screen: when even a pessimistic free-flight estimate clears the segment inside the boundary by a wide
-    // margin the path does not scatter here and the binary64 ln is not needed (the exact comparison below is unchanged)
-    const float hf = (float)neg_inv_density * logf((float)xi);
-    const float hf_err = 4e-7f * fabsf((float)neg_inv_density);
-    if (hf > (float)distance_inside_boundary * 1.001f + hf_err) return false;
-    const double hit_distance = neg_inv_density * log(xi);
-    if (hit_distance > distance_inside_boundary) return false;
-    tm = t1 + hit_distance / ray_length;
-    return true;
-}
-
-// binary32 screen of a medium against a known hit at t: the scatter point lies at t1 + dist/len with t1 >= 0, so a free flight
-// that clearly overshoots the known hit cannot win whatever the boundary does
-__device__ __forceinline__ bool free_flight_overshoots(double neg_inv_density, double xi, double t, const D3& ld) {
-    const float hf = (float)neg_inv_density * logf((float)xi);
-    const float hf_err = 4e-7f * fabsf((float)neg_inv_density);
-    const float len_f = sqrtf((float)ld.x * (float)ld.x + (float)ld.y * (float)ld.y + (float)ld.z * (float)ld.z);
-    return hf > (float)t * len_f * 1.001f + hf_err;
-}
-
 // The ray in a medium's space (Medium::xform): ConstantMedium::hit measures ray_length on it (volume.rs:55).  XF: the
 // medium may sit under a Transform.
 template <bool XF>
@@ -389,8 +364,8 @@ __device__ __forceinline__ bool medium_boundary_hits(const SceneView& sv, const 
         return sphere_entry_exit(sv.geom[med.single_sphere].d, br, t1, t2);
     }
     uint32_t bp;
-    if (!closest_hit<COUNT, false>(sv, med.root, r, -INFINITY, INFINITY, s_mem, stack, stride, t1, bp, cnt)) return false;
-    return closest_hit<COUNT, false>(sv, med.root, r, t1 + 0.0001, INFINITY, s_mem, stack, stride, t2, bp, cnt);
+    if (!closest_hit<COUNT, false, true>(sv, med.root, r, -INFINITY, INFINITY, s_mem, stack, stride, t1, bp, cnt)) return false;
+    return closest_hit<COUNT, false, true>(sv, med.root, r, t1 + 0.0001, INFINITY, s_mem, stack, stride, t2, bp, cnt);
 }
 
 // ConstantMedium::hit (volume.rs:37-73) for a medium whose boundary is a single Sphere, on the caller's interval
@@ -415,6 +390,7 @@ __device__ __forceinline__ bool sample_sphere_medium(const SceneView& sv, const 
 // (hits.rs:39-46 takes the minimum t over all children, media included).
 template <bool COUNT, int MEDIA>
 struct PathIO {  // k_extend: rays come from the current ray stream, hits go to the hit stream
+    static constexpr bool any_time = false;  // camera rays and their scattered successors carry get_ray's time in [0, 1)
     const SceneView& sv;
     const RayRec* __restrict__ rays;
     HitRec* __restrict__ hits;
@@ -1455,7 +1431,7 @@ __global__ void __launch_bounds__(WALK_BLOCK, LEAN ? RT_WALK_LEAN_MIN_BLOCKS : R
                     if (ENTRIES || (pn == medium && mn.n_entry != MEDIUM_NO_ENTRIES)) {
                         // both ends of the segment lie inside the same boundary: only the world leaves that overlap it can be met
                         for (uint32_t e = 0; e < mn.n_entry && stay; e++) stay = !leaf_beats_scatter(sv, mn.entry[e], nr, 1e-8, tn, med_rank);
-                    } else if (closest_hit<false, true>(sv, sv.world_root, nr, 1e-8, tn, s_mem, stack, WALK_BLOCK, ts, ps, &cnt)) {
+                    } else if (closest_hit<false, true, false>(sv, sv.world_root, nr, 1e-8, tn, s_mem, stack, WALK_BLOCK, ts, ps, &cnt)) {
                         stay = !(ts < tn || sv.meta[ps].rank < med_rank);
                     }
                 }
@@ -1527,7 +1503,7 @@ __global__ void __launch_bounds__(TAIL_BLOCK, 1) k_tail(SceneView sv, RenderPara
             my_segments++;
             double t = INFINITY;
             uint32_t prim = 0xFFFFFFFFu, kind = HIT_MISS;
-            if (closest_hit<false, true>(sv, sv.world_root, r, 1e-8, INFINITY, s_mem, stack, TAIL_BLOCK, t, prim, &cnt)) kind = HIT_SURFACE;
+            if (closest_hit<false, true, false>(sv, sv.world_root, r, 1e-8, INFINITY, s_mem, stack, TAIL_BLOCK, t, prim, &cnt)) kind = HIT_SURFACE;
             if (sv.n_media) sample_media<false, true, true>(sv, P.seed, r, pixel, sidx, segment, t, prim, kind, s_mem, stack, TAIL_BLOCK, &cnt);
             RayD nr;
             D3 nbeta;

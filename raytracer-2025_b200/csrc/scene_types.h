@@ -225,6 +225,7 @@ struct SceneView {
     const WalkLean* walk_lean;  // the scene qualifies for the lean random walk (one record), or nullptr: the generic k_walk
     const ShadeLean* shade_lean;  // the constants of the lean shade-class kernels (one record), or nullptr: every class generic
     uint32_t shade_lean_mask;     // bit c: shade class c runs its lean kernel (ShadeLean)
+    uint32_t moving;              // some sphere moves (center_vec != 0): rays with a time outside [0, 1] cull no box (make_rayf)
 };
 
 }  // namespace rt

@@ -86,7 +86,8 @@ struct RayF {
 };
 #endif
 
-__device__ __forceinline__ void make_rayf(const RayD& r, RayF& f) {
+// moving: the scene holds a moving sphere (SceneView::moving) and the ray may carry any time.
+__device__ __forceinline__ void make_rayf(const RayD& r, RayF& f, bool moving) {
     // An axis whose 1/d overflows binary32 range (d == 0, denormal, NaN) takes no part in culling:
     // its error bound is infinite, so its slab is (-inf, +inf).  Conservative, and only rays exactly
     // parallel to an axis plane pay for it.
@@ -98,6 +99,11 @@ __device__ __forceinline__ void make_rayf(const RayD& r, RayF& f) {
     };
     bool cx, cy, cz;
     f.idx = inv(r.d.x, cx), f.idy = inv(r.d.y, cy), f.idz = inv(r.d.z, cz);
+    // The box of a moving sphere bounds its centre over times [0, 1] only (sphere.rs:35-51), while Sphere::hit places it at any
+    // time: a ray whose time lies outside (or is NaN) culls no box at all, and gets the brute-force answer by testing every
+    // primitive.  Only the query kernels of scenes with a moving sphere pay for the check: the render's rays carry get_ray's
+    // times in [0, 1).
+    if (moving && !(r.time >= 0.0 && r.time <= 1.0)) cx = cy = cz = true;
     const float nox = (float)(-r.o.x * (double)f.idx);
     const float noy = (float)(-r.o.y * (double)f.idy);
     const float noz = (float)(-r.o.z * (double)f.idz);
@@ -322,7 +328,8 @@ __device__ __forceinline__ void stage_nodes(const SceneView& sv, float4* smem_no
 // descending; the warp switches to the (binary64, expensive) primitive tests when every lane still
 // traversing has a parked leaf, or a lane meets a second one.  This keeps the primitive-test code
 // converged: the first version ran it with 3-7 of 32 lanes active (profiles/r01_v1_*).
-template <bool COUNT, bool USE_RANK>
+// ANY_TIME: r may carry a time outside [0, 1] (make_rayf).
+template <bool COUNT, bool USE_RANK, bool ANY_TIME>
 __device__ __forceinline__ bool closest_hit(const SceneView& sv, uint32_t root, const RayD& r, double tmin, double tmax,
                                             const float4* __restrict__ smem_nodes, uint32_t* __restrict__ stack, int stride,
                                             double& best_t, uint32_t& best_prim, TraceCounters* cnt) {
@@ -364,7 +371,7 @@ __device__ __forceinline__ bool closest_hit(const SceneView& sv, uint32_t root, 
         test_leaf(root);
     } else {
         RayF f;
-        make_rayf(r, f);
+        make_rayf(r, f, ANY_TIME && sv.moving);
         const float tmin_f = __double2float_rd(tmin);
         int sp = 0;
         uint32_t cur = root;         // node to visit next; INVALID_REF when the stack ran out
@@ -563,7 +570,7 @@ __device__ __forceinline__ void trace_persistent(const SceneView& sv, IO& io, ui
 #endif
                     if (it < n && io.load(it, r, tbest, prim, prim_rank)) {
                         item = it;
-                        make_rayf(r, f);
+                        make_rayf(r, f, IO::any_time && sv.moving);
                         have = true;
                         tmax_f = __double2float_ru(tbest);
                         cached_xform = 0xFFFFFFFFu;
@@ -599,7 +606,7 @@ __device__ __forceinline__ void trace_persistent(const SceneView& sv, IO& io, ui
                         uint32_t pit = FIFO_INVALID_ITEM;
                         if (it < n && io.load(it, pr, ptmax, p0, r0)) {
                             pit = it;
-                            make_rayf(pr, pf);
+                            make_rayf(pr, pf, IO::any_time && sv.moving);
                         } else {
                             pr.o = pr.d = D3{0.0, 0.0, 0.0}, pr.time = 0.0;
                             pf.idx = pf.idy = pf.idz = pf.nxl = pf.nyl = pf.nzl = pf.nxh = pf.nyh = pf.nzh = 0.f;
@@ -855,6 +862,35 @@ __device__ __forceinline__ bool sphere_entry_exit(const double* __restrict__ g, 
     const double2 a3 = __ldg(reinterpret_cast<const double2*>(g) + 3);
     double near_root, far_root;
     return sphere_entry_exit_at(D3{a0.x, a0.y, a1.x}, D3{a1.y, a2.x, a2.y}, a3.x, r, t1, t2, near_root, far_root);
+}
+
+// ConstantMedium::hit after the two boundary hits t1 < t2 (volume.rs:46-73) on the caller's interval [1e-8, inf): true and the
+// scatter distance when the path scatters inside.  lr: the ray in the medium's space.
+__device__ __forceinline__ bool medium_free_flight(double t1, double t2, const RayD& lr, double neg_inv_density, double xi, double& tm) {
+    if (t1 < 1e-8) t1 = 1e-8;  // clamp to the caller's interval [1e-8, inf)
+    if (t1 >= t2) return false;
+    if (t1 < 0.0) t1 = 0.0;
+    const double ray_length = length(lr.d);
+    const double distance_inside_boundary = (t2 - t1) * ray_length;
+    // binary32 screen: when even a pessimistic free-flight estimate clears the segment inside the boundary by a wide
+    // margin the path does not scatter here and the binary64 ln is not needed (the exact comparison below is unchanged)
+    const float hf = (float)neg_inv_density * logf((float)xi);
+    const float hf_err = 4e-7f * fabsf((float)neg_inv_density);
+    if (hf > (float)distance_inside_boundary * 1.001f + hf_err) return false;
+    const double hit_distance = neg_inv_density * log(xi);
+    if (hit_distance > distance_inside_boundary) return false;
+    tm = t1 + hit_distance / ray_length;
+    return true;
+}
+
+// binary32 screen of a medium against a known hit at t: the scatter point lies at t1 + dist/len with t1 >= 0, so a free flight
+// that clearly overshoots the known hit cannot win whatever the boundary does.  Below |d| = 1e-18 the binary32 squares of the
+// components are subnormal or zero and len_f comes out too short, so such a direction is not screened.
+__device__ __forceinline__ bool free_flight_overshoots(double neg_inv_density, double xi, double t, const D3& ld) {
+    const float hf = (float)neg_inv_density * logf((float)xi);
+    const float hf_err = 4e-7f * fabsf((float)neg_inv_density);
+    const float len_f = sqrtf((float)ld.x * (float)ld.x + (float)ld.y * (float)ld.y + (float)ld.z * (float)ld.z);
+    return len_f >= 1e-18f && hf > (float)t * len_f * 1.001f + hf_err;
 }
 
 }  // namespace rt

@@ -215,6 +215,41 @@ __global__ void k_material_emitted(SceneView sv, const uint32_t* mat, const doub
     st3(out + 3 * i, material_emitted(sv, mat[i], h));
 }
 
+// The box test of every traversal: make_rayf + slab (traverse.cuh).  The binary64 interval bounds are converted the way the
+// traversal converts them - t_min rounded down, t_max rounded up to binary32 - so a caller passes the query's own bounds.
+// in8: o(3) d(3) t_min t_max; box6: lo(3) hi(3); out: 1 when the box is kept
+__global__ void k_slab(const double* in, const float* box, int n, uint8_t* out) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double* x = in + 8 * i;
+    RayD r;
+    r.o = ld3(x), r.d = ld3(x + 3), r.time = 0.0;
+    RayF f;
+    make_rayf(r, f, false);
+    float tnear;
+    out[i] = slab(f, box + 6 * i, box + 6 * i + 3, __double2float_rd(x[6]), __double2float_ru(x[7]), tnear) ? 1 : 0;
+}
+
+// medium_free_flight (traverse.cuh) with the medium's ray direction d.  in7: t1 t2 d(3) neg_inv_density xi; out2: ok, tm
+__global__ void k_medium_free_flight(const double* in, int n, double* out) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double* x = in + 7 * i;
+    RayD lr;
+    lr.o = D3{0.0, 0.0, 0.0}, lr.d = ld3(x + 2), lr.time = 0.0;
+    double tm = 0.0;
+    const bool ok = medium_free_flight(x[0], x[1], lr, x[5], x[6], tm);
+    out[2 * i] = ok ? 1.0 : 0.0, out[2 * i + 1] = tm;
+}
+
+// free_flight_overshoots (traverse.cuh).  in6: neg_inv_density xi t d(3); out: 1 when the screen says the free flight overshoots t
+__global__ void k_free_flight_overshoots(const double* in, int n, uint8_t* out) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double* x = in + 6 * i;
+    out[i] = free_flight_overshoots(x[0], x[1], x[2], ld3(x + 3)) ? 1 : 0;
+}
+
 }  // namespace
 
 // ---- C entry points (ctypes, tests/device_kat.py) -------------------------------------------------
@@ -355,6 +390,24 @@ int kat_material_emitted(const void* h, const uint32_t* mat, const double* in5, 
         check_indices(mat, n, s.n_materials, "material");
         Buffers b; double* d_out = b.out<double>(3 * (size_t)n);
         k_material_emitted<<<grid(n), BLOCK>>>(s.sv, b.in(mat, n), b.in(in5, 5 * (size_t)n), n, d_out); fetch(out3, d_out, 3 * (size_t)n);
+    });
+}
+int kat_slab(const double* in8, const float* box6, int n, uint8_t* out) {
+    return guarded([&] {
+        Buffers b; uint8_t* d_out = b.out<uint8_t>(n);
+        k_slab<<<grid(n), BLOCK>>>(b.in(in8, 8 * (size_t)n), b.in(box6, 6 * (size_t)n), n, d_out); fetch(out, d_out, n);
+    });
+}
+int kat_medium_free_flight(const double* in7, int n, double* out2) {
+    return guarded([&] {
+        Buffers b; double* d_out = b.out<double>(2 * (size_t)n);
+        k_medium_free_flight<<<grid(n), BLOCK>>>(b.in(in7, 7 * (size_t)n), n, d_out); fetch(out2, d_out, 2 * (size_t)n);
+    });
+}
+int kat_free_flight_overshoots(const double* in6, int n, uint8_t* out) {
+    return guarded([&] {
+        Buffers b; uint8_t* d_out = b.out<uint8_t>(n);
+        k_free_flight_overshoots<<<grid(n), BLOCK>>>(b.in(in6, 6 * (size_t)n), n, d_out); fetch(out, d_out, n);
     });
 }
 

@@ -79,6 +79,9 @@ def lib():
         L.kat_lights_pdf.argtypes = [P, C.c_int, P, P, C.c_int, P]
         L.kat_lights_random.argtypes = [P, C.c_int, P, P, C.c_int, P]
         L.kat_material_emitted.argtypes = [P, P, P, C.c_int, P]
+        L.kat_slab.argtypes = [P, P, C.c_int, P]
+        L.kat_medium_free_flight.argtypes = [P, C.c_int, P]
+        L.kat_free_flight_overshoots.argtypes = [P, C.c_int, P]
         _lib = L
     return _lib
 
@@ -130,6 +133,38 @@ def disney_generate(params15, thin, v_out, front_face, pick, u):
     _check(lib().kat_disney_generate(params.ctypes.data, int(bool(thin)), v_out.ctypes.data, ff.ctypes.data, pick.ctypes.data, u.ctypes.data,
                                      len(v_out), out.ctypes.data))
     return out[:, :3], out[:, 3].astype(np.int64)
+
+
+def slab(o, d, t_min, t_max, lo, hi):
+    """make_rayf + slab of the traversal, one call per row: o, d (n, 3) binary64, t_min / t_max (n,) binary64 (rounded to binary32
+    down / up as the traversal does), lo / hi (n, 3) binary32 boxes -> (n,) bool, True when the box is kept."""
+    inp = np.ascontiguousarray(np.column_stack([_f64(o, 3), _f64(d, 3), _f64(t_min), _f64(t_max)]))
+    box = np.ascontiguousarray(np.column_stack([np.asarray(lo, np.float32).reshape(-1, 3), np.asarray(hi, np.float32).reshape(-1, 3)]))
+    n = len(inp)
+    out = np.zeros(n, np.uint8)
+    _check(lib().kat_slab(inp.ctypes.data, box.ctypes.data, n, out.ctypes.data))
+    return out != 0
+
+
+def medium_free_flight(t1, t2, d, neg_inv_density, xi):
+    """medium_free_flight of one medium per row -> (ok (n,) bool, tm (n,))."""
+    d = _f64(d, 3)
+    n = len(d)
+    inp = np.ascontiguousarray(np.column_stack([np.broadcast_to(t1, n), np.broadcast_to(t2, n), d, np.broadcast_to(neg_inv_density, n),
+                                                np.broadcast_to(xi, n)]))
+    out = np.zeros((n, 2))
+    _check(lib().kat_medium_free_flight(inp.ctypes.data, n, out.ctypes.data))
+    return out[:, 0] != 0.0, out[:, 1]
+
+
+def free_flight_overshoots(neg_inv_density, xi, t, d):
+    """free_flight_overshoots per row -> (n,) bool."""
+    d = _f64(d, 3)
+    n = len(d)
+    inp = np.ascontiguousarray(np.column_stack([np.broadcast_to(neg_inv_density, n), np.broadcast_to(xi, n), np.broadcast_to(t, n), d]))
+    out = np.zeros(n, np.uint8)
+    _check(lib().kat_free_flight_overshoots(inp.ctypes.data, n, out.ctypes.data))
+    return out != 0
 
 
 class DeviceScene:

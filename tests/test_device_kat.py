@@ -568,3 +568,217 @@ def test_material_emitted(gpu, rt, orc):
         compare("material_emitted", got, want, rel=REL)
         if k == len(flat) - 1:
             assert np.all(got == 0.0)
+
+
+# ---- the box test (make_rayf + slab) against exact rational arithmetic ------------------------------------------------------------
+# The traversal's box test is binary32 with a hand-derived error slack; every query's claim to the brute-force answer rests on it never
+# culling a box that the exact ray enters.  The reference here is the closed slab interval of the EXACT binary64 ray against the
+# binary32 box, intersected with [t_min, t_max], in fractions.Fraction.  Property: exact interval non-empty => slab keeps the box.
+
+def exact_slab_nonempty(o, d, lo, hi, t_min, t_max):
+    """{t in [t_min, t_max] : lo <= o + t d <= hi} != {} for one row, exactly (infinite bounds allowed, no NaN)."""
+    from fractions import Fraction as F
+    lo_t = None if t_min == -math.inf else F(t_min)
+    hi_t = None if t_max == math.inf else F(t_max)
+    for k in range(3):
+        if lo[k] > hi[k]:
+            return False
+        ok, dk_, lk, hk = F(o[k]), F(d[k]), F(float(lo[k])), F(float(hi[k]))
+        if dk_ == 0:
+            if not (lk <= ok <= hk):
+                return False
+            continue
+        a, b = (lk - ok) / dk_, (hk - ok) / dk_
+        if a > b:
+            a, b = b, a
+        lo_t = a if lo_t is None else max(lo_t, a)
+        hi_t = b if hi_t is None else min(hi_t, b)
+    return lo_t is None or hi_t is None or lo_t <= hi_t
+
+
+def slab_reference(o, d, lo, hi, t_min, t_max):
+    """exact_slab_nonempty for every row.  Rows that binary64 interval arithmetic proves empty by a wide margin are decided there (the
+    rounding error of (lo - o) / d is a few 1e-16 relative, the margin is 1e-9); every other row goes through Fraction."""
+    o, d, t_min, t_max = (np.asarray(a, np.float64) for a in (o, d, t_min, t_max))
+    lo64, hi64 = np.asarray(lo, np.float32).astype(np.float64), np.asarray(hi, np.float32).astype(np.float64)
+    with np.errstate(all="ignore"):
+        a, b = (lo64 - o) / d, (hi64 - o) / d
+        near, far = np.minimum(a, b), np.maximum(a, b)
+        par = d == 0
+        inside = (lo64 <= o) & (o <= hi64)
+        near = np.where(par, np.where(inside, -np.inf, np.inf), near)
+        far = np.where(par, np.where(inside, np.inf, -np.inf), far)
+        tn = np.maximum(near.max(axis=1), t_min)
+        tf = np.minimum(far.min(axis=1), t_max)
+        margin = 1e-9 * (np.abs(tn) + np.abs(tf)) + 1e-300
+        clear = np.isfinite(a).all(axis=1) & np.isfinite(b).all(axis=1) & np.isfinite(tn) & np.isfinite(tf) & (tn - tf > margin)
+        clear |= (np.asarray(lo, np.float32) > np.asarray(hi, np.float32)).any(axis=1)
+        clear |= par.any(axis=1) & ~(inside | ~par).all(axis=1)
+    out = np.zeros(len(o), bool)
+    for i in np.flatnonzero(~clear):
+        out[i] = exact_slab_nonempty(o[i], d[i], lo[i], hi[i], float(t_min[i]), float(t_max[i]))
+    return out
+
+
+def f32_down(x):
+    x = np.asarray(x, np.float64)
+    f = x.astype(np.float32)
+    return np.where(f.astype(np.float64) > x, np.nextafter(f, np.float32(-np.inf)), f).astype(np.float32)
+
+
+def f32_up(x):
+    x = np.asarray(x, np.float64)
+    f = x.astype(np.float32)
+    return np.where(f.astype(np.float64) < x, np.nextafter(f, np.float32(np.inf)), f).astype(np.float32)
+
+
+def slab_cases(rng, n):
+    """(o, d, t_min, t_max, lo, hi): random rows and the adversarial families - a box face exactly at the ray's crossing, o on a face,
+    d components of 0, subnormal or around the 1/d clamp at 1e30, o * (1/d) beyond binary32 range, boxes at +-1e30, degenerate boxes."""
+    parts = []
+
+    def add(o, d, lo, hi, tmin=None, tmax=None):
+        m = len(o)
+        tmin = np.full(m, 1e-8) if tmin is None else np.broadcast_to(tmin, m)
+        tmax = np.full(m, np.inf) if tmax is None else np.broadcast_to(tmax, m)
+        parts.append((np.asarray(o, np.float64), np.asarray(d, np.float64), np.asarray(tmin, np.float64), np.asarray(tmax, np.float64),
+                      np.asarray(lo, np.float32), np.asarray(hi, np.float32)))
+
+    q = n // 8
+    # random rays and boxes at mixed scales
+    scale = 10.0 ** rng.integers(-3, 4, (q, 1))
+    c = rng.normal(size=(q, 3)) * scale
+    e = rng.uniform(0, 1, (q, 3)) * scale
+    add(rng.normal(size=(q, 3)) * scale * 3, rng.normal(size=(q, 3)), c - e, c + e, tmax=np.where(rng.uniform(size=q) < 0.5, np.inf, rng.uniform(0, 20, q) * scale[:, 0]))
+    # a face exactly at the crossing point p = o + t d: the tight binary32 box around p, and the zero-size box at each rounding of p
+    o, d = rng.normal(size=(q, 3)) * 5, rng.normal(size=(q, 3))
+    t = rng.uniform(0.1, 10, (q, 1))
+    p = o + t * d
+    add(o, d, f32_down(p), f32_up(p))
+    add(o, d, f32_down(p), f32_down(p))
+    add(o, d, f32_up(p), f32_up(p))
+    # t_min / t_max at the crossing and a binary64 ulp either side
+    tt = t[:, 0]
+    lo, hi = f32_down(p), f32_up(p)
+    add(o, d, lo, hi, tmin=np.nextafter(tt, np.inf), tmax=np.nextafter(tt, np.inf) * 2)
+    add(o, d, lo, hi, tmin=np.zeros(q), tmax=np.nextafter(tt, -np.inf))
+    # o on a face (binary32-representable origins), the ray leaving, entering or skimming the box
+    o32 = (rng.normal(size=(q, 3)) * 3).astype(np.float32)
+    ext = rng.uniform(0.01, 2, (q, 3)).astype(np.float32)
+    lo, hi = o32.copy(), o32 + ext
+    ax = rng.integers(0, 3, q)
+    d = rng.normal(size=(q, 3))
+    d[np.arange(q), ax] = np.where(rng.uniform(size=q) < 0.3, 0.0, d[np.arange(q), ax])
+    add(o32.astype(np.float64), d, lo, hi)
+    # special direction components and huge origins / boxes
+    specials = np.array([0.0, -0.0, 5e-324, -5e-324, 1e-310, 1e-300, 1e-30 * (1 + 2.0 ** -52), 1e-30 * (1 - 2.0 ** -52), -1e-30 * (1 + 2.0 ** -52),
+                         -1e-30 * (1 - 2.0 ** -52), 1e-30, 1e-20, 1e20])
+    o = rng.normal(size=(q, 3)) * 10.0 ** rng.integers(0, 21, (q, 1))
+    d = rng.normal(size=(q, 3))
+    for k in range(3):
+        sel = rng.uniform(size=q) < 0.4
+        d[sel, k] = rng.choice(specials, sel.sum())
+    box_c = np.where(rng.uniform(size=(q, 1)) < 0.3, np.sign(rng.normal(size=(q, 3))) * 1e30, o + rng.normal(size=(q, 3)) * 10.0 ** rng.integers(0, 21, (q, 1)))
+    box_e = np.abs(box_c) * rng.uniform(0, 1e-6, (q, 3)) + rng.uniform(0, 3, (q, 3))
+    add(o, d, f32_down(box_c - box_e), f32_up(box_c + box_e))
+    # the same boxes, rays aimed at their centres
+    add(o, (box_c - o) * rng.choice(specials[-3:], (q, 1)), f32_down(box_c - box_e), f32_up(box_c + box_e))
+    return tuple(np.concatenate([p_[k] for p_ in parts]) for k in range(6))
+
+
+def test_slab_reference_self_checks():
+    """The exact reference on hand cases, and its binary64 prefilter against Fraction on every row of a sample."""
+    inf = math.inf
+    lo, hi = np.float32([0, 0, 0]), np.float32([1, 1, 1])
+    assert exact_slab_nonempty([-1, 0.5, 0.5], [1, 0, 0], lo, hi, 0, inf)
+    assert exact_slab_nonempty([-1, 1.0, 0.5], [1, 0, 0], lo, hi, 0, inf)  # in the face plane y = 1: closed slab
+    assert not exact_slab_nonempty([-1, np.nextafter(1.0, 2), 0.5], [1, 0, 0], lo, hi, 0, inf)
+    assert exact_slab_nonempty([-1, 0.5, 0.5], [1, 0, 0], lo, hi, 0, 1.0)  # t_max exactly at the entry
+    assert not exact_slab_nonempty([-1, 0.5, 0.5], [1, 0, 0], lo, hi, 0, np.nextafter(1.0, 0))
+    assert exact_slab_nonempty([-1, 1, 0.5], [1, -1, 0], lo, hi, 0, inf)  # touches the edge x = y = 0 only
+    assert not exact_slab_nonempty([-1, 1, 0.5], [1, -np.nextafter(1.0, 2), 0], lo, hi, 0, inf)
+    assert exact_slab_nonempty([-1, 1, 0.5], [1, -np.nextafter(1.0, 0), 0], lo, hi, 0, inf)
+    assert exact_slab_nonempty([2, 0.5, 0.5], [1, 0, 0], lo, hi, -inf, inf)  # behind the origin, unbounded interval
+    assert not exact_slab_nonempty([2, 0.5, 0.5], [1, 0, 0], lo, hi, 0, inf)
+    assert exact_slab_nonempty([0.5, 0.5, 0.5], [5e-324, 0, 0], np.float32([0.5, 0, 0]), np.float32([0.5, 1, 1]), 0, inf)
+    assert not exact_slab_nonempty([0, 0, 0], [1, 1, 1], np.float32([1, 1, 1]), np.float32([0, 2, 2]), -inf, inf)  # inverted box
+    rng = np.random.default_rng(1)
+    o, d, tmin, tmax, lo, hi = slab_cases(rng, 16000)
+    full = np.array([exact_slab_nonempty(o[i], d[i], lo[i], hi[i], float(tmin[i]), float(tmax[i])) for i in range(len(o))])
+    assert np.array_equal(slab_reference(o, d, lo, hi, tmin, tmax), full)
+    assert 0.1 < full.mean() < 0.9  # both answers are well represented
+
+
+@pytest.mark.gpu
+def test_slab_never_culls_an_entered_box(gpu):
+    rng = np.random.default_rng(2025)
+    o, d, tmin, tmax, lo, hi = slab_cases(rng, 1_000_000)
+    kept = dk.slab(o, d, tmin, tmax, lo, hi)
+    # only the rows the slab test rejects can violate the property: the exact reference runs on those
+    rej = np.flatnonzero(~kept)
+    exact = slab_reference(o[rej], d[rej], lo[rej], hi[rej], tmin[rej], tmax[rej])
+    bad = rej[exact]
+    assert len(bad) == 0, f"{len(bad)} boxes culled that the exact ray enters, e.g. o={o[bad[0]]!r} d={d[bad[0]]!r} lo={lo[bad[0]]!r} " \
+                          f"hi={hi[bad[0]]!r} t=[{tmin[bad[0]]!r}, {tmax[bad[0]]!r}]"
+    # information only: how often a box the exact ray misses is kept
+    sample = rng.choice(np.flatnonzero(kept), min(20000, int(kept.sum())), replace=False)
+    fp = ~slab_reference(o[sample], d[sample], lo[sample], hi[sample], tmin[sample], tmax[sample])
+    print(f"\nslab: {len(o)} rows, {len(rej)} culled (all exact misses), false-positive rate among kept boxes ~{fp.mean():.4f}")
+
+
+# ---- the binary32 screens of the media sampling ----------------------------------------------------------------------------------
+# medium_free_flight and free_flight_overshoots skip the binary64 ln when a binary32 estimate decides; a screen that rejects must never
+# disagree with the binary64 decision.
+
+def media_screen_inputs():
+    xis = np.array([2.0 ** -53, 1 - 2.0 ** -53, 1 - 2 * 2.0 ** -53, 1 - 1000 * 2.0 ** -53, 0.5, 0.123456789, 0.9, 1e-3])
+    densities = np.array([1e-38, 1.0, 1e30, 1e300])
+    lens = np.array([1e-25, 1e-20, 1e-19, 1.0, 1e20])
+    rel = np.array([-0.9, -0.5, -1e-4, -1e-6, -1e-9, -1e-12, 0.0, 1e-12, 1e-9, 1e-6, 1e-4])
+    X, Dn, Ln, R = (a.ravel() for a in np.meshgrid(xis, densities, lens, rel, indexing="ij"))
+    rng = np.random.default_rng(7)
+    u = rng.normal(size=(len(X), 3))
+    u[::3, 1:] = 0.0  # axis-parallel directions too
+    d = u / np.linalg.norm(u, axis=1, keepdims=True) * Ln[:, None]
+    return X, -1.0 / Dn, d, R
+
+
+def length64(d):
+    return np.sqrt(d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1] + d[:, 2] * d[:, 2])  # device_math.cuh length()
+
+
+@pytest.mark.gpu
+def test_medium_free_flight_screen(gpu):
+    xi, nid, d, rel = media_screen_inputs()
+    hit = nid * np.log(xi)
+    L = length64(d)
+    # the segment inside the boundary is the free-flight distance (1 + rel): t1 = 1, t2 = 1 + hit (1 + rel) / |d|
+    t1 = np.ones(len(xi))
+    with np.errstate(all="ignore"):
+        t2 = t1 + hit * (1 + rel) / L
+    ok, tm = dk.medium_free_flight(t1, t2, d, nid, xi)
+    with np.errstate(all="ignore"):
+        dist = (t2 - t1) * L
+        want = (t1 < t2) & ~(hit > dist)
+    # rel == 0 rows sit on the decision itself, where the device's and numpy's ln may differ in the last bit
+    far = rel != 0
+    assert np.array_equal(ok[far], want[far]), f"{int((ok != want)[far].sum())} free-flight decisions differ from binary64"
+    assert not (~ok & want & (hit < dist)).any(), "the screen rejected a free flight that scatters inside"
+
+
+@pytest.mark.gpu
+def test_free_flight_overshoots_screen(gpu):
+    """True only where the binary64 scatter point t1 + ln(xi) * neg_inv_density / |d| (t1 >= 0) lies beyond t.  rel < 0: t short of
+    the free flight by that fraction."""
+    xi, nid, d, rel = media_screen_inputs()
+    hit = nid * np.log(xi)
+    L = length64(d)
+    with np.errstate(all="ignore"):
+        t = hit / L * (1 + rel)
+    keep = np.isfinite(t) & (t > 0)
+    xi, nid, d, rel, hit, L, t = xi[keep], nid[keep], d[keep], rel[keep], hit[keep], L[keep], t[keep]
+    over = dk.free_flight_overshoots(nid, xi, t, d)
+    wrong = over & ~(hit / L > t)
+    assert not wrong.any(), f"{int(wrong.sum())} screens claim an overshoot the binary64 free flight does not make, e.g. |d| = " \
+                            f"{L[wrong][:4]}, density = {(-1 / nid[wrong])[:4]}, xi = {xi[wrong][:4]}, rel = {rel[wrong][:4]}"
+    assert over[rel <= -0.5].any()  # the screen does fire where the flight clearly overshoots
