@@ -449,6 +449,7 @@ struct ScatterRecord {
     ONB uvw;
     Ray ray;
     bool error = false;  // an unwrap()/expect() of the reference would have panicked
+    bool fuzzed = false;  // SCATTER_RAY: the direction went through random_unit_vector (sin, cos), a Metal's fuzz
     // DisneyPDF { uvw, v_out, front_face, params }, disney.rs:515-520
     Vec3 v_out;
     bool front_face = false;
@@ -493,6 +494,7 @@ struct Metal : Material {  // material.rs:82-95
         s.kind = SCATTER_RAY;
         s.attenuation = albedo;
         s.ray = Ray(rec.p, reflected, r_in.time);
+        s.fuzzed = true;
         return s;
     }
 };
@@ -1582,68 +1584,104 @@ static Vec3 background_value(const Scene& sc, const rt_camera& cam, const Ray& r
     return sc.textures[cam.background_tex]->value(u, v, p);
 }
 
-// Camera::ray_color, camera.rs:275-325.  `error` is set where the reference would panic.
+// One level of Camera::ray_color (camera.rs:286-321): world.hit of r, then emission and the scatter of the hit.  `error` is set
+// where the reference would panic.  Returns whether the path goes on with s.next: a ScatterRecord::Ray (s.attenuation), or a
+// direction generated by the mixture pdf (s.albedo_x_pscatter, s.pdf_val).
+struct Segment {
+    bool hit = false;
+    HitRecord rec;
+    Vec3 background;               // miss: background_value
+    Vec3 emission;                 // hit: rec.mat->emitted
+    ScatterKind kind = SCATTER_NONE;
+    Vec3 attenuation;              // SCATTER_RAY
+    bool fuzzed = false;           // SCATTER_RAY: ScatterRecord::fuzzed
+    Vec3 albedo_x_pscatter;        // the pdf kinds
+    double pdf_val = 0.0;
+    bool generated = false;        // the pdf kinds: generate() returned Some
+    Ray next;
+    bool error = false;
+};
+static bool ray_step(const Scene& sc, const rt_camera& cam, const Ray& r, PathCtx& ctx, Segment& s) {
+    bool& error = s.error;
+    if (!sc.world->hit(r, Interval::raw(1e-8, INF), ctx, s.rec)) {
+        s.background = background_value(sc, cam, r, error);
+        return false;
+    }
+    s.hit = true;
+    const HitRecord& rec = s.rec;
+    s.emission = rec.mat->emitted(r, rec);
+    ScatterRecord srec = rec.mat->scatter(r, rec, ctx, 0);
+    s.kind = srec.kind;
+    if (srec.error) {
+        error = true;
+        return false;
+    }
+    if (srec.kind == SCATTER_NONE) return false;
+    if (srec.kind == SCATTER_RAY) {
+        s.attenuation = srec.attenuation;
+        s.fuzzed = srec.fuzzed;
+        s.next = srec.ray;
+        return true;
+    }
+    // MixturePDF over (material pdf, HittablePDF(lights)) — camera.rs:297-304, pdf.rs:66-120
+    Rand2 pick = ctx.draw(RT_SLOT_MIXTURE);
+    Vec3 generate_vec;
+    bool generated = true;
+    if (sc.lights && !(pick.a < 0.5)) {
+        Rand2 dirxi = ctx.draw(RT_SLOT_DIRECTION);
+        LightSample ls;
+        ls.leaf = (uint32_t)sc.light_leaves.size() - 1;
+        for (uint32_t i = 0; i < sc.light_leaves.size(); i++)
+            if (pick.b < sc.light_leaves[i].cdf) {
+                ls.leaf = i;
+                break;
+            }
+        ls.r1 = dirxi.a, ls.r2 = dirxi.b;
+        generate_vec = sc.lights->random(rec.p, ls);
+        if (ls.error) error = true;
+    } else {
+        generated = pdf_generate(srec, ctx, generate_vec, error);
+    }
+    if (error) return false;
+    s.generated = generated;
+    if (!generated) return false;  // `generate()` returned None: Color::BLACK (camera.rs:313-315)
+    Ray scattered(rec.p, generate_vec, r.time);
+    Vec3 albedo_x_pscatter;
+    double value0;
+    if (!pdf_value(srec, scattered.dir, albedo_x_pscatter, value0)) {
+        error = true;
+        return false;
+    }
+    double pdf_val = value0;
+    if (sc.lights) {
+        double value1 = sc.lights->pdf_value(rec.p, scattered.dir);
+        if (std::isnan(value1)) error = true;                 // hits.rs:64 assert
+        if (value0 == 0.0 && value1 == 0.0) error = true;     // pdf.rs:105-109 panic
+        pdf_val = value0 * 0.5 + value1 * 0.5;
+    }
+    if (pdf_val == 0.0) error = true;  // camera.rs:309
+    s.next = scattered;
+    s.albedo_x_pscatter = albedo_x_pscatter;
+    s.pdf_val = pdf_val;
+    return !error;
+}
+
+// Camera::ray_color, camera.rs:275-325: ray_step, then the recursion.  `error` is set where the reference would panic.
 static Vec3 ray_color(const Scene& sc, const rt_camera& cam, const Ray& r, uint32_t depth, PathCtx& ctx, RenderCounters& cnt, bool& error) {
     if (depth == 0) return Vec3(0, 0, 0);
     ctx.segment = cam.max_depth - depth;
     cnt.segments++;
-    HitRecord rec;
-    if (!sc.world->hit(r, Interval::raw(1e-8, INF), ctx, rec)) return background_value(sc, cam, r, error);
-
-    Vec3 color_from_emission = rec.mat->emitted(r, rec);
-    ScatterRecord srec = rec.mat->scatter(r, rec, ctx, 0);
-    if (srec.error) {
+    Segment s;
+    const bool goes_on = ray_step(sc, cam, r, ctx, s);
+    if (s.error) {
         error = true;
         return Vec3(0, 0, 0);
     }
-    if (srec.kind == SCATTER_NONE) return color_from_emission;
-
-    Vec3 color_from_scatter;
-    if (srec.kind == SCATTER_RAY) {
-        Vec3 L = ray_color(sc, cam, srec.ray, depth - 1, ctx, cnt, error);
-        color_from_scatter = srec.attenuation * L;
-    } else {
-        // MixturePDF over (material pdf, HittablePDF(lights)) — camera.rs:297-304, pdf.rs:66-120
-        Rand2 pick = ctx.draw(RT_SLOT_MIXTURE);
-        Vec3 generate_vec;
-        bool generated = true;
-        if (sc.lights && !(pick.a < 0.5)) {
-            Rand2 dirxi = ctx.draw(RT_SLOT_DIRECTION);
-            LightSample ls;
-            ls.leaf = (uint32_t)sc.light_leaves.size() - 1;
-            for (uint32_t i = 0; i < sc.light_leaves.size(); i++)
-                if (pick.b < sc.light_leaves[i].cdf) {
-                    ls.leaf = i;
-                    break;
-                }
-            ls.r1 = dirxi.a, ls.r2 = dirxi.b;
-            generate_vec = sc.lights->random(rec.p, ls);
-            if (ls.error) error = true;
-        } else {
-            generated = pdf_generate(srec, ctx, generate_vec, error);
-        }
-        if (error) return Vec3(0, 0, 0);
-        if (!generated) return color_from_emission + Vec3(0, 0, 0);  // `generate()` returned None: Color::BLACK (camera.rs:313-315)
-        Ray scattered(rec.p, generate_vec, r.time);
-        Vec3 albedo_x_pscatter;
-        double value0;
-        if (!pdf_value(srec, scattered.dir, albedo_x_pscatter, value0)) {
-            error = true;
-            return Vec3(0, 0, 0);
-        }
-        double pdf_val = value0;
-        if (sc.lights) {
-            double value1 = sc.lights->pdf_value(rec.p, scattered.dir);
-            if (std::isnan(value1)) error = true;                 // hits.rs:64 assert
-            if (value0 == 0.0 && value1 == 0.0) error = true;     // pdf.rs:105-109 panic
-            pdf_val = value0 * 0.5 + value1 * 0.5;
-        }
-        if (pdf_val == 0.0) error = true;  // camera.rs:309
-        if (error) return Vec3(0, 0, 0);
-        Vec3 sample_color = ray_color(sc, cam, scattered, depth - 1, ctx, cnt, error);
-        color_from_scatter = (albedo_x_pscatter * sample_color) / pdf_val;
-    }
-    Vec3 ret = color_from_emission + color_from_scatter;
+    if (!s.hit) return s.background;
+    if (!goes_on) return s.kind == SCATTER_NONE ? s.emission : s.emission + Vec3(0, 0, 0);
+    Vec3 L = ray_color(sc, cam, s.next, depth - 1, ctx, cnt, error);
+    Vec3 color_from_scatter = s.kind == SCATTER_RAY ? s.attenuation * L : (s.albedo_x_pscatter * L) / s.pdf_val;
+    Vec3 ret = s.emission + color_from_scatter;
     if (std::isnan(ret[0]) || std::isnan(ret[1]) || std::isnan(ret[2])) error = true;  // camera.rs:323
     return ret;
 }
@@ -1771,11 +1809,11 @@ int orc_render(const void* s, const rt_camera* cam, const rt_render_opts* opts, 
     const uint32_t tiles_x = (W + 7) / 8;
     uint64_t paths = 0, segments = 0, errors = 0;
 #ifdef _OPENMP
-    if (threads > 0) omp_set_num_threads(threads);
+    const int team = threads > 0 ? threads : omp_get_max_threads();  // this call only: later calls keep the default
 #else
     (void)threads;
 #endif
-#pragma omp parallel for schedule(dynamic, 16) reduction(+ : paths, segments, errors)
+#pragma omp parallel for num_threads(team) schedule(dynamic, 16) reduction(+ : paths, segments, errors)
     for (int64_t pix = 0; pix < (int64_t)W * H; pix++) {
         uint32_t i = (uint32_t)(pix % W), j = (uint32_t)(pix / W);
         uint32_t tile = (j / 8) * tiles_x + (i / 8);
@@ -1970,6 +2008,35 @@ int orc_kat_lights_random(const void* s, const double* origin, uint32_t leaf, do
     Vec3 d = sc.lights->random(Vec3(origin), ls);
     for (int k = 0; k < 3; k++) out3[k] = d[k];
     return ls.error ? 0 : 1;
+}
+// One level of ray_color per row (ray_step), with the draws addressed by (seeds[i]; ids[3i] pixel, ids[3i+1] sample, ids[3i+2]
+// segment) and media enabled.  out28 per row: hit (0 miss, 1 surface, 2 medium), object id (the leaf shape or the ConstantMedium),
+// t, background(3), emission(3), scatter kind, attenuation(3), albedo_x_pscatter(3), pdf_val, next ray o(3) d(3) time, goes on,
+// generated, error, fuzzed (a SCATTER_RAY direction that went through sin / cos).
+int orc_kat_shade_step(const void* s, const rt_camera* cam, const rt_ray* rays, const uint64_t* seeds, const uint32_t* ids, uint64_t n, double* out28) {
+    const Scene& sc = *(const Scene*)s;
+#pragma omp parallel for schedule(dynamic, 64)
+    for (int64_t k = 0; k < (int64_t)n; k++) {
+        PathCtx ctx;
+        ctx.seed = seeds[k], ctx.pixel = ids[3 * k], ctx.sample = ids[3 * k + 1], ctx.segment = ids[3 * k + 2];
+        Ray r(Vec3(rays[k].origin), Vec3(rays[k].direction), rays[k].time);
+        Segment g;
+        const bool goes_on = ray_step(sc, *cam, r, ctx, g);
+        double* o = out28 + 28 * k;
+        const bool medium = g.hit && sc.by_object[g.rec.prim_id] && dynamic_cast<const ConstantMedium*>(sc.by_object[g.rec.prim_id]);
+        o[0] = g.hit ? (medium ? 2.0 : 1.0) : 0.0;
+        o[1] = g.hit ? (double)g.rec.prim_id : (double)RT_NONE;
+        o[2] = g.hit ? g.rec.t : INF;
+        for (int c = 0; c < 3; c++) {
+            o[3 + c] = g.background[c], o[6 + c] = g.emission[c], o[10 + c] = g.attenuation[c], o[13 + c] = g.albedo_x_pscatter[c];
+            o[17 + c] = g.next.orig[c], o[20 + c] = g.next.dir[c];
+        }
+        o[9] = (double)g.kind;
+        o[16] = g.pdf_val;
+        o[23] = g.next.time;
+        o[24] = goes_on ? 1.0 : 0.0, o[25] = g.generated ? 1.0 : 0.0, o[26] = g.error ? 1.0 : 0.0, o[27] = g.fuzzed ? 1.0 : 0.0;
+    }
+    return 0;
 }
 // texture / environment lookups on a built scene (used to cross-check the device textures)
 void orc_texture_value(const void* s, uint32_t tex, double u, double v, const double* p, double* out) {

@@ -57,6 +57,7 @@ def lib():
         L.orc_kat_lights_pdf_value.restype = C.c_double
         L.orc_kat_lights_pdf_value.argtypes = [C.c_void_p, D, D]
         L.orc_kat_lights_random.argtypes = [C.c_void_p, D, C.c_uint32, C.c_double, C.c_double, D]
+        L.orc_kat_shade_step.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]
         L.orc_camera_ray.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p]
         _lib = L
     return _lib
@@ -123,6 +124,22 @@ class OracleScene:
         out = (C.c_double * 7)()
         kind = self.L.orc_kat_scatter(self.h, mat, ray.ctypes.data, d(*p, *normal, u, v, 1.0 if front_face else 0.0), d(*xi), out)
         return kind, list(out)[0:3], list(out)[3:6], bool(out[6])
+
+    def shade_step(self, rays, seeds, ids3, camera=None):
+        """One level of ray_color per row (ray_step): world.hit with media, emission, scatter, the mixture pdf and the next ray, the
+        draws addressed by (seeds[i]; ids3[i] = pixel, sample, segment).  -> dict of arrays (hit: 0 miss, 1 surface, 2 medium;
+        object: the leaf shape or the ConstantMedium; kind: the ScatterKind; goes_on: the recursion continues with the next ray; fuzzed:
+        a SCATTER_RAY direction that went through sin / cos)."""
+        cam = camera if camera is not None else self.host.camera
+        rays = np.ascontiguousarray(rays, dtype=rt.rt_ray_dtype)
+        n = len(rays)
+        seeds, ids3 = np.ascontiguousarray(seeds, dtype=np.uint64), np.ascontiguousarray(ids3, dtype=np.uint32).reshape(n, 3)
+        out = np.zeros((n, 28))
+        self.L.orc_kat_shade_step(self.h, C.byref(cam), rays.ctypes.data, seeds.ctypes.data, ids3.ctypes.data, n, out.ctypes.data)
+        return dict(hit=out[:, 0].astype(np.int64), object=out[:, 1].astype(np.uint32), t=out[:, 2], background=out[:, 3:6], emission=out[:, 6:9],
+                    kind=out[:, 9].astype(np.int64), attenuation=out[:, 10:13], albedo_x_pscatter=out[:, 13:16], pdf_val=out[:, 16],
+                    o=out[:, 17:20], d=out[:, 20:23], time=out[:, 23], goes_on=out[:, 24] != 0.0, generated=out[:, 25] != 0.0,
+                    error=out[:, 26] != 0.0, fuzzed=out[:, 27] != 0.0)
 
     def lights_pdf_value(self, origin, direction):
         return self.L.orc_kat_lights_pdf_value(self.h, d(*origin), d(*direction))

@@ -14,6 +14,7 @@
 
 #include "kernels.h"  // before shade.cuh: traverse.cuh needs its macros
 #include "shade.cuh"
+#include "shade_step.cuh"
 #include "compile.h"
 
 using namespace rt;
@@ -32,6 +33,11 @@ struct KatScene {
     uint32_t lights_flat = 1;
     bool has_lean = false;
     LeanLights lean{};
+    const ShadeLean* d_shade_lean = nullptr;  // the scene's ShadeLean / WalkLean records on the device, or nullptr
+    const WalkLean* d_walk_lean = nullptr;
+    uint32_t shade_lean_mask = 0, walk_thick = RT_NONE;
+    std::vector<uint32_t> prim_class;  // device primitive -> its compiled shade class (PrimMeta::kind_mat bits 26..29)
+    std::vector<Medium> media;
     std::vector<uint32_t> prim_of_object;  // object id -> device primitive index (meta[].object), RT_NONE elsewhere
     uint32_t n_textures = 0, n_materials = 0, n_remaps = 0;
     std::vector<void*> allocs;
@@ -250,6 +256,74 @@ __global__ void k_free_flight_overshoots(const double* in, int n, uint8_t* out) 
     out[i] = free_flight_overshoots(x[0], x[1], x[2], ld3(x + 3)) ? 1 : 0;
 }
 
+
+// One path segment (shade_step.cuh) per element.  in (rays): the ray; in4: beta(3), t; ids6: pixel, sample, segment, prim, kind,
+// max_depth; seeds.  out16: the contribution added to the element's own zeroed accumulator(3), next ray o(3) d(3) time, nbeta(3),
+// alive, change of the error counter, unused.  LEAN: 0 = shade_one<CLS>; 1 = the lean kernels' code with the ShadeLean record
+// (shade_one<CLS, true>, or lean_isotropic_scatter with axp[prim] for SC_ISOTROPIC); 2 = lean_isotropic_scatter with the WalkLean
+// record (the lean walk's segment).  nr and nbeta start as the ray and beta, as shade_one sets them.
+template <uint32_t CLS, int LEAN>
+__global__ void k_shade_step(SceneView sv, RenderParams P0, const ShadeLean* SL, const WalkLean* WL, const rt_ray* rays, const double* in4,
+                             const uint32_t* ids6, const uint64_t* seeds, int n, double* acc3, Counters* counters, double* out16) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t* id = ids6 + 6 * i;
+    RenderParams P = P0;
+    P.seed = seeds[i], P.cam.max_depth = id[5];
+    // contribute() adds at accum + 3 * pixel: point accum so that this lands on the element's own three doubles (address
+    // arithmetic on integers, the pixel index may be any 28-bit value)
+    WavefrontState W{};
+    W.accum = reinterpret_cast<double*>(reinterpret_cast<uintptr_t>(acc3 + 3 * (size_t)i) - (uintptr_t)id[0] * 3u * sizeof(double));
+    W.counters = counters + i;
+    RayD r;
+    r.o = ld3(rays[i].origin), r.d = ld3(rays[i].direction), r.time = rays[i].time;
+    const D3 beta = ld3(in4 + 4 * i);
+    const double t = in4[4 * i + 3];
+    RayD nr = r;
+    D3 nbeta = beta;
+    bool alive;
+    if constexpr (LEAN == 2)
+        alive = lean_isotropic_scatter(sv, WL->lights, ld3(WL->axp), P, W, r, beta, id[0], id[1], id[2], t, nr, nbeta);
+    else if constexpr (LEAN == 1 && CLS == SC_ISOTROPIC)
+        alive = lean_isotropic_scatter(sv, SL->lights, ld3(SL->axp[id[3]]), P, W, r, beta, id[0], id[1], id[2], t, nr, nbeta);
+    else
+        alive = shade_one<CLS, LEAN == 1>(sv, P, W, r, beta, id[0], id[1], id[2], t, id[3], id[4], nr, nbeta, LEAN ? &SL->lights : nullptr);
+    double* o = out16 + 16 * i;
+    st3(o, nr.o), st3(o + 3, nr.d);
+    o[6] = nr.time;
+    st3(o + 7, nbeta);
+    o[10] = alive ? 1.0 : 0.0;
+    o[11] = (double)counters[i].errors;
+    o[12] = o[13] = o[14] = o[15] = 0.0;
+}
+
+// k_generate's camera ray: camera_ray(cam, seed, j * image_width + i, sidx).  in3: i, j, sidx
+__global__ void k_camera_ray(rt_camera cam, uint64_t seed, const uint32_t* in3, int n, rt_ray* out) {
+    int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const uint32_t* x = in3 + 3 * k;
+    RayD r;
+    camera_ray(cam, seed, x[1] * cam.image_width + x[0], x[2], r);
+    st3(out[k].origin, r.o), st3(out[k].direction, r.d);
+    out[k].time = r.time;
+}
+
+template <uint32_t CLS, int LEAN>
+void launch_shade_step(const KatScene& s, const RenderParams& P, Buffers& b, const rt_ray* rays, const double* in4, const uint32_t* ids6,
+                       const uint64_t* seeds, int n, double* out16) {
+    double* d_acc = b.out<double>(3 * (size_t)n);
+    Counters* d_cnt = b.out<Counters>(n);
+    if (cudaMemset(d_acc, 0, 3 * (size_t)n * sizeof(double)) != cudaSuccess || cudaMemset(d_cnt, 0, (size_t)n * sizeof(Counters)) != cudaSuccess)
+        throw std::string("cudaMemset failed");
+    double* d_out = b.out<double>(16 * (size_t)n);
+    k_shade_step<CLS, LEAN><<<grid(n), BLOCK>>>(s.sv, P, s.d_shade_lean, s.d_walk_lean, b.in(rays, n), b.in(in4, 4 * (size_t)n), b.in(ids6, 6 * (size_t)n),
+                                                b.in(seeds, n), n, d_acc, d_cnt, d_out);
+    fetch(out16, d_out, 16 * (size_t)n);
+    std::vector<double> acc(3 * (size_t)n);
+    fetch(acc.data(), d_acc, acc.size());
+    for (int i = 0; i < n; i++) out16[16 * i + 12] = acc[3 * i], out16[16 * i + 13] = acc[3 * i + 1], out16[16 * i + 14] = acc[3 * i + 2];
+}
+
 }  // namespace
 
 // ---- C entry points (ctypes, tests/device_kat.py) -------------------------------------------------
@@ -282,6 +356,11 @@ void* kat_scene_create(const rt_scene_desc* desc) {
         else if (!cs.walk_lean.empty())
             s->lean = cs.walk_lean[0].lights, s->has_lean = true;
         s->n_textures = (uint32_t)cs.textures.size(), s->n_materials = (uint32_t)cs.materials.size(), s->n_remaps = (uint32_t)cs.remaps.size();
+        s->d_shade_lean = s->put<ShadeLean>(cs.shade_lean), s->d_walk_lean = s->put<WalkLean>(cs.walk_lean);
+        s->shade_lean_mask = cs.shade_lean.empty() ? 0u : cs.shade_lean_mask;
+        s->walk_thick = cs.walk_lean.empty() ? RT_NONE : cs.walk_lean[0].thick;
+        for (auto& m : cs.meta) s->prim_class.push_back((m.kind_mat >> META_CLASS_SHIFT) & 15u);
+        s->media = cs.media;
         s->prim_of_object.assign(desc->n_objects, RT_NONE);
         for (size_t p = 0; p < cs.meta.size(); p++) s->prim_of_object[cs.meta[p].object] = (uint32_t)p;
         return s;
@@ -315,6 +394,73 @@ int kat_light_table(const rt_scene_desc* desc, uint32_t* kind, uint32_t* xform, 
     for (size_t i = 0; i < cs.lights.size() && i < cap; i++)
         kind[i] = cs.lights[i].kind, xform[i] = cs.lights[i].xform, weight[i] = cs.lights[i].weight, cdf[i] = cs.lights[i].cdf;
     return (int)cs.lights.size();
+}
+
+// lean_info: shade_lean_mask (0 without a ShadeLean record), has WalkLean, the WalkLean thick medium (RT_NONE), n_media
+void kat_scene_lean_info(const void* h, uint32_t* out4) {
+    const KatScene& s = *(const KatScene*)h;
+    out4[0] = s.shade_lean_mask, out4[1] = s.d_walk_lean != nullptr, out4[2] = s.walk_thick, out4[3] = (uint32_t)s.media.size();
+}
+// the compiled shade class of every device primitive (PrimMeta::kind_mat bits 26..29)
+void kat_prim_class(const void* h, uint32_t* out, uint32_t n) {
+    const KatScene& s = *(const KatScene*)h;
+    for (uint32_t i = 0; i < n && i < s.prim_class.size(); i++) out[i] = s.prim_class[i];
+}
+// every medium: object id of its ConstantMedium, flags (MEDIUM_THICK), Transform chain (RT_NONE: none)
+void kat_media(const void* h, uint32_t* object, uint32_t* flags, uint32_t* xform, uint32_t n) {
+    const KatScene& s = *(const KatScene*)h;
+    for (uint32_t i = 0; i < n && i < s.media.size(); i++) object[i] = s.media[i].object, flags[i] = s.media[i].flags, xform[i] = s.media[i].xform;
+}
+
+// One segment per element through shade_one<cls> (lean 0), the lean shade kernels' code (lean 1: classes SC_DIFFUSE, SC_TEXTURED,
+// SC_ISOTROPIC) or the lean walk's lean_isotropic_scatter (lean 2).  out16 per element: next ray o(3) d(3) time, nbeta(3), alive,
+// errors, contribution(3), unused.
+int kat_shade_step(const void* h, const rt_camera* cam, uint32_t cls, int lean, const rt_ray* rays, const double* in4,
+                   const uint32_t* ids6, const uint64_t* seeds, int n, double* out16) {
+    const KatScene& s = *(const KatScene*)h;
+    if (lean == 1 && !(s.shade_lean_mask & (1u << cls))) return fail("class " + std::to_string(cls) + " is not lean in this scene");
+    if (lean == 2 && (!s.d_walk_lean || cls != SC_ISOTROPIC)) return fail("the scene has no lean walk");
+    if (lean < 0 || lean > 2) return fail("bad lean");
+    return guarded([&] {
+        for (int i = 0; i < n; i++) {
+            const uint32_t* id = ids6 + 6 * i;
+            const bool medium = id[4] == HIT_MEDIUM, surface = id[4] == HIT_SURFACE;
+            if (id[4] > HIT_MEDIUM || (surface && id[3] >= s.sv.n_prims) || (medium && id[3] >= s.sv.n_media)) throw std::string("primitive index out of range");
+            if (id[0] >= (1u << IDS_PIXEL_BITS) || id[1] >= (1u << IDS_SAMPLE_BITS) || id[2] >= (1u << IDS_SEGMENT_BITS)) throw std::string("path id out of range");
+            // the hit kinds each instantiation reads: a miss has no primitive, a medium index is no primitive index
+            if (id[4] == HIT_MISS && cls != SC_MISS && cls != SC_OTHER) throw std::string("a miss goes to SC_MISS or SC_OTHER");
+            if (id[4] != HIT_MISS && cls == SC_MISS) throw std::string("SC_MISS only shades misses");
+            if (medium && cls != SC_ISOTROPIC && cls != SC_OTHER) throw std::string("a medium hit goes to SC_ISOTROPIC or SC_OTHER");
+            if (lean == 2 && !(medium && id[3] == s.walk_thick)) throw std::string("the lean walk only scatters in its thick medium");
+            if (lean == 1 && cls == SC_ISOTROPIC && !(medium && id[3] < SHADE_LEAN_MEDIA)) throw std::string("lean isotropic: not a medium");
+        }
+        RenderParams P{};
+        P.cam = *cam;
+        P.lights_flat = s.lights_flat;
+        Buffers b;
+        switch (cls * 4 + (uint32_t)lean) {
+#define RT_KAT_CLS(C)                                                                     \
+    case C * 4: launch_shade_step<C, 0>(s, P, b, rays, in4, ids6, seeds, n, out16); break;
+            RT_KAT_CLS(SC_MISS) RT_KAT_CLS(SC_DIFFUSE) RT_KAT_CLS(SC_TEXTURED) RT_KAT_CLS(SC_ISOTROPIC) RT_KAT_CLS(SC_METAL)
+            RT_KAT_CLS(SC_DIELECTRIC) RT_KAT_CLS(SC_EMISSIVE) RT_KAT_CLS(SC_DISNEY) RT_KAT_CLS(SC_OTHER)
+#undef RT_KAT_CLS
+            case SC_DIFFUSE * 4 + 1: launch_shade_step<SC_DIFFUSE, 1>(s, P, b, rays, in4, ids6, seeds, n, out16); break;
+            case SC_TEXTURED * 4 + 1: launch_shade_step<SC_TEXTURED, 1>(s, P, b, rays, in4, ids6, seeds, n, out16); break;
+            case SC_ISOTROPIC * 4 + 1: launch_shade_step<SC_ISOTROPIC, 1>(s, P, b, rays, in4, ids6, seeds, n, out16); break;
+            case SC_ISOTROPIC * 4 + 2: launch_shade_step<SC_ISOTROPIC, 2>(s, P, b, rays, in4, ids6, seeds, n, out16); break;
+            default: throw std::string("no such shade class instantiation");
+        }
+    });
+}
+
+// camera_ray of k_generate per row.  in3: i, j, sidx
+int kat_camera_ray(const rt_camera* cam, uint64_t seed, const uint32_t* in3, int n, rt_ray* out) {
+    return guarded([&] {
+        Buffers b;
+        rt_ray* d_out = b.out<rt_ray>(n);
+        k_camera_ray<<<grid(n), BLOCK>>>(*cam, seed, b.in(in3, 3 * (size_t)n), n, d_out);
+        fetch(out, d_out, n);
+    });
 }
 
 int kat_disney_evaluate(const double* params15, int thin, const double* v_out, const double* v_in, const int* front_face, int n, double* out5) {

@@ -20,6 +20,7 @@ CSRC = os.path.join(ROOT, "raytracer-2025_b200", "csrc")
 HARNESS = os.path.join(HERE, "device_kat.cu")
 LINKED = [os.path.join(CSRC, "compile.cpp"), os.path.join(CSRC, "bvh_build.cpp")]
 RT_NONE = 0xFFFFFFFF
+RAY_DTYPE = np.dtype([("origin", "<f8", (3,)), ("direction", "<f8", (3,)), ("time", "<f8")])  # rt_ray
 
 _lib = None
 
@@ -82,6 +83,11 @@ def lib():
         L.kat_slab.argtypes = [P, P, C.c_int, P]
         L.kat_medium_free_flight.argtypes = [P, C.c_int, P]
         L.kat_free_flight_overshoots.argtypes = [P, C.c_int, P]
+        L.kat_scene_lean_info.argtypes = [P, P]
+        L.kat_prim_class.argtypes = [P, P, C.c_uint32]
+        L.kat_media.argtypes = [P, P, P, P, C.c_uint32]
+        L.kat_shade_step.argtypes = [P, P, C.c_uint32, C.c_int, P, P, P, P, C.c_int, P]
+        L.kat_camera_ray.argtypes = [P, C.c_uint64, P, C.c_int, P]
         _lib = L
     return _lib
 
@@ -167,6 +173,15 @@ def free_flight_overshoots(neg_inv_density, xi, t, d):
     return out != 0
 
 
+def camera_ray(camera, seed, i, j, sidx):
+    """k_generate's camera_ray for every row (i, j, sidx broadcast together) -> rt_ray records."""
+    inp = np.ascontiguousarray(np.column_stack(np.broadcast_arrays(np.asarray(i), np.asarray(j), np.asarray(sidx))), dtype=np.uint32)
+    n = len(inp)
+    out = np.zeros(n, dtype=RAY_DTYPE)
+    _check(lib().kat_camera_ray(C.addressof(camera), int(seed), inp.ctypes.data, n, out.ctypes.data))
+    return out
+
+
 class DeviceScene:
     """The product's compiled tables of `host_scene` on the device, for the shading wrappers."""
 
@@ -182,6 +197,13 @@ class DeviceScene:
         n_obj = host_scene.desc.contents.n_objects
         self.prim_of_object = np.zeros(n_obj, np.uint32)
         self.L.kat_prim_of_object(self.h, self.prim_of_object.ctypes.data, n_obj)
+        lean = np.zeros(4, np.uint32)
+        self.L.kat_scene_lean_info(self.h, lean.ctypes.data)
+        self.shade_lean_mask, self.has_walk_lean, self.walk_thick, n_media = (int(x) for x in lean)
+        self.prim_class = np.zeros(self.n_prims, np.uint32)
+        self.L.kat_prim_class(self.h, self.prim_class.ctypes.data, self.n_prims)
+        self.medium_object, self.medium_flags, self.medium_xform = (np.zeros(n_media, np.uint32) for _ in range(3))
+        self.L.kat_media(self.h, self.medium_object.ctypes.data, self.medium_flags.ctypes.data, self.medium_xform.ctypes.data, n_media)
 
     def __del__(self):
         try:
@@ -249,3 +271,17 @@ class DeviceScene:
         out, mat = np.zeros((n, 3)), _u32(np.broadcast_to(mat, n))
         _check(self.L.kat_material_emitted(self.h, mat.ctypes.data, inp.ctypes.data, n, out.ctypes.data))
         return out
+
+    def shade_step(self, camera, cls, lean, rays, beta, t, ids6, seeds):
+        """One path segment per row (shade_step.cuh): shade_one<cls> (lean 0), the lean shade kernels' code (lean 1) or the lean walk's
+        lean_isotropic_scatter (lean 2).  rays: rt_ray records; beta (n, 3); t (n,); ids6 (n, 6): pixel, sample, segment, device
+        primitive or medium index, hit kind, max_depth; seeds (n,).  -> dict of next o, d, time, nbeta, alive, errors, contribution."""
+        rays = np.ascontiguousarray(rays)
+        n = len(rays)
+        in4 = np.ascontiguousarray(np.column_stack([_f64(beta, 3), _f64(t)]))
+        ids6, seeds = _u32(ids6).reshape(n, 6), np.ascontiguousarray(seeds, dtype=np.uint64)
+        out = np.zeros((n, 16))
+        _check(self.L.kat_shade_step(self.h, C.addressof(camera), int(cls), int(lean), rays.ctypes.data, in4.ctypes.data, ids6.ctypes.data,
+                                     seeds.ctypes.data, n, out.ctypes.data))
+        return dict(o=out[:, 0:3], d=out[:, 3:6], time=out[:, 6], nbeta=out[:, 7:10], alive=out[:, 10] != 0.0, errors=out[:, 11].astype(np.int64),
+                    contribution=out[:, 12:15])

@@ -125,6 +125,40 @@ def compare_hits(rt, got, want, rel=0.0):
     assert np.all(np.isinf(got["t"][~hit]))
 
 
+def materials_scene(rt):
+    """Every material / texture / light kind of configs 1-3 plus Mix, Transparent, Portal, checker, image (nearest + bilinear),
+    triangle and transformed lights, a defocus camera."""
+    rng = np.random.default_rng(7)
+    b = rt.Builder(3)
+    tex_img = b.image(rng.uniform(0, 1, (16, 8, 4)).astype(np.float32))
+    tex_raw = b.image(rng.uniform(0, 1, (5, 7, 4)).astype(np.float32), raw=True)
+    white = b.lambertian(b.solid(0.8, 0.8, 0.8))
+    mats = [
+        b.lambertian(tex_img), b.lambertian(tex_raw), b.lambertian(b.checker(0.5, b.solid(1, 1, 1), tex_img)),
+        b.lambertian(b.noise(2.0)), b.metal([0.9, 0.8, 0.7], 0.3), b.dielectric(b.solid(0.9, 1.0, 0.9), 1.33),
+        b.mix(white, b.metal([1, 1, 1], 0.0), 0.4), b.transparent(),
+        b.portal([0.9, 0.9, 1.0], [0.0, 0.0, -6.0], b.quat_axis_angle([0, 1, 0], 20.0)),
+        b.diffuse_light(b.solid(0.5, 0.4, 0.3), inner=white), b.isotropic(b.solid(0.5, 0.5, 0.9)),
+    ]
+    objs = []
+    for k, m in enumerate(mats):
+        x, y = (k % 4) * 2.2 - 3.3, (k // 4) * 2.2 - 2.0
+        objs.append(b.sphere([x, y, 0], 1.0, m) if k % 2 == 0 else b.quad([x - 0.9, y - 0.9, 0], [1.8, 0, 0], [0, 1.8, 0], m))
+    floor = b.quad([-8, -3.2, -8], [16, 0, 0], [0, 0, 16], white)
+    light = b.diffuse_light(b.solid(10, 10, 10))
+    q = b.quat_axis_angle([1, 0, 0], 25.0)
+    l1 = b.transform(b.quad([-1, 0, -1], [2, 0, 0], [0, 0, 2], light), offset=[0, 6, 2], quat=q, scale=[1.5, 1.5, 1.5])
+    l2 = b.triangle([3, 5, -1], [2, 0, 0], [0, 0, 2], light)
+    world = b.list([b.bvh(objs), floor, l1, l2])
+    e = b.empty()
+    lights = b.list([b.transform(b.quad([-1, 0, -1], [2, 0, 0], [0, 0, 2], e), offset=[0, 6, 2], quat=q, scale=[1.5, 1.5, 1.5]),
+                     b.list([b.triangle([3, 5, -1], [2, 0, 0], [0, 0, 2], e), b.sphere([-3.3, 0.2, 0], 1.0, e)])])  # the metal ball
+    hs = b.finish(world, lights, width=48, spp=16, max_depth=10, vfov=50, look_from=(0, 1, 12), look_at=(0, 0, 0),
+                  background=b.gradient([1, 1, 1], [0.5, 0.7, 1.0]), defocus_angle=0.8, focus_dist=12.0)
+    hs._builder = b
+    return hs
+
+
 def disney_scene(rt, with_lights=True, width=64, spp=16, depth=8, seed=2):
     """Five Disney spheres covering every lobe + one with a base-colour image texture (obj.rs:271-293)."""
     rng = np.random.default_rng(seed)
