@@ -402,6 +402,53 @@ int rt_world_hit_device(const rt_scene* scene, const rt_ray* d_rays, const doubl
                         uint64_t n, double t_min, double t_max, uint64_t seed, uint32_t segment,
                         uint32_t flags, rt_hit_record* d_out, void* stream, rt_stats* stats);
 
+/* Shade: the step of ray_color after world.hit (camera.rs:288-321) for a batch of records as rt_world_hit
+ * writes them, so that a client can run the path loop itself (INTEGRATION.md):
+ *     rays = rt_camera_rays(sample 0); beta = 1; radiance = 0; state = RT_PATH_ALIVE
+ *     for segment in 0 .. max_depth: rt_world_hit(rays, t_max_i = state & RT_PATH_ALIVE ? t_max : NaN,
+ *                                                  seed, segment); rt_shade(..., seed, segment)
+ * reproduces rt_render at one sample per pixel (sqrt_spp = 1).  The path state of row i is updated in place:
+ *   - Active rows: row i is active iff state[i] & RT_PATH_ALIVE.  Of an inactive row only the state byte is
+ *     read, and nothing is written.
+ *   - An active row leaves with state = RT_PATH_ALIVE iff the path goes on, with rays[i] / beta[i] its next
+ *     ray and throughput (otherwise they are left as they were), after the render's cuts: segment + 1 >=
+ *     max_depth, and a zero throughput.  RT_PATH_ERROR is set iff the render counts an error in rt_stats
+ *     for this segment: a case where the reference panics, or a NaN contribution (camera.rs:323); such a
+ *     path may still go on.  The other bits are cleared.
+ *   - radiance[i] (3 binary64) gets beta * emitted, or beta * the background of camera->background_tex
+ *     looked up on the ray direction for a miss; NaN contributions are dropped.
+ *   - Draws: philox(seed; pixel = i, sample = 0, segment, slot) in the renderer's slots (MATERIAL,
+ *     MIXTURE, DIRECTION, MIX + 256 * level, DISNEY), the addressing rt_world_hit uses for its media.
+ *   - The record is the HitRecord: p, normal, u, v, front_face and material are used as given, a
+ *     RemappedMaterial is applied here; t and prim_id are not read.  A record with inst_id != RT_NONE
+ *     and a non-finite normal is a Transform normal that could not be normalised (the reference
+ *     panics).  A record with kind > RT_HIT_MEDIUM, or a non-miss record with material >= n_materials,
+ *     ends its path with RT_PATH_ERROR.
+ *   - camera: only max_depth and background_tex are read.  RT_ERR_INVALID for a null pointer,
+ *     background_tex >= n_textures or segment >= max_depth (the reference never runs that segment).
+ * `stats` gets segments = n, errors = the rows that leave with RT_PATH_ERROR, kernel_launches and
+ * ms_total (the launch alone).  `flags` must be 0 (RT_ERR_INVALID otherwise); every refusal comes
+ * before anything is copied.  Host-pointer version copies in and out (rays, beta, radiance and state
+ * are updated in place); the _device version takes device pointers and enqueues on `stream`. */
+#define RT_PATH_ALIVE 1u /* state bit 0: the path goes on with rays[i] / beta[i] */
+#define RT_PATH_ERROR 2u /* state bit 1: this segment hit a case where the reference panics */
+
+int rt_shade(const rt_scene* scene, const rt_camera* camera, const rt_hit_record* records, uint64_t n, uint64_t seed,
+             uint32_t segment, uint32_t flags, rt_ray* rays, double* beta, double* radiance, uint8_t* state,
+             rt_stats* stats);
+int rt_shade_device(const rt_scene* scene, const rt_camera* camera /* host pointer */, const rt_hit_record* d_records,
+                    uint64_t n, uint64_t seed, uint32_t segment, uint32_t flags, rt_ray* d_rays, double* d_beta,
+                    double* d_radiance, uint8_t* d_state, void* stream, rt_stats* stats);
+
+/* Camera rays: Camera::get_ray (camera.rs:247-273) of stratum `sample` (0 <= sample < sqrt_spp^2:
+ * s_i = sample / sqrt_spp, s_j = sample % sqrt_spp) through every pixel, the ray rt_render traces first:
+ * out[j * image_width + i] for pixel (i, j), image_width * image_height rays, with the draws
+ * philox(seed; pixel, sample, 0, RT_SLOT_CAM_*).  Runs on the current device (no scene), like
+ * rt_tonemap_device.  RT_ERR_INVALID for a null pointer, a bad sample or more than 2^32 - 16 pixels.
+ * The host-pointer version returns when `out` is filled; the _device version enqueues on `stream`. */
+int rt_camera_rays(const rt_camera* camera, uint64_t seed, uint32_t sample, rt_ray* out);
+int rt_camera_rays_device(const rt_camera* camera, uint64_t seed, uint32_t sample, rt_ray* d_out, void* stream);
+
 typedef enum rt_accum_type { RT_ACCUM_F32 = 0, RT_ACCUM_F64 = 1 } rt_accum_type;
 
 typedef struct rt_render_opts {

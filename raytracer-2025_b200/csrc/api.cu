@@ -724,6 +724,138 @@ int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_
     return rc;
 }
 
+// The host-side refusals of rt_shade / rt_shade_device, made before anything is allocated or copied
+static int shade_refusal(const rt_scene* s, const rt_camera* cam, uint32_t segment, uint32_t flags) {
+    if (flags != 0) return set_err(RT_ERR_INVALID, "rt_shade takes no flags (flags must be 0)");
+    if (cam->background_tex >= s->info.n_textures) return set_err(RT_ERR_INVALID, "camera.background_tex out of range");
+    if (segment >= cam->max_depth) return set_err(RT_ERR_INVALID, "segment >= camera.max_depth: the reference never runs that segment");
+    return RT_OK;
+}
+
+int rt_shade_device(const rt_scene* s, const rt_camera* cam, const rt_hit_record* d_records, uint64_t n, uint64_t seed, uint32_t segment,
+                    uint32_t flags, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, void* stream, rt_stats* stats) {
+    if (!s || !cam || (n && (!d_records || !d_rays || !d_beta || !d_radiance || !d_state))) return set_err(RT_ERR_INVALID, "null argument");
+    if (const int refused = shade_refusal(s, cam, segment, flags)) return refused;
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned long long* d_errors = nullptr;
+    int rc = RT_OK;
+    DeviceGuard guard;
+    try {
+        // the error count is only kept for `stats`: its word is allocated, cleared and read back outside the timed launch
+        if (stats && n) {
+            CU(cudaSetDevice(s->device));
+            CU(cudaMallocAsync((void**)&d_errors, sizeof(unsigned long long), st));
+            CU(cudaMemsetAsync(d_errors, 0, sizeof(unsigned long long), st));
+        }
+        rc = run_batch(s, n, 0, stream, stats, [&](bool, unsigned long long*, int, cudaStream_t bs) {
+            RenderParams P{};
+            P.cam = *cam;
+            P.seed = seed;
+            P.lights_flat = s->lights_flat;
+            int grid = s->sm_count * 8;
+            const uint64_t need = (n + SHADE_BLOCK - 1) / SHADE_BLOCK;
+            if ((uint64_t)grid > need) grid = (int)need;
+            launch_shade_records(s->view, P, d_records, n, s->info.n_materials, segment, d_rays, d_beta, d_radiance, d_state, d_errors, grid, bs);
+            return 1;
+        });
+        if (rc == RT_OK && d_errors) {
+            unsigned long long h_errors = 0;
+            CU(cudaMemcpyAsync(&h_errors, d_errors, sizeof(h_errors), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            stats->errors = h_errors;
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    if (d_errors) cudaFreeAsync(d_errors, st);
+    return rc;
+}
+
+int rt_shade(const rt_scene* s, const rt_camera* cam, const rt_hit_record* records, uint64_t n, uint64_t seed, uint32_t segment, uint32_t flags,
+             rt_ray* rays, double* beta, double* radiance, uint8_t* state, rt_stats* stats) {
+    if (!s || !cam || (n && (!records || !rays || !beta || !radiance || !state))) return set_err(RT_ERR_INVALID, "null argument");
+    if (const int refused = shade_refusal(s, cam, segment, flags)) return refused;
+    if (n == 0) {
+        if (stats) std::memset(stats, 0, sizeof(*stats));
+        return RT_OK;
+    }
+    rt_hit_record* d_rec = nullptr;
+    rt_ray* d_rays = nullptr;
+    double *d_beta = nullptr, *d_rad = nullptr;
+    uint8_t* d_state = nullptr;
+    int rc = RT_OK;
+    DeviceGuard guard;
+    try {
+        CU(cudaSetDevice(s->device));
+        scratch_alloc(&d_rec, n * sizeof(rt_hit_record));
+        scratch_alloc(&d_rays, n * sizeof(rt_ray));
+        scratch_alloc(&d_beta, n * 3 * sizeof(double));
+        scratch_alloc(&d_rad, n * 3 * sizeof(double));
+        scratch_alloc(&d_state, n);
+        CU(cudaMemcpy(d_rec, records, n * sizeof(rt_hit_record), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_beta, beta, n * 3 * sizeof(double), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_rad, radiance, n * 3 * sizeof(double), cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(d_state, state, n, cudaMemcpyHostToDevice));
+        rc = rt_shade_device(s, cam, d_rec, n, seed, segment, flags, d_rays, d_beta, d_rad, d_state, nullptr, stats);
+        if (rc == RT_OK) {
+            CU(cudaDeviceSynchronize());
+            CU(cudaMemcpy(rays, d_rays, n * sizeof(rt_ray), cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(beta, d_beta, n * 3 * sizeof(double), cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(radiance, d_rad, n * 3 * sizeof(double), cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(state, d_state, n, cudaMemcpyDeviceToHost));
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    scratch_free(d_rec);
+    scratch_free(d_rays);
+    scratch_free(d_beta);
+    scratch_free(d_rad);
+    scratch_free(d_state);
+    return rc;
+}
+
+int rt_camera_rays_device(const rt_camera* cam, uint64_t seed, uint32_t sample, rt_ray* d_out, void* stream) {
+    if (!cam || !d_out) return set_err(RT_ERR_INVALID, "null argument");
+    if ((uint64_t)sample >= (uint64_t)cam->sqrt_spp * cam->sqrt_spp) return set_err(RT_ERR_INVALID, "sample >= sqrt_spp^2");
+    const uint64_t n = (uint64_t)cam->image_width * cam->image_height;
+    if (n > 0xFFFFFFF0ull) return set_err(RT_ERR_INVALID, "more than 2^32 - 16 pixels");
+    int device, sms;
+    int rc = check_device(-1, device, sms);
+    if (rc != RT_OK || n == 0) return rc;
+    int grid = sms * 8;
+    if ((uint64_t)grid > (n + 255) / 256) grid = (int)((n + 255) / 256);
+    launch_camera_rays(*cam, seed, sample, n, d_out, grid, (cudaStream_t)stream);
+    if (cudaGetLastError() != cudaSuccess) return set_err(RT_ERR_CUDA, "k_camera_rays launch failed");
+    return RT_OK;
+}
+
+int rt_camera_rays(const rt_camera* cam, uint64_t seed, uint32_t sample, rt_ray* out) {
+    if (!cam || !out) return set_err(RT_ERR_INVALID, "null argument");
+    if ((uint64_t)sample >= (uint64_t)cam->sqrt_spp * cam->sqrt_spp) return set_err(RT_ERR_INVALID, "sample >= sqrt_spp^2");
+    const uint64_t n = (uint64_t)cam->image_width * cam->image_height;
+    if (n > 0xFFFFFFF0ull) return set_err(RT_ERR_INVALID, "more than 2^32 - 16 pixels");
+    int device, sms;
+    int rc = check_device(-1, device, sms);
+    if (rc != RT_OK || n == 0) return rc;
+    keep_pool_memory(device);
+    rt_ray* d = nullptr;
+    cudaStream_t st = cudaStreamPerThread;
+    try {
+        CU(cudaMallocAsync((void**)&d, n * sizeof(rt_ray), st));
+        rc = rt_camera_rays_device(cam, seed, sample, d, st);
+        if (rc == RT_OK) {
+            CU(cudaMemcpyAsync(out, d, n * sizeof(rt_ray), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    if (d) cudaFreeAsync(d, st);
+    return rc;
+}
+
 static uint64_t count_partition_pixels(uint32_t W, uint32_t H, uint32_t part_index, uint32_t part_count) {
     uint32_t tiles_x = (W + 7) / 8, tiles_y = (H + 7) / 8;
     uint64_t n = 0;

@@ -1452,6 +1452,92 @@ void launch_world_hit_surface(const SceneView& sv, const rt_ray* d_rays, const d
                           n, tmin, tmax, d_out, d_counters);
 }
 
+// rt_shade: the step of ray_color after world.hit (camera.rs:288-321) for a batch of rt_hit_records, one row per thread, the
+// general instantiation of the render's step (shade_hit<SC_OTHER> + end_segment) with the draws philox(seed; pixel = i,
+// sample = 0, segment, slot).  contribute() adds to radiance + 3 i.  Defined after the render kernels, as the world-hit family.
+__global__ void __launch_bounds__(SHADE_BLOCK, shade_blocks(SC_OTHER, false))
+    k_shade_records(SceneView sv, RenderParams P, const rt_hit_record* __restrict__ records, uint64_t n, uint32_t n_materials, uint32_t segment,
+                    rt_ray* __restrict__ rays, double* __restrict__ beta, double* __restrict__ radiance, uint8_t* __restrict__ state,
+                    unsigned long long* n_errors) {
+    // contribute() and end_segment() count errors at &W.counters->errors: that is this thread's own word of s_errors (address
+    // arithmetic on integers, as tests/device_kat.cu does), so that a row knows whether its segment added one
+    __shared__ unsigned long long s_errors[SHADE_BLOCK];
+    WavefrontState W{};
+    W.accum = radiance;
+    W.counters = reinterpret_cast<Counters*>(reinterpret_cast<uintptr_t>(s_errors + threadIdx.x) - offsetof(Counters, errors));
+    unsigned long long errors = 0;
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        if (!(state[i] & RT_PATH_ALIVE)) continue;  // an inactive row: nothing else of it is read or written
+        s_errors[threadIdx.x] = 0;
+        const uint32_t pixel = (uint32_t)i;
+        const double* rp = reinterpret_cast<const double*>(rays + i);
+        RayD r;
+        r.o = D3{rp[0], rp[1], rp[2]};
+        r.d = D3{rp[3], rp[4], rp[5]};
+        r.time = rp[6];
+        const D3 b = ld3(beta + 3 * i);
+        const rt_hit_record& rec = records[i];
+        const uint32_t kind = rec.kind;
+        RayD nr = r;
+        D3 nbeta = b;
+        bool alive = false, error = false;
+        if (kind > RT_HIT_MEDIUM || (kind != RT_HIT_MISS && rec.material >= n_materials)) {
+            error = true;  // a malformed record (it comes from outside the library): nothing of it is used
+        } else if (kind == RT_HIT_MISS) {
+            D3 bg;
+            if (background_value(sv, P.cam.background_tex, r.d, bg))
+                contribute(P, W, pixel, b * bg);
+            else
+                error = true;
+        } else {
+            HitInfo h;
+            h.p = ld3(rec.p);
+            h.normal = ld3(rec.normal);
+            h.u = rec.u, h.v = rec.v;
+            h.front_face = rec.front_face != 0;
+            h.material = rec.material;
+            // shade_one's hit_ok is what surface_hit_info / hit_to_world return: true without a Transform; under one, false iff
+            // some Transform of the chain left a normal unit_vector could not make finite.  A non-finite normal stays non-finite
+            // through the rest of the chain (scaling and rotating keep an inf or NaN component), and a chain of finite steps ends
+            // finite, so the record's normal tells it exactly.
+            const bool hit_ok = rec.inst_id == RT_NONE || finite3(h.normal);
+            shade_hit<SC_OTHER>(sv, P, W, r, b, pixel, 0u, segment, h, hit_ok, nr, nbeta, alive, error, nullptr);
+        }
+        alive = end_segment(P, W, segment, alive, error, nbeta);
+        const bool err = s_errors[threadIdx.x] != 0;  // a panic, or a NaN contribution contribute() dropped
+        errors += err ? 1u : 0u;
+        if (alive) {
+            double* wp = reinterpret_cast<double*>(rays + i);
+            wp[0] = nr.o.x, wp[1] = nr.o.y, wp[2] = nr.o.z;
+            wp[3] = nr.d.x, wp[4] = nr.d.y, wp[5] = nr.d.z;
+            wp[6] = nr.time;
+            beta[3 * i + 0] = nbeta.x, beta[3 * i + 1] = nbeta.y, beta[3 * i + 2] = nbeta.z;
+        }
+        state[i] = (uint8_t)((alive ? RT_PATH_ALIVE : 0u) | (err ? RT_PATH_ERROR : 0u));
+    }
+    if (errors && n_errors) atomicAdd(n_errors, errors);
+}
+void launch_shade_records(const SceneView& sv, const RenderParams& P, const rt_hit_record* d_records, uint64_t n, uint32_t n_materials,
+                          uint32_t segment, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, unsigned long long* d_errors,
+                          int grid, cudaStream_t s) {
+    k_shade_records<<<grid, SHADE_BLOCK, 0, s>>>(sv, P, d_records, n, n_materials, segment, d_rays, d_beta, d_radiance, d_state, d_errors);
+}
+
+// rt_camera_rays: Camera::get_ray of stratum `sample` through every pixel, k_generate's camera_ray, in the render's pixel order
+__global__ void __launch_bounds__(256) k_camera_rays(rt_camera cam, uint64_t seed, uint32_t sample, uint64_t n, rt_ray* __restrict__ out) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        RayD r;
+        camera_ray(cam, seed, (uint32_t)i, sample, r);
+        double* wp = reinterpret_cast<double*>(out + i);
+        wp[0] = r.o.x, wp[1] = r.o.y, wp[2] = r.o.z;
+        wp[3] = r.d.x, wp[4] = r.d.y, wp[5] = r.d.z;
+        wp[6] = r.time;
+    }
+}
+void launch_camera_rays(const rt_camera& cam, uint64_t seed, uint32_t sample, uint64_t n, rt_ray* d_out, int grid, cudaStream_t s) {
+    k_camera_rays<<<grid, 256, 0, s>>>(cam, seed, sample, n, d_out);
+}
+
 int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks_per_sm, int* walk_blocks_per_sm) {
     // dynamic shared memory above 48 KB is opt-in
     cudaError_t e = cudaSuccess;

@@ -156,6 +156,13 @@ void launch_world_hit_surface(const SceneView& sv, const rt_ray* d_rays, const d
 void launch_world_hit_record(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin,
                              double tmax, uint64_t seed, uint32_t segment, bool count, const HitRec* d_surface, rt_hit_record* d_out,
                              unsigned long long* d_counters, int grid, cudaStream_t s);
+// rt_shade: the render's step after world.hit (shade_hit<SC_OTHER>, end_segment) for every row of d_state with RT_PATH_ALIVE,
+// from its rt_hit_record; *d_errors (may be nullptr) gets the rows that end with RT_PATH_ERROR.  `grid` CTAs of SHADE_BLOCK threads.
+void launch_shade_records(const SceneView& sv, const RenderParams& P, const rt_hit_record* d_records, uint64_t n, uint32_t n_materials,
+                          uint32_t segment, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, unsigned long long* d_errors,
+                          int grid, cudaStream_t s);
+// rt_camera_rays: d_out[pixel] = Camera::get_ray of stratum `sample` (k_generate's camera_ray), `grid` CTAs of 256 threads
+void launch_camera_rays(const rt_camera& cam, uint64_t seed, uint32_t sample, uint64_t n, rt_ray* d_out, int grid, cudaStream_t s);
 void launch_init(const WavefrontState& W, const RenderParams& P, int grid, cudaStream_t s);
 void launch_generate(const SceneView& sv, const RenderParams& P, const WavefrontState& W, int grid, cudaStream_t s);
 void launch_extend(const SceneView& sv, const RenderParams& P, const WavefrontState& W, bool count, int grid, size_t smem_bytes, cudaStream_t s);

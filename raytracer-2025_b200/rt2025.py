@@ -21,11 +21,13 @@ RT_ACCUM_F64 = 1
 RT_BUILD_NO_REF_RANKS = 1
 RT_BUILD_DEVICE_LBVH = 2
 RT_HIT_MISS, RT_HIT_SURFACE, RT_HIT_MEDIUM = 0, 1, 2  # rt_hit_record.kind
+RT_PATH_ALIVE, RT_PATH_ERROR = 1, 2  # rt_shade path state bits
 
 # every symbol include/rt2025.h declares (tests check that the library exports them all)
 ABI_SYMBOLS = [
     "rt_scene_create", "rt_scene_destroy", "rt_closest_hit", "rt_closest_hit_device", "rt_occluded", "rt_occluded_device", "rt_transmittance",
-    "rt_transmittance_device", "rt_world_hit", "rt_world_hit_device", "rt_render",
+    "rt_transmittance_device", "rt_world_hit", "rt_world_hit_device", "rt_shade", "rt_shade_device",
+    "rt_camera_rays", "rt_camera_rays_device", "rt_render",
     "rt_render_device", "rt_render_rgb8", "rt_render_multi", "rt_render_multi_rgb8", "rt_tonemap", "rt_tonemap_device", "rt_scene_get_info", "rt_scene_get_ranks", "rt_last_error",
     "rt_abi_version", "rt_device_count",
 ]
@@ -234,6 +236,13 @@ def product_lib(required=True):
                                        C.c_uint32, C.c_void_p, C.POINTER(rt_stats)]
             L.rt_world_hit_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint64,
                                               C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+        if hasattr(L, "rt_shade"):  # absent from older builds selected with RT2025_LIB for A/B runs
+            L.rt_shade.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p,
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+            L.rt_shade_device.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+            L.rt_camera_rays.argtypes = [C.POINTER(rt_camera), C.c_uint64, C.c_uint32, C.c_void_p]
+            L.rt_camera_rays_device.argtypes = [C.POINTER(rt_camera), C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p]
         L.rt_render.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
                                 C.POINTER(rt_stats)]
         L.rt_render_device.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
@@ -528,6 +537,32 @@ class Scene:
                                           C.byref(st)), self.L)
         return st
 
+    def shade(self, records, rays, beta, radiance, state, seed=0, segment=0, camera=None, flags=0):
+        """rt_shade: the step of ray_color after world.hit for the rows with state & RT_PATH_ALIVE, from the records world_hit
+        returned for `rays`, with the draws of (seed, pixel = row index, sample 0, segment).  Updates the caller's arrays in place:
+        rays (rt_ray_dtype) and beta (n x 3 float64) of the paths that go on, radiance (n x 3 float64, the segment's contribution
+        is added) and state (uint8 RT_PATH_* bits).  Returns the stats."""
+        cam = camera if camera is not None else self.host.camera
+        records = np.ascontiguousarray(records, dtype=rt_hit_record_dtype)
+        n = len(records)
+        for name, a, dt, shape in (("rays", rays, rt_ray_dtype, (n,)), ("beta", beta, np.float64, (n, 3)), ("radiance", radiance, np.float64, (n, 3)),
+                                   ("state", state, np.uint8, (n,))):
+            if not (isinstance(a, np.ndarray) and a.dtype == dt and a.shape == shape and a.flags.c_contiguous and a.flags.writeable):
+                raise ValueError(f"{name}: a writeable C-contiguous {np.dtype(dt)} array of shape {shape} is updated in place")
+        st = rt_stats()
+        _check(self.L.rt_shade(self.h, C.byref(cam), records.ctypes.data, n, seed, segment, flags, rays.ctypes.data, beta.ctypes.data,
+                               radiance.ctypes.data, state.ctypes.data, C.byref(st)), self.L)
+        return st
+
+    def shade_device(self, d_records_ptr, n, d_rays_ptr, d_beta_ptr, d_radiance_ptr, d_state_ptr, seed=0, segment=0, camera=None, flags=0,
+                     stream=None):
+        """rt_shade_device: the same on device buffers (n records, n rays, n x 3 beta and radiance doubles, n state bytes)."""
+        cam = camera if camera is not None else self.host.camera
+        st = rt_stats()
+        _check(self.L.rt_shade_device(self.h, C.byref(cam), d_records_ptr, n, seed, segment, flags, d_rays_ptr, d_beta_ptr, d_radiance_ptr,
+                                      d_state_ptr, stream, C.byref(st)), self.L)
+        return st
+
     def render_opts(self, seed=1, accum_type=RT_ACCUM_F64, part_index=0, part_count=1, sample_begin=0, sample_end=0,
                     flags=0, max_paths_in_flight=0, no_binning=False, classic_media_order=False):
         o = rt_render_opts()
@@ -590,6 +625,21 @@ def render_multi(scenes, camera=None, **kw):
     st = rt_stats()
     _check(L.rt_render_multi(handles, len(scenes), C.byref(cam), C.byref(o), img.ctypes.data, C.byref(st)), L)
     return img, st
+
+
+def camera_rays(camera, seed, sample=0):
+    """rt_camera_rays: Camera::get_ray of stratum `sample` through every pixel, image_width * image_height rays in the render's
+    pixel order (pixel = j * image_width + i)."""
+    L = product_lib()
+    out = np.empty(camera.image_width * camera.image_height, dtype=rt_ray_dtype)
+    _check(L.rt_camera_rays(C.byref(camera), seed, sample, out.ctypes.data), L)
+    return out
+
+
+def camera_rays_device(camera, seed, sample, d_out_ptr, stream=None):
+    """rt_camera_rays_device: the same into image_width * image_height rays at d_out_ptr on the current device."""
+    L = product_lib()
+    _check(L.rt_camera_rays_device(C.byref(camera), seed, sample, d_out_ptr, stream), L)
 
 
 def tonemap_device(d_accum_ptr, n_pixels, d_rgb_ptr, toon_map=0, accum_type=RT_ACCUM_F32, stream=None):

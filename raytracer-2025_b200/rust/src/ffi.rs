@@ -109,6 +109,8 @@ pub struct rt_hit { pub t: f64, pub prim_id: u32, pub inst_id: u32, pub u: f32, 
 pub const RT_HIT_MISS: u32 = 0;
 pub const RT_HIT_SURFACE: u32 = 1;
 pub const RT_HIT_MEDIUM: u32 = 2;
+pub const RT_PATH_ALIVE: u8 = 1;
+pub const RT_PATH_ERROR: u8 = 2;
 #[repr(C)] #[derive(Clone, Copy, Default)]
 pub struct rt_hit_record {
     pub t: f64, pub p: [f64; 3], pub normal: [f64; 3], pub u: f64, pub v: f64,
@@ -126,6 +128,10 @@ extern "C" {
     pub fn rt_transmittance_device(scene: *const rt_scene, d_rays: *const rt_ray, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, flags: u32, d_out: *mut f64, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_world_hit(scene: *const rt_scene, rays: *const rt_ray, t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, seed: u64, segment: u32, flags: u32, out: *mut rt_hit_record, stats: *mut rt_stats) -> i32;
     pub fn rt_world_hit_device(scene: *const rt_scene, d_rays: *const rt_ray, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, seed: u64, segment: u32, flags: u32, d_out: *mut rt_hit_record, stream: *mut c_void, stats: *mut rt_stats) -> i32;
+    pub fn rt_shade(scene: *const rt_scene, cam: *const rt_camera, records: *const rt_hit_record, n: u64, seed: u64, segment: u32, flags: u32, rays: *mut rt_ray, beta: *mut f64, radiance: *mut f64, state: *mut u8, stats: *mut rt_stats) -> i32;
+    pub fn rt_shade_device(scene: *const rt_scene, cam: *const rt_camera, d_records: *const rt_hit_record, n: u64, seed: u64, segment: u32, flags: u32, d_rays: *mut rt_ray, d_beta: *mut f64, d_radiance: *mut f64, d_state: *mut u8, stream: *mut c_void, stats: *mut rt_stats) -> i32;
+    pub fn rt_camera_rays(cam: *const rt_camera, seed: u64, sample: u32, out: *mut rt_ray) -> i32;
+    pub fn rt_camera_rays_device(cam: *const rt_camera, seed: u64, sample: u32, d_out: *mut rt_ray, stream: *mut c_void) -> i32;
     pub fn rt_render(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, accum: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_device(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, d_accum: *mut c_void, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_rgb8(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, rgb: *mut u8, stats: *mut rt_stats) -> i32;
