@@ -302,6 +302,8 @@ typedef struct rt_stats {
  * The answer is that of a test of every primitive (the oracle's brute-force mode): the box
  * test never culls a hit, also where the reference's AABB::hit inside a BVH would (rays that
  * graze a box face, edge or corner).  This holds for every query below.
+ * A batch holds at most 2^32 - 16 rays: a larger n is RT_ERR_INVALID for every query below and
+ * rt_shade, refused before anything is allocated or copied.
  * Host-pointer version copies in and out; the _device version takes device pointers and
  * enqueues on `stream` (a cudaStream_t passed as void*; NULL = default stream). */
 #define RT_OPT_COUNT 1u
@@ -420,10 +422,11 @@ int rt_world_hit_device(const rt_scene* scene, const rt_ray* d_rays, const doubl
  *   - Draws: philox(seed; pixel = i, sample = 0, segment, slot) in the renderer's slots (MATERIAL,
  *     MIXTURE, DIRECTION, MIX + 256 * level, DISNEY), the addressing rt_world_hit uses for its media.
  *   - The record is the HitRecord: p, normal, u, v, front_face and material are used as given, a
- *     RemappedMaterial is applied here; t and prim_id are not read.  A record with inst_id != RT_NONE
- *     and a non-finite normal is a Transform normal that could not be normalised (the reference
- *     panics).  A record with kind > RT_HIT_MEDIUM, or a non-miss record with material >= n_materials,
- *     ends its path with RT_PATH_ERROR.
+ *     RemappedMaterial is applied here; t, prim_id and reserved are not read, nor any field of a miss
+ *     but its kind.  front_face: any nonzero value means front.  inst_id is only a flag, never an
+ *     index: a record with inst_id != RT_NONE and a non-finite normal is a Transform normal that
+ *     could not be normalised (the reference panics).  A record with kind > RT_HIT_MEDIUM, or a
+ *     non-miss record with material >= n_materials, ends its path with RT_PATH_ERROR.
  *   - camera: only max_depth and background_tex are read.  RT_ERR_INVALID for a null pointer,
  *     background_tex >= n_textures or segment >= max_depth (the reference never runs that segment).
  * `stats` gets segments = n, errors = the rows that leave with RT_PATH_ERROR, kernel_launches and

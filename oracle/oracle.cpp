@@ -369,15 +369,16 @@ struct NoiseTexture : Texture {  // texture.rs:191-196, utils/perlin.rs:40-89
         double uvw[3];
         for (int a = 0; a < 3; a++) {
             double fl = std::floor(p[a]);
-            ijk[a] = std::isnan(fl) ? 0 : (fl >= 9.2e18 ? INT64_MAX : (fl <= -9.2e18 ? INT64_MIN : (int64_t)fl));
+            // Rust `as i64`: NaN -> 0, saturating at -2^63 and 2^63 - 1 (every double below 2^63 in magnitude converts exactly)
+            ijk[a] = std::isnan(fl) ? 0 : (fl >= 0x1p63 ? INT64_MAX : (fl < -0x1p63 ? INT64_MIN : (int64_t)fl));
             uvw[a] = p[a] - fl;
         }
         Vec3 c[2][2][2];
         for (int di = 0; di < 2; di++)
             for (int dj = 0; dj < 2; dj++)
-                for (int dk = 0; dk < 2; dk++) {
-                    uint32_t idx = tab->perm_x[(uint64_t)(ijk[0] + di) & 255] ^ tab->perm_y[(uint64_t)(ijk[1] + dj) & 255] ^
-                                   tab->perm_z[(uint64_t)(ijk[2] + dk) & 255];
+                for (int dk = 0; dk < 2; dk++) {  // ijk + 1 wraps at INT64_MAX: add in uint64_t
+                    uint32_t idx = tab->perm_x[((uint64_t)ijk[0] + di) & 255] ^ tab->perm_y[((uint64_t)ijk[1] + dj) & 255] ^
+                                   tab->perm_z[((uint64_t)ijk[2] + dk) & 255];
                     c[di][dj][dk] = Vec3(tab->randvec[idx]);
                 }
         // perlin_interp, perlin.rs:73-89
@@ -422,6 +423,8 @@ struct HitRecord {
     const Material* mat = nullptr;
     double t = 0, u = 0, v = 0;
     bool front_face = false;
+    // a Transform of the chain could not normalise its normal: the reference panics there (shapes.rs:107, .expect)
+    bool normal_panic = false;
     uint32_t prim_id = RT_NONE, inst_id = RT_NONE;
     static HitRecord make(Vec3 p, Vec3 normal, const Material* mat, double t, double u, double v, const Ray& r_in) {  // hit.rs:24-43
         HitRecord h;
@@ -1184,7 +1187,7 @@ struct Transform : Hittable {  // shapes.rs:23-133
         if (!object->hit(local_ray, interval, ctx, rec)) return false;
         rec.p = transform(rec.p);
         Vec3 n;
-        unit_vector(q.rotate_vector(vdiv(rec.normal, scale)), n);
+        if (!unit_vector(q.rotate_vector(vdiv(rec.normal, scale)), n)) rec.normal_panic = true;
         rec.normal = n;
         if (rec.inst_id == RT_NONE) rec.inst_id = id;
         return true;
@@ -1601,15 +1604,21 @@ struct Segment {
     Ray next;
     bool error = false;
 };
-static bool ray_step(const Scene& sc, const rt_camera& cam, const Ray& r, PathCtx& ctx, Segment& s) {
+// The step after world.hit (camera.rs:288-321) on the HitRecord `rec` of r, or on a miss (rec == nullptr): the background, or
+// emission, scatter, the mixture pdf and the next ray.  A record whose Transform normal could not be normalised is the panic of
+// Transform::hit; its emission is still evaluated, as the device adds it before it ends the path.
+static bool shade_record(const Scene& sc, const rt_camera& cam, const Ray& r, const HitRecord* hit, PathCtx& ctx, Segment& s) {
     bool& error = s.error;
-    if (!sc.world->hit(r, Interval::raw(1e-8, INF), ctx, s.rec)) {
+    if (!hit) {
         s.background = background_value(sc, cam, r, error);
         return false;
     }
     s.hit = true;
+    s.rec = *hit;
     const HitRecord& rec = s.rec;
+    if (rec.normal_panic) error = true;
     s.emission = rec.mat->emitted(r, rec);
+    if (error) return false;
     ScatterRecord srec = rec.mat->scatter(r, rec, ctx, 0);
     s.kind = srec.kind;
     if (srec.error) {
@@ -1664,6 +1673,11 @@ static bool ray_step(const Scene& sc, const rt_camera& cam, const Ray& r, PathCt
     s.albedo_x_pscatter = albedo_x_pscatter;
     s.pdf_val = pdf_val;
     return !error;
+}
+static bool ray_step(const Scene& sc, const rt_camera& cam, const Ray& r, PathCtx& ctx, Segment& s) {
+    HitRecord rec;
+    const bool hit = sc.world->hit(r, Interval::raw(1e-8, INF), ctx, rec);
+    return shade_record(sc, cam, r, hit ? &rec : nullptr, ctx, s);
 }
 
 // Camera::ray_color, camera.rs:275-325: ray_step, then the recursion.  `error` is set where the reference would panic.
@@ -2009,6 +2023,17 @@ int orc_kat_lights_random(const void* s, const double* origin, uint32_t leaf, do
     for (int k = 0; k < 3; k++) out3[k] = d[k];
     return ls.error ? 0 : 1;
 }
+static void write_segment(const Segment& g, bool goes_on, double hit_kind, double object, double t, double* o) {
+    o[0] = hit_kind, o[1] = object, o[2] = t;
+    for (int c = 0; c < 3; c++) {
+        o[3 + c] = g.background[c], o[6 + c] = g.emission[c], o[10 + c] = g.attenuation[c], o[13 + c] = g.albedo_x_pscatter[c];
+        o[17 + c] = g.next.orig[c], o[20 + c] = g.next.dir[c];
+    }
+    o[9] = (double)g.kind;
+    o[16] = g.pdf_val;
+    o[23] = g.next.time;
+    o[24] = goes_on ? 1.0 : 0.0, o[25] = g.generated ? 1.0 : 0.0, o[26] = g.error ? 1.0 : 0.0, o[27] = g.fuzzed ? 1.0 : 0.0;
+}
 // One level of ray_color per row (ray_step), with the draws addressed by (seeds[i]; ids[3i] pixel, ids[3i+1] sample, ids[3i+2]
 // segment) and media enabled.  out28 per row: hit (0 miss, 1 surface, 2 medium), object id (the leaf shape or the ConstantMedium),
 // t, background(3), emission(3), scatter kind, attenuation(3), albedo_x_pscatter(3), pdf_val, next ray o(3) d(3) time, goes on,
@@ -2022,19 +2047,40 @@ int orc_kat_shade_step(const void* s, const rt_camera* cam, const rt_ray* rays, 
         Ray r(Vec3(rays[k].origin), Vec3(rays[k].direction), rays[k].time);
         Segment g;
         const bool goes_on = ray_step(sc, *cam, r, ctx, g);
-        double* o = out28 + 28 * k;
         const bool medium = g.hit && sc.by_object[g.rec.prim_id] && dynamic_cast<const ConstantMedium*>(sc.by_object[g.rec.prim_id]);
-        o[0] = g.hit ? (medium ? 2.0 : 1.0) : 0.0;
-        o[1] = g.hit ? (double)g.rec.prim_id : (double)RT_NONE;
-        o[2] = g.hit ? g.rec.t : INF;
-        for (int c = 0; c < 3; c++) {
-            o[3 + c] = g.background[c], o[6 + c] = g.emission[c], o[10 + c] = g.attenuation[c], o[13 + c] = g.albedo_x_pscatter[c];
-            o[17 + c] = g.next.orig[c], o[20 + c] = g.next.dir[c];
+        write_segment(g, goes_on, g.hit ? (medium ? 2.0 : 1.0) : 0.0, g.hit ? (double)g.rec.prim_id : (double)RT_NONE, g.hit ? g.rec.t : INF,
+                      out28 + 28 * k);
+    }
+    return 0;
+}
+// shade_record on given rt_hit_records, the step rt_shade runs (include/rt2025.h): p, normal, u, v and the material are used as
+// given, front_face is != 0; t, prim_id and reserved are not read, nor anything of a miss but its kind.  A record of kind >
+// RT_HIT_MEDIUM, or a non-miss record with material >= n_materials, is an error and shades nothing; inst_id != RT_NONE with a
+// non-finite normal is the Transform panic.  out28 as orc_kat_shade_step, with hit = the record's kind, object RT_NONE and t NaN.
+int orc_kat_shade_record(const void* s, const rt_camera* cam, const rt_ray* rays, const rt_hit_record* records, const uint64_t* seeds,
+                         const uint32_t* ids, uint64_t n, double* out28) {
+    const Scene& sc = *(const Scene*)s;
+#pragma omp parallel for schedule(dynamic, 64)
+    for (int64_t k = 0; k < (int64_t)n; k++) {
+        PathCtx ctx;
+        ctx.seed = seeds[k], ctx.pixel = ids[3 * k], ctx.sample = ids[3 * k + 1], ctx.segment = ids[3 * k + 2];
+        Ray r(Vec3(rays[k].origin), Vec3(rays[k].direction), rays[k].time);
+        const rt_hit_record& h = records[k];
+        Segment g;
+        bool goes_on = false;
+        if (h.kind > RT_HIT_MEDIUM || (h.kind != RT_HIT_MISS && h.material >= sc.materials.size())) {
+            g.error = true;
+        } else if (h.kind == RT_HIT_MISS) {
+            goes_on = shade_record(sc, *cam, r, nullptr, ctx, g);
+        } else {
+            HitRecord rec;
+            rec.p = Vec3(h.p), rec.normal = Vec3(h.normal), rec.u = h.u, rec.v = h.v, rec.front_face = h.front_face != 0;
+            rec.mat = sc.materials[h.material].get();
+            rec.inst_id = h.inst_id;
+            rec.normal_panic = h.inst_id != RT_NONE && !(std::isfinite(h.normal[0]) && std::isfinite(h.normal[1]) && std::isfinite(h.normal[2]));
+            goes_on = shade_record(sc, *cam, r, &rec, ctx, g);
         }
-        o[9] = (double)g.kind;
-        o[16] = g.pdf_val;
-        o[23] = g.next.time;
-        o[24] = goes_on ? 1.0 : 0.0, o[25] = g.generated ? 1.0 : 0.0, o[26] = g.error ? 1.0 : 0.0, o[27] = g.fuzzed ? 1.0 : 0.0;
+        write_segment(g, goes_on, (double)h.kind, (double)RT_NONE, std::nan(""), out28 + 28 * k);
     }
     return 0;
 }

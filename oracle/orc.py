@@ -58,6 +58,7 @@ def lib():
         L.orc_kat_lights_pdf_value.argtypes = [C.c_void_p, D, D]
         L.orc_kat_lights_random.argtypes = [C.c_void_p, D, C.c_uint32, C.c_double, C.c_double, D]
         L.orc_kat_shade_step.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]
+        L.orc_kat_shade_record.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]
         L.orc_camera_ray.argtypes = [C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p]
         _lib = L
     return _lib
@@ -136,10 +137,21 @@ class OracleScene:
         seeds, ids3 = np.ascontiguousarray(seeds, dtype=np.uint64), np.ascontiguousarray(ids3, dtype=np.uint32).reshape(n, 3)
         out = np.zeros((n, 28))
         self.L.orc_kat_shade_step(self.h, C.byref(cam), rays.ctypes.data, seeds.ctypes.data, ids3.ctypes.data, n, out.ctypes.data)
-        return dict(hit=out[:, 0].astype(np.int64), object=out[:, 1].astype(np.uint32), t=out[:, 2], background=out[:, 3:6], emission=out[:, 6:9],
-                    kind=out[:, 9].astype(np.int64), attenuation=out[:, 10:13], albedo_x_pscatter=out[:, 13:16], pdf_val=out[:, 16],
-                    o=out[:, 17:20], d=out[:, 20:23], time=out[:, 23], goes_on=out[:, 24] != 0.0, generated=out[:, 25] != 0.0,
-                    error=out[:, 26] != 0.0, fuzzed=out[:, 27] != 0.0)
+        return _segments(out)
+
+    def shade_record(self, rays, records, seeds, ids3, camera=None):
+        """The step rt_shade runs, on given rt_hit_records (shade_record: ray_step after world.hit), with the draws addressed as in
+        shade_step.  -> the dict of shade_step; hit is the record's kind, object RT_NONE and t NaN (neither is read)."""
+        cam = camera if camera is not None else self.host.camera
+        rays = np.ascontiguousarray(rays, dtype=rt.rt_ray_dtype)
+        records = np.ascontiguousarray(records, dtype=rt.rt_hit_record_dtype)
+        n = len(rays)
+        assert len(records) == n
+        seeds, ids3 = np.ascontiguousarray(seeds, dtype=np.uint64), np.ascontiguousarray(ids3, dtype=np.uint32).reshape(n, 3)
+        out = np.zeros((n, 28))
+        self.L.orc_kat_shade_record(self.h, C.byref(cam), rays.ctypes.data, records.ctypes.data, seeds.ctypes.data, ids3.ctypes.data, n,
+                                    out.ctypes.data)
+        return _segments(out)
 
     def lights_pdf_value(self, origin, direction):
         return self.L.orc_kat_lights_pdf_value(self.h, d(*origin), d(*direction))
@@ -153,6 +165,14 @@ class OracleScene:
         out = (C.c_double * 3)()
         self.L.orc_texture_value(self.h, tex, u, v, d(*p), out)
         return np.array(out)
+
+
+def _segments(out):
+    """The 28 columns of orc_kat_shade_step / orc_kat_shade_record as named arrays."""
+    return dict(hit=out[:, 0].astype(np.int64), object=out[:, 1].astype(np.uint32), t=out[:, 2], background=out[:, 3:6], emission=out[:, 6:9],
+                kind=out[:, 9].astype(np.int64), attenuation=out[:, 10:13], albedo_x_pscatter=out[:, 13:16], pdf_val=out[:, 16],
+                o=out[:, 17:20], d=out[:, 20:23], time=out[:, 23], goes_on=out[:, 24] != 0.0, generated=out[:, 25] != 0.0,
+                error=out[:, 26] != 0.0, fuzzed=out[:, 27] != 0.0)
 
 
 def disney_evaluate(params15, thin, v_out, v_in, front_face):

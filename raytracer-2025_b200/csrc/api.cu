@@ -253,13 +253,18 @@ int check_device(int requested, int& device, int& sm_count) {
     return RT_OK;
 }
 
+// The batch limit of the ray queries and rt_shade, checked before anything is allocated or copied
+static int batch_refusal(uint64_t n) {
+    return n > 0xFFFFFFF0ull ? set_err(RT_ERR_INVALID, "more than 2^32 - 16 rays in one batch") : RT_OK;
+}
+
 // The body of the _device batch queries: the batch size check, RT_OPT_COUNT counters, event timing and `stats`.
 // launch(count, d_counters, grid, stream) enqueues the kernels and returns how many it launched.
 template <class Launch>
 int run_batch(const rt_scene* s, uint64_t n, uint32_t flags, void* stream, rt_stats* stats, Launch launch) {
     if (stats) std::memset(stats, 0, sizeof(*stats));
     if (n == 0) return RT_OK;
-    if (n > 0xFFFFFFF0ull) return set_err(RT_ERR_INVALID, "more than 2^32 rays in one batch");
+    if (const int refused = batch_refusal(n)) return refused;
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long* d_cnt = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
@@ -553,6 +558,7 @@ int rt_closest_hit(const rt_scene* s, const rt_ray* rays, uint64_t n, double t_m
         if (stats) std::memset(stats, 0, sizeof(*stats));
         return RT_OK;
     }
+    if (const int refused = batch_refusal(n)) return refused;
     rt_ray* d_rays = nullptr;
     rt_hit* d_out = nullptr;
     int rc = RT_OK;
@@ -591,6 +597,7 @@ int rt_occluded(const rt_scene* s, const rt_ray* rays, const double* t_max_per_r
         if (stats) std::memset(stats, 0, sizeof(*stats));
         return RT_OK;
     }
+    if (const int refused = batch_refusal(n)) return refused;
     rt_ray* d_rays = nullptr;
     double* d_tmax = nullptr;
     uint8_t* d_out = nullptr;
@@ -643,6 +650,7 @@ int rt_transmittance(const rt_scene* s, const rt_ray* rays, const double* t_max_
         if (stats) std::memset(stats, 0, sizeof(*stats));
         return RT_OK;
     }
+    if (const int refused = batch_refusal(n)) return refused;
     rt_ray* d_rays = nullptr;
     double* d_tmax = nullptr;
     double* d_out = nullptr;
@@ -696,6 +704,7 @@ int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_
         if (stats) std::memset(stats, 0, sizeof(*stats));
         return RT_OK;
     }
+    if (const int refused = batch_refusal(n)) return refused;
     rt_ray* d_rays = nullptr;
     double* d_tmax = nullptr;
     rt_hit_record* d_out = nullptr;
@@ -725,7 +734,8 @@ int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_
 }
 
 // The host-side refusals of rt_shade / rt_shade_device, made before anything is allocated or copied
-static int shade_refusal(const rt_scene* s, const rt_camera* cam, uint32_t segment, uint32_t flags) {
+static int shade_refusal(const rt_scene* s, const rt_camera* cam, uint64_t n, uint32_t segment, uint32_t flags) {
+    if (const int refused = batch_refusal(n)) return refused;
     if (flags != 0) return set_err(RT_ERR_INVALID, "rt_shade takes no flags (flags must be 0)");
     if (cam->background_tex >= s->info.n_textures) return set_err(RT_ERR_INVALID, "camera.background_tex out of range");
     if (segment >= cam->max_depth) return set_err(RT_ERR_INVALID, "segment >= camera.max_depth: the reference never runs that segment");
@@ -735,7 +745,7 @@ static int shade_refusal(const rt_scene* s, const rt_camera* cam, uint32_t segme
 int rt_shade_device(const rt_scene* s, const rt_camera* cam, const rt_hit_record* d_records, uint64_t n, uint64_t seed, uint32_t segment,
                     uint32_t flags, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, void* stream, rt_stats* stats) {
     if (!s || !cam || (n && (!d_records || !d_rays || !d_beta || !d_radiance || !d_state))) return set_err(RT_ERR_INVALID, "null argument");
-    if (const int refused = shade_refusal(s, cam, segment, flags)) return refused;
+    if (const int refused = shade_refusal(s, cam, n, segment, flags)) return refused;
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long* d_errors = nullptr;
     int rc = RT_OK;
@@ -774,7 +784,7 @@ int rt_shade_device(const rt_scene* s, const rt_camera* cam, const rt_hit_record
 int rt_shade(const rt_scene* s, const rt_camera* cam, const rt_hit_record* records, uint64_t n, uint64_t seed, uint32_t segment, uint32_t flags,
              rt_ray* rays, double* beta, double* radiance, uint8_t* state, rt_stats* stats) {
     if (!s || !cam || (n && (!records || !rays || !beta || !radiance || !state))) return set_err(RT_ERR_INVALID, "null argument");
-    if (const int refused = shade_refusal(s, cam, segment, flags)) return refused;
+    if (const int refused = shade_refusal(s, cam, n, segment, flags)) return refused;
     if (n == 0) {
         if (stats) std::memset(stats, 0, sizeof(*stats));
         return RT_OK;

@@ -14,9 +14,20 @@ class _Perlin(C.Structure):
     _fields_ = [("randvec", (C.c_double * 3) * 256), ("perm_x", C.c_uint32 * 256), ("perm_y", C.c_uint32 * 256), ("perm_z", C.c_uint32 * 256)]
 
 
+def _as_i64(x):
+    """Rust's `f64 as i64`: NaN -> 0, saturating at -2^63 and 2^63 - 1."""
+    if math.isnan(x):
+        return 0
+    if x >= 2.0 ** 63:
+        return 2 ** 63 - 1
+    if x <= -2.0 ** 63:
+        return -2 ** 63
+    return int(x)
+
+
 def _noise(t, p):  # perlin.rs:41-60
-    fl = [math.floor(x) for x in p]
-    i, j, k = (int(x) for x in fl)
+    fl = [float("nan") if math.isnan(x) else (x if math.isinf(x) else float(math.floor(x))) for x in p]
+    i, j, k = (_as_i64(x) for x in fl)  # (i + di) & 255 below: the low byte of the wrapping i64 sum
     u, v, w = (p[a] - fl[a] for a in range(3))
     uu, vv, ww = (x * x * (3.0 - 2.0 * x) for x in (u, v, w))  # perlin.rs:74
     accum = 0.0
@@ -57,15 +68,52 @@ def test_noise_texture_matches_a_plain_restatement(rt, orc):
     rng = np.random.default_rng(5)
     pts = [list(rng.uniform(-300.0, 300.0, 3)) for _ in range(400)]
     pts += [[0.5, -0.5, 2.5], [-1e-9, 255.999, -256.0], [1e5 + 0.25, -1e5 - 0.75, 3.125], [-0.0, 0.0, 0.0]]
+    pts += saturation_points(rng)
     worst = 0.0
     for p in pts:
         want = 0.5 * (1.0 + math.sin(scale * p[2] + 10.0 * _turb(tab, p, 7)))  # texture.rs:193-194
         got = osc.texture_value(tex, 0.0, 0.0, p)
-        assert got[0] == got[1] == got[2]
-        worst = max(worst, abs(got[0] - want))
+        assert got[0] == got[1] == got[2] or math.isnan(got[0])
+        assert math.isnan(got[0]) == math.isnan(want), (p, got[0], want)
+        if not math.isnan(want):
+            worst = max(worst, abs(got[0] - want))
     assert worst <= 4e-16, worst  # one ulp of a value in [0, 1]: libm's sin is the only operation that may differ
     # lattice points: noise is exactly zero, so turbulence is zero and the marble value is 0.5 (1 + sin(scale z))
     for p in ([3.0, -7.0, 12.0], [-255.0, 256.0, 0.0], [1024.0, 2.0, -5.0]):
         assert _noise(tab, p) == 0.0
         got = osc.texture_value(tex, 0.0, 0.0, p)
         assert got[0] == 0.5 * (1.0 + math.sin(scale * p[2]))
+
+
+# where `as i64` saturates: floor(p) at and around 2^63 (the largest double below it is 2^63 - 1024), infinities and NaN
+SATURATION = [9.1e18, 9.2e18, 9.21e18, 9.22e18, float(np.nextafter(2.0 ** 63, 0.0)), 2.0 ** 63, 1e19]
+SATURATION = SATURATION + [-x for x in SATURATION] + [float("inf"), float("-inf"), float("nan")]
+
+
+def saturation_points(rng):
+    """Each saturation value on each axis, the other two axes fractional."""
+    out = []
+    for x in SATURATION:
+        for a in range(3):
+            for _ in range(2):
+                p = list(rng.uniform(-50.0, 50.0, 3))
+                p[a] = x
+                out.append(p)
+    return out
+
+
+def test_noise_saturates_like_rust_as_i64(rt, orc):
+    """The lattice index of a coordinate at or beyond 2^63 is i64::MAX (i64::MIN below -2^63), not the value the last exact
+    conversion gives, and NaN is index 0.  A known answer of the marble texture at p = (9.21e18, 0.5, 0.3)."""
+    b = rt.Builder(17)
+    tex = b.noise(1.0)
+    hs = b.finish(b.list([b.sphere([0, 0, 0], 1.0, b.lambertian(tex))]), width=8, spp=1)
+    d = hs.desc.contents
+    tab = C.cast(d.perlins, C.POINTER(_Perlin)).contents
+    osc = orc.OracleScene(hs)
+    tex = C.c_uint32.from_address(d.materials + 176 * int(hs.objects()[0]["material"]) + 4).value
+    assert _as_i64(9.21e18) == 9210000000000000000 and _as_i64(2.0 ** 63) == 2 ** 63 - 1 and _as_i64(-1e19) == -2 ** 63
+    p = [9.21e18, 0.5, 0.3]
+    want = 0.5 * (1.0 + math.sin(p[2] + 10.0 * _turb(tab, p, 7)))
+    got = osc.texture_value(tex, 0.0, 0.0, p)
+    assert abs(got[0] - want) <= 4e-16 and abs(want - 0.8738799519358917) <= 4e-16, (got[0], want)
