@@ -452,6 +452,59 @@ int rt_shade_device(const rt_scene* scene, const rt_camera* camera /* host point
 int rt_camera_rays(const rt_camera* camera, uint64_t seed, uint32_t sample, rt_ray* out);
 int rt_camera_rays_device(const rt_camera* camera, uint64_t seed, uint32_t sample, rt_ray* d_out, void* stream);
 
+/* Path ids: the three entries above with the address of each row's draws given per row, so that a client
+ * loop runs any number of samples per pixel and may compact, permute and refill its batch.  The id is
+ * the render's own path id (rt2025_rng.h): a row's draws are philox(seed; pixel, sample, segment, slot).
+ * Ids are addresses and are not range-checked: a pixel beyond the image or a stratum >= sqrt_spp^2 gets
+ * what the same arithmetic gives.
+ *   - rt_camera_rays_ids: out[i] = Camera::get_ray of pixel (ids[i].pixel % image_width,
+ *     ids[i].pixel / image_width) and stratum ids[i].sample (s_i = sample / sqrt_spp, s_j = sample %
+ *     sqrt_spp), with the draws philox(seed; pixel, sample, 0, RT_SLOT_CAM_*); segment is not read.
+ *     Runs on the current device (no scene), like rt_camera_rays.  RT_ERR_INVALID for a null pointer,
+ *     n > 2^32 - 16, image_width == 0 or sqrt_spp == 0.
+ *   - rt_world_hit_ids: rt_world_hit, with the free-flight draw of media[m] for row i at
+ *     philox(seed; ids[i].pixel, ids[i].sample, ids[i].segment, RT_MEDIUM_SLOT(m)).  Only rows that take
+ *     draws (a scene with media and a non-empty interval) read their id.  Everything else, refusals and
+ *     stats included, is rt_world_hit's.
+ *   - rt_shade_ids: rt_shade, with the draws of row i addressed by ids[i] and ids[i].segment in place of
+ *     `segment`, in the draws and in the depth cut.  radiance + 3 i is still indexed by row: a client
+ *     that holds several samples of one pixel sums them itself.  A row that leaves with RT_PATH_ALIVE
+ *     gets ids[i].segment += 1; no other field of ids is ever written, and an inactive row reads and
+ *     writes nothing but its state byte.  An active row with ids[i].segment >= max_depth (a segment the
+ *     reference never runs) ends with RT_PATH_ERROR, counts in stats.errors, and nothing else of it is
+ *     read or written.  The refusals are rt_shade's but the segment test.
+ * Each pins its twin bit for bit:
+ *   - rt_world_hit(..., segment = s) equals rt_world_hit_ids with ids[i] = (i, 0, s);
+ *   - rt_shade(..., segment = s) equals rt_shade_ids with the same ids, apart from the segment update;
+ *   - rt_camera_rays(sample = s) equals rt_camera_rays_ids with ids[i] = (i, s, any).
+ * So the loop of rt_shade, with ids (pixel, stratum, 0) for every path and the rows summed into a
+ * framebuffer by pixel, reproduces rt_render at any sqrt_spp (INTEGRATION.md §5).  Host-pointer versions
+ * copy in and out (rt_shade_ids copies ids back); the _device versions take device pointers (the camera
+ * stays a host pointer) and enqueue on `stream`. */
+typedef struct rt_path_id {
+    uint32_t pixel;     /* the render's pixel index j * image_width + i */
+    uint32_t sample;    /* the stratum s_i * sqrt_spp + s_j */
+    uint32_t segment;   /* the number of world.hit calls made on the path before this one */
+    uint32_t reserved;  /* never read or written by the library */
+} rt_path_id;           /* 16 bytes */
+
+int rt_camera_rays_ids(const rt_camera* camera, uint64_t seed, const rt_path_id* ids, uint64_t n, rt_ray* out);
+int rt_camera_rays_ids_device(const rt_camera* camera, uint64_t seed, const rt_path_id* d_ids, uint64_t n,
+                              rt_ray* d_out, void* stream);
+int rt_world_hit_ids(const rt_scene* scene, const rt_ray* rays, const rt_path_id* ids,
+                     const double* t_max_per_ray /* n values or NULL */, uint64_t n, double t_min, double t_max,
+                     uint64_t seed, uint32_t flags, rt_hit_record* out, rt_stats* stats);
+int rt_world_hit_ids_device(const rt_scene* scene, const rt_ray* d_rays, const rt_path_id* d_ids,
+                            const double* d_t_max_per_ray, uint64_t n, double t_min, double t_max, uint64_t seed,
+                            uint32_t flags, rt_hit_record* d_out, void* stream, rt_stats* stats);
+int rt_shade_ids(const rt_scene* scene, const rt_camera* camera, const rt_hit_record* records, rt_path_id* ids,
+                 uint64_t n, uint64_t seed, uint32_t flags, rt_ray* rays, double* beta, double* radiance,
+                 uint8_t* state, rt_stats* stats);
+int rt_shade_ids_device(const rt_scene* scene, const rt_camera* camera /* host pointer */,
+                        const rt_hit_record* d_records, rt_path_id* d_ids, uint64_t n, uint64_t seed, uint32_t flags,
+                        rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, void* stream,
+                        rt_stats* stats);
+
 typedef enum rt_accum_type { RT_ACCUM_F32 = 0, RT_ACCUM_F64 = 1 } rt_accum_type;
 
 typedef struct rt_render_opts {

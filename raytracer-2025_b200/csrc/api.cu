@@ -314,6 +314,45 @@ int run_batch(const rt_scene* s, uint64_t n, uint32_t flags, void* stream, rt_st
     return rc;
 }
 
+// The body of rt_shade_device / rt_shade_ids_device after the refusals: the error word for `stats`, then run_batch with the grid of
+// SHADE_BLOCK-thread CTAs.  launch(P, d_errors, grid, stream) enqueues the one kernel.
+template <class Launch>
+int run_shade(const rt_scene* s, const rt_camera* cam, uint64_t n, uint64_t seed, void* stream, rt_stats* stats, Launch launch) {
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned long long* d_errors = nullptr;
+    int rc = RT_OK;
+    DeviceGuard guard;
+    try {
+        // the error count is only kept for `stats`: its word is allocated, cleared and read back outside the timed launch
+        if (stats && n) {
+            CU(cudaSetDevice(s->device));
+            CU(cudaMallocAsync((void**)&d_errors, sizeof(unsigned long long), st));
+            CU(cudaMemsetAsync(d_errors, 0, sizeof(unsigned long long), st));
+        }
+        rc = run_batch(s, n, 0, stream, stats, [&](bool, unsigned long long*, int, cudaStream_t bs) {
+            RenderParams P{};
+            P.cam = *cam;
+            P.seed = seed;
+            P.lights_flat = s->lights_flat;
+            int grid = s->sm_count * 8;
+            const uint64_t need = (n + SHADE_BLOCK - 1) / SHADE_BLOCK;
+            if ((uint64_t)grid > need) grid = (int)need;
+            launch(P, d_errors, grid, bs);
+            return 1;
+        });
+        if (rc == RT_OK && d_errors) {
+            unsigned long long h_errors = 0;
+            CU(cudaMemcpyAsync(&h_errors, d_errors, sizeof(h_errors), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            stats->errors = h_errors;
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    if (d_errors) cudaFreeAsync(d_errors, st);
+    return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -679,33 +718,53 @@ int rt_transmittance(const rt_scene* s, const rt_ray* rays, const double* t_max_
     return rc;
 }
 
-int rt_world_hit_device(const rt_scene* s, const rt_ray* d_rays, const double* d_t_max_per_ray, uint64_t n, double t_min, double t_max,
-                        uint64_t seed, uint32_t segment, uint32_t flags, rt_hit_record* d_out, void* stream, rt_stats* stats) {
-    if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
+// The body of rt_world_hit_device / rt_world_hit_ids_device: the surface pass into a stream-ordered scratch buffer (16 bytes per
+// ray), then the record pass, with the draws of row i at (i, 0, segment) or, when d_ids is given, at d_ids[i].
+static int world_hit_batch(const rt_scene* s, const rt_ray* d_rays, const rt_path_id* d_ids, const double* d_t_max_per_ray, uint64_t n,
+                           double t_min, double t_max, uint64_t seed, uint32_t segment, uint32_t flags, rt_hit_record* d_out, void* stream,
+                           rt_stats* stats) {
     return run_batch(s, n, flags, stream, stats, [&](bool count, unsigned long long* d_cnt, int grid, cudaStream_t st) {
-        // the surface pass writes the surface winner of every ray (16 bytes) to a stream-ordered scratch buffer; the record pass reads it
+        // the record pass reads the surface winner of every ray from the scratch buffer
         HitRec* d_surface = nullptr;
         CU(cudaMallocAsync((void**)&d_surface, n * sizeof(HitRec), st));
         launch_world_hit_surface(s->view, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, count, d_surface, d_cnt, grid, s->stack_bytes, st);
         int grid_m = s->sm_count * 8;
         const uint64_t need = (n + MEDIA_BLOCK - 1) / MEDIA_BLOCK;
         if ((uint64_t)grid_m > need) grid_m = (int)need;
-        launch_world_hit_record(s->view, s->generic_media, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, seed, segment, count, d_surface, d_out,
-                                d_cnt, grid_m, st);
+        if (d_ids)
+            launch_world_hit_record_ids(s->view, s->generic_media, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, seed, d_ids, count, d_surface,
+                                        d_out, d_cnt, grid_m, st);
+        else
+            launch_world_hit_record(s->view, s->generic_media, d_rays, d_t_max_per_ray, (uint32_t)n, t_min, t_max, seed, segment, count, d_surface,
+                                    d_out, d_cnt, grid_m, st);
         CU(cudaFreeAsync(d_surface, st));
         return 2;
     });
 }
 
-int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_ray, uint64_t n, double t_min, double t_max, uint64_t seed,
-                 uint32_t segment, uint32_t flags, rt_hit_record* out, rt_stats* stats) {
-    if (!s || (n && (!rays || !out))) return set_err(RT_ERR_INVALID, "null argument");
+int rt_world_hit_device(const rt_scene* s, const rt_ray* d_rays, const double* d_t_max_per_ray, uint64_t n, double t_min, double t_max,
+                        uint64_t seed, uint32_t segment, uint32_t flags, rt_hit_record* d_out, void* stream, rt_stats* stats) {
+    if (!s || (n && (!d_rays || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
+    return world_hit_batch(s, d_rays, nullptr, d_t_max_per_ray, n, t_min, t_max, seed, segment, flags, d_out, stream, stats);
+}
+
+int rt_world_hit_ids_device(const rt_scene* s, const rt_ray* d_rays, const rt_path_id* d_ids, const double* d_t_max_per_ray, uint64_t n,
+                            double t_min, double t_max, uint64_t seed, uint32_t flags, rt_hit_record* d_out, void* stream, rt_stats* stats) {
+    if (!s || (n && (!d_rays || !d_ids || !d_out))) return set_err(RT_ERR_INVALID, "null argument");
+    return world_hit_batch(s, d_rays, d_ids, d_t_max_per_ray, n, t_min, t_max, seed, 0, flags, d_out, stream, stats);
+}
+
+// The body of rt_world_hit / rt_world_hit_ids: copy in, the _device entry on the default stream, copy out.  `ids` is nullptr for
+// rt_world_hit.
+static int world_hit_host(const rt_scene* s, const rt_ray* rays, const rt_path_id* ids, const double* t_max_per_ray, uint64_t n, double t_min,
+                          double t_max, uint64_t seed, uint32_t segment, uint32_t flags, rt_hit_record* out, rt_stats* stats) {
     if (n == 0) {
         if (stats) std::memset(stats, 0, sizeof(*stats));
         return RT_OK;
     }
     if (const int refused = batch_refusal(n)) return refused;
     rt_ray* d_rays = nullptr;
+    rt_path_id* d_ids = nullptr;
     double* d_tmax = nullptr;
     rt_hit_record* d_out = nullptr;
     int rc = RT_OK;
@@ -715,11 +774,15 @@ int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_
         scratch_alloc(&d_rays, n * sizeof(rt_ray));
         scratch_alloc(&d_out, n * sizeof(rt_hit_record));
         CU(cudaMemcpy(d_rays, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice));
+        if (ids) {
+            scratch_alloc(&d_ids, n * sizeof(rt_path_id));
+            CU(cudaMemcpy(d_ids, ids, n * sizeof(rt_path_id), cudaMemcpyHostToDevice));
+        }
         if (t_max_per_ray) {
             scratch_alloc(&d_tmax, n * sizeof(double));
             CU(cudaMemcpy(d_tmax, t_max_per_ray, n * sizeof(double), cudaMemcpyHostToDevice));
         }
-        rc = rt_world_hit_device(s, d_rays, d_tmax, n, t_min, t_max, seed, segment, flags, d_out, nullptr, stats);
+        rc = world_hit_batch(s, d_rays, d_ids, d_tmax, n, t_min, t_max, seed, segment, flags, d_out, nullptr, stats);
         if (rc == RT_OK) {
             CU(cudaDeviceSynchronize());
             CU(cudaMemcpy(out, d_out, n * sizeof(rt_hit_record), cudaMemcpyDeviceToHost));
@@ -728,16 +791,33 @@ int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_
         rc = set_err(RT_ERR_CUDA, f.what);
     }
     scratch_free(d_rays);
+    scratch_free(d_ids);
     scratch_free(d_tmax);
     scratch_free(d_out);
     return rc;
 }
 
-// The host-side refusals of rt_shade / rt_shade_device, made before anything is allocated or copied
-static int shade_refusal(const rt_scene* s, const rt_camera* cam, uint64_t n, uint32_t segment, uint32_t flags) {
+int rt_world_hit(const rt_scene* s, const rt_ray* rays, const double* t_max_per_ray, uint64_t n, double t_min, double t_max, uint64_t seed,
+                 uint32_t segment, uint32_t flags, rt_hit_record* out, rt_stats* stats) {
+    if (!s || (n && (!rays || !out))) return set_err(RT_ERR_INVALID, "null argument");
+    return world_hit_host(s, rays, nullptr, t_max_per_ray, n, t_min, t_max, seed, segment, flags, out, stats);
+}
+
+int rt_world_hit_ids(const rt_scene* s, const rt_ray* rays, const rt_path_id* ids, const double* t_max_per_ray, uint64_t n, double t_min,
+                     double t_max, uint64_t seed, uint32_t flags, rt_hit_record* out, rt_stats* stats) {
+    if (!s || (n && (!rays || !ids || !out))) return set_err(RT_ERR_INVALID, "null argument");
+    return world_hit_host(s, rays, ids, t_max_per_ray, n, t_min, t_max, seed, 0, flags, out, stats);
+}
+
+// The host-side refusals of rt_shade / rt_shade_device and of their _ids forms, made before anything is allocated or copied
+static int shade_refusal(const rt_scene* s, const rt_camera* cam, uint64_t n, uint32_t flags) {
     if (const int refused = batch_refusal(n)) return refused;
     if (flags != 0) return set_err(RT_ERR_INVALID, "rt_shade takes no flags (flags must be 0)");
     if (cam->background_tex >= s->info.n_textures) return set_err(RT_ERR_INVALID, "camera.background_tex out of range");
+    return RT_OK;
+}
+// rt_shade's one segment for the whole batch (the _ids forms test each row's segment on the device)
+static int segment_refusal(const rt_camera* cam, uint32_t segment) {
     if (segment >= cam->max_depth) return set_err(RT_ERR_INVALID, "segment >= camera.max_depth: the reference never runs that segment");
     return RT_OK;
 }
@@ -745,51 +825,32 @@ static int shade_refusal(const rt_scene* s, const rt_camera* cam, uint64_t n, ui
 int rt_shade_device(const rt_scene* s, const rt_camera* cam, const rt_hit_record* d_records, uint64_t n, uint64_t seed, uint32_t segment,
                     uint32_t flags, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, void* stream, rt_stats* stats) {
     if (!s || !cam || (n && (!d_records || !d_rays || !d_beta || !d_radiance || !d_state))) return set_err(RT_ERR_INVALID, "null argument");
-    if (const int refused = shade_refusal(s, cam, n, segment, flags)) return refused;
-    cudaStream_t st = (cudaStream_t)stream;
-    unsigned long long* d_errors = nullptr;
-    int rc = RT_OK;
-    DeviceGuard guard;
-    try {
-        // the error count is only kept for `stats`: its word is allocated, cleared and read back outside the timed launch
-        if (stats && n) {
-            CU(cudaSetDevice(s->device));
-            CU(cudaMallocAsync((void**)&d_errors, sizeof(unsigned long long), st));
-            CU(cudaMemsetAsync(d_errors, 0, sizeof(unsigned long long), st));
-        }
-        rc = run_batch(s, n, 0, stream, stats, [&](bool, unsigned long long*, int, cudaStream_t bs) {
-            RenderParams P{};
-            P.cam = *cam;
-            P.seed = seed;
-            P.lights_flat = s->lights_flat;
-            int grid = s->sm_count * 8;
-            const uint64_t need = (n + SHADE_BLOCK - 1) / SHADE_BLOCK;
-            if ((uint64_t)grid > need) grid = (int)need;
-            launch_shade_records(s->view, P, d_records, n, s->info.n_materials, segment, d_rays, d_beta, d_radiance, d_state, d_errors, grid, bs);
-            return 1;
-        });
-        if (rc == RT_OK && d_errors) {
-            unsigned long long h_errors = 0;
-            CU(cudaMemcpyAsync(&h_errors, d_errors, sizeof(h_errors), cudaMemcpyDeviceToHost, st));
-            CU(cudaStreamSynchronize(st));
-            stats->errors = h_errors;
-        }
-    } catch (const CudaFail& f) {
-        rc = set_err(RT_ERR_CUDA, f.what);
-    }
-    if (d_errors) cudaFreeAsync(d_errors, st);
-    return rc;
+    if (const int refused = shade_refusal(s, cam, n, flags)) return refused;
+    if (const int refused = segment_refusal(cam, segment)) return refused;
+    return run_shade(s, cam, n, seed, stream, stats, [&](const RenderParams& P, unsigned long long* d_errors, int grid, cudaStream_t bs) {
+        launch_shade_records(s->view, P, d_records, n, s->info.n_materials, segment, d_rays, d_beta, d_radiance, d_state, d_errors, grid, bs);
+    });
 }
 
-int rt_shade(const rt_scene* s, const rt_camera* cam, const rt_hit_record* records, uint64_t n, uint64_t seed, uint32_t segment, uint32_t flags,
-             rt_ray* rays, double* beta, double* radiance, uint8_t* state, rt_stats* stats) {
-    if (!s || !cam || (n && (!records || !rays || !beta || !radiance || !state))) return set_err(RT_ERR_INVALID, "null argument");
-    if (const int refused = shade_refusal(s, cam, n, segment, flags)) return refused;
+int rt_shade_ids_device(const rt_scene* s, const rt_camera* cam, const rt_hit_record* d_records, rt_path_id* d_ids, uint64_t n, uint64_t seed,
+                        uint32_t flags, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, void* stream, rt_stats* stats) {
+    if (!s || !cam || (n && (!d_records || !d_ids || !d_rays || !d_beta || !d_radiance || !d_state))) return set_err(RT_ERR_INVALID, "null argument");
+    if (const int refused = shade_refusal(s, cam, n, flags)) return refused;
+    return run_shade(s, cam, n, seed, stream, stats, [&](const RenderParams& P, unsigned long long* d_errors, int grid, cudaStream_t bs) {
+        launch_shade_records_ids(s->view, P, d_records, n, s->info.n_materials, d_ids, d_rays, d_beta, d_radiance, d_state, d_errors, grid, bs);
+    });
+}
+
+// The body of rt_shade / rt_shade_ids after the refusals: copy in, the _device entry on the default stream, copy out.  `ids` is
+// nullptr for rt_shade.
+static int shade_host(const rt_scene* s, const rt_camera* cam, const rt_hit_record* records, rt_path_id* ids, uint64_t n, uint64_t seed,
+                      uint32_t segment, uint32_t flags, rt_ray* rays, double* beta, double* radiance, uint8_t* state, rt_stats* stats) {
     if (n == 0) {
         if (stats) std::memset(stats, 0, sizeof(*stats));
         return RT_OK;
     }
     rt_hit_record* d_rec = nullptr;
+    rt_path_id* d_ids = nullptr;
     rt_ray* d_rays = nullptr;
     double *d_beta = nullptr, *d_rad = nullptr;
     uint8_t* d_state = nullptr;
@@ -807,23 +868,46 @@ int rt_shade(const rt_scene* s, const rt_camera* cam, const rt_hit_record* recor
         CU(cudaMemcpy(d_beta, beta, n * 3 * sizeof(double), cudaMemcpyHostToDevice));
         CU(cudaMemcpy(d_rad, radiance, n * 3 * sizeof(double), cudaMemcpyHostToDevice));
         CU(cudaMemcpy(d_state, state, n, cudaMemcpyHostToDevice));
-        rc = rt_shade_device(s, cam, d_rec, n, seed, segment, flags, d_rays, d_beta, d_rad, d_state, nullptr, stats);
+        if (ids) {
+            scratch_alloc(&d_ids, n * sizeof(rt_path_id));
+            CU(cudaMemcpy(d_ids, ids, n * sizeof(rt_path_id), cudaMemcpyHostToDevice));
+            rc = rt_shade_ids_device(s, cam, d_rec, d_ids, n, seed, flags, d_rays, d_beta, d_rad, d_state, nullptr, stats);
+        } else {
+            rc = rt_shade_device(s, cam, d_rec, n, seed, segment, flags, d_rays, d_beta, d_rad, d_state, nullptr, stats);
+        }
         if (rc == RT_OK) {
             CU(cudaDeviceSynchronize());
             CU(cudaMemcpy(rays, d_rays, n * sizeof(rt_ray), cudaMemcpyDeviceToHost));
             CU(cudaMemcpy(beta, d_beta, n * 3 * sizeof(double), cudaMemcpyDeviceToHost));
             CU(cudaMemcpy(radiance, d_rad, n * 3 * sizeof(double), cudaMemcpyDeviceToHost));
             CU(cudaMemcpy(state, d_state, n, cudaMemcpyDeviceToHost));
+            if (ids) CU(cudaMemcpy(ids, d_ids, n * sizeof(rt_path_id), cudaMemcpyDeviceToHost));
         }
     } catch (const CudaFail& f) {
         rc = set_err(RT_ERR_CUDA, f.what);
     }
     scratch_free(d_rec);
+    scratch_free(d_ids);
     scratch_free(d_rays);
     scratch_free(d_beta);
     scratch_free(d_rad);
     scratch_free(d_state);
     return rc;
+}
+
+int rt_shade(const rt_scene* s, const rt_camera* cam, const rt_hit_record* records, uint64_t n, uint64_t seed, uint32_t segment, uint32_t flags,
+             rt_ray* rays, double* beta, double* radiance, uint8_t* state, rt_stats* stats) {
+    if (!s || !cam || (n && (!records || !rays || !beta || !radiance || !state))) return set_err(RT_ERR_INVALID, "null argument");
+    if (const int refused = shade_refusal(s, cam, n, flags)) return refused;
+    if (const int refused = segment_refusal(cam, segment)) return refused;
+    return shade_host(s, cam, records, nullptr, n, seed, segment, flags, rays, beta, radiance, state, stats);
+}
+
+int rt_shade_ids(const rt_scene* s, const rt_camera* cam, const rt_hit_record* records, rt_path_id* ids, uint64_t n, uint64_t seed, uint32_t flags,
+                 rt_ray* rays, double* beta, double* radiance, uint8_t* state, rt_stats* stats) {
+    if (!s || !cam || (n && (!records || !ids || !rays || !beta || !radiance || !state))) return set_err(RT_ERR_INVALID, "null argument");
+    if (const int refused = shade_refusal(s, cam, n, flags)) return refused;
+    return shade_host(s, cam, records, ids, n, seed, 0, flags, rays, beta, radiance, state, stats);
 }
 
 int rt_camera_rays_device(const rt_camera* cam, uint64_t seed, uint32_t sample, rt_ray* d_out, void* stream) {
@@ -862,6 +946,54 @@ int rt_camera_rays(const rt_camera* cam, uint64_t seed, uint32_t sample, rt_ray*
     } catch (const CudaFail& f) {
         rc = set_err(RT_ERR_CUDA, f.what);
     }
+    if (d) cudaFreeAsync(d, st);
+    return rc;
+}
+
+// The host-side refusals of rt_camera_rays_ids / _device: ids are addresses and are not range-checked, but the stratum arithmetic
+// divides by image_width and sqrt_spp
+static int camera_rays_ids_refusal(const rt_camera* cam, const rt_path_id* ids, uint64_t n, const rt_ray* out) {
+    if (!cam || (n && (!ids || !out))) return set_err(RT_ERR_INVALID, "null argument");
+    if (const int refused = batch_refusal(n)) return refused;
+    if (cam->image_width == 0) return set_err(RT_ERR_INVALID, "camera.image_width == 0");
+    if (cam->sqrt_spp == 0) return set_err(RT_ERR_INVALID, "camera.sqrt_spp == 0");
+    return RT_OK;
+}
+
+int rt_camera_rays_ids_device(const rt_camera* cam, uint64_t seed, const rt_path_id* d_ids, uint64_t n, rt_ray* d_out, void* stream) {
+    if (const int refused = camera_rays_ids_refusal(cam, d_ids, n, d_out)) return refused;
+    int device, sms;
+    int rc = check_device(-1, device, sms);
+    if (rc != RT_OK || n == 0) return rc;
+    int grid = sms * 8;
+    if ((uint64_t)grid > (n + 255) / 256) grid = (int)((n + 255) / 256);
+    launch_camera_rays_ids(*cam, seed, d_ids, n, d_out, grid, (cudaStream_t)stream);
+    if (cudaGetLastError() != cudaSuccess) return set_err(RT_ERR_CUDA, "k_camera_rays_ids launch failed");
+    return RT_OK;
+}
+
+int rt_camera_rays_ids(const rt_camera* cam, uint64_t seed, const rt_path_id* ids, uint64_t n, rt_ray* out) {
+    if (const int refused = camera_rays_ids_refusal(cam, ids, n, out)) return refused;
+    int device, sms;
+    int rc = check_device(-1, device, sms);
+    if (rc != RT_OK || n == 0) return rc;
+    keep_pool_memory(device);
+    rt_path_id* d_ids = nullptr;
+    rt_ray* d = nullptr;
+    cudaStream_t st = cudaStreamPerThread;
+    try {
+        CU(cudaMallocAsync((void**)&d_ids, n * sizeof(rt_path_id), st));
+        CU(cudaMallocAsync((void**)&d, n * sizeof(rt_ray), st));
+        CU(cudaMemcpyAsync(d_ids, ids, n * sizeof(rt_path_id), cudaMemcpyHostToDevice, st));
+        rc = rt_camera_rays_ids_device(cam, seed, d_ids, n, d, st);
+        if (rc == RT_OK) {
+            CU(cudaMemcpyAsync(out, d, n * sizeof(rt_ray), cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+        }
+    } catch (const CudaFail& f) {
+        rc = set_err(RT_ERR_CUDA, f.what);
+    }
+    if (d_ids) cudaFreeAsync(d_ids, st);
     if (d) cudaFreeAsync(d, st);
     return rc;
 }

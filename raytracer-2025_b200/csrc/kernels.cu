@@ -699,11 +699,13 @@ __global__ void __launch_bounds__(MEDIA_BLOCK) k_transmittance(SceneView sv, con
 // Every medium competes on the caller's interval [tmin, t_max_i] as ConstantMedium::hit (volume.rs:37-73) does there, with the
 // free-flight draw philox(seed; pixel = i, sample = 0, segment, RT_MEDIUM_SLOT(medium_index)); the nearest t wins, an exact tie
 // goes to the lower rank.  The winner's HitRecord is rebuilt in world space.  GENERIC / XF as in k_transmittance.
-template <bool COUNT, bool GENERIC, bool XF>
+// IDS (rt_world_hit_ids): the draws are addressed by ids[i] = (pixel, sample, segment) instead of (i, 0, segment), and ids[i] is
+// only loaded for a row that takes draws; `segment` is not read.  The IDS instantiations are made after the render kernels.
+template <bool COUNT, bool GENERIC, bool XF, bool IDS>
 __global__ void __launch_bounds__(MEDIA_BLOCK) k_world_hit_record(SceneView sv, const rt_ray* __restrict__ rays, const double* __restrict__ tmax_per_ray,
                                                                 uint32_t n, double tmin, double tmax, uint64_t seed, uint32_t segment,
                                                                 const HitRec* __restrict__ surface, rt_hit_record* __restrict__ out,
-                                                                unsigned long long* counters) {
+                                                                unsigned long long* counters, const rt_path_id* __restrict__ ids) {
     extern __shared__ float4 s_mem[];  // traversal stacks for boundaries that are not a single sphere
     uint32_t* stack = reinterpret_cast<uint32_t*>(s_mem) + threadIdx.x;
     TraceCounters cnt{0, 0};
@@ -723,6 +725,8 @@ __global__ void __launch_bounds__(MEDIA_BLOCK) k_world_hit_record(SceneView sv, 
             r.time = rp[6];
         }
         uint32_t rank = kind == HIT_SURFACE ? sv.meta[prim].rank : 0xFFFFFFFFu;
+        uint32_t pixel = i, sample = 0u, seg = segment;
+        if (IDS && media) pixel = ids[i].pixel, sample = ids[i].sample, seg = ids[i].segment;
         MediumDraws draws;
         for (uint32_t m = 0; media && m < sv.n_media; m++) {
             const Medium& med = sv.media[m];
@@ -742,7 +746,7 @@ __global__ void __launch_bounds__(MEDIA_BLOCK) k_world_hit_record(SceneView sv, 
             if (t1 < 0.0) t1 = 0.0;
             const double ray_length = length(lr.d);
             const double distance_inside_boundary = (t2 - t1) * ray_length;
-            const double hit_distance = med.neg_inv_density * log(draws.get(seed, i, 0u, segment, med.medium_index));
+            const double hit_distance = med.neg_inv_density * log(draws.get(seed, pixel, sample, seg, med.medium_index));
             if (hit_distance > distance_inside_boundary) continue;
             const double tm = t1 + hit_distance / ray_length;
             // the medium competes with the other children of its container like any hit
@@ -1368,11 +1372,11 @@ void launch_world_hit_record(const SceneView& sv, bool generic, const rt_ray* d_
     mv.n_cached_nodes = 0;
     const size_t media_smem = generic ? (size_t)sv.media_stack_entries * MEDIA_BLOCK * sizeof(uint32_t) : 0;  // <= 64 KB, opted in by kernel_setup
     const bool xf = sv.media_xform != 0;
-    auto k = generic ? (count ? (xf ? k_world_hit_record<true, true, true> : k_world_hit_record<true, true, false>)
-                              : (xf ? k_world_hit_record<false, true, true> : k_world_hit_record<false, true, false>))
-                     : (count ? (xf ? k_world_hit_record<true, false, true> : k_world_hit_record<true, false, false>)
-                              : (xf ? k_world_hit_record<false, false, true> : k_world_hit_record<false, false, false>));
-    k<<<grid, MEDIA_BLOCK, media_smem, s>>>(mv, d_rays, d_tmax_per_ray, n, tmin, tmax, seed, segment, d_surface, d_out, d_counters);
+    auto k = generic ? (count ? (xf ? k_world_hit_record<true, true, true, false> : k_world_hit_record<true, true, false, false>)
+                              : (xf ? k_world_hit_record<false, true, true, false> : k_world_hit_record<false, true, false, false>))
+                     : (count ? (xf ? k_world_hit_record<true, false, true, false> : k_world_hit_record<true, false, false, false>)
+                              : (xf ? k_world_hit_record<false, false, true, false> : k_world_hit_record<false, false, false, false>));
+    k<<<grid, MEDIA_BLOCK, media_smem, s>>>(mv, d_rays, d_tmax_per_ray, n, tmin, tmax, seed, segment, d_surface, d_out, d_counters, nullptr);
 }
 template <uint32_t CLS>
 static void launch_shade_cls(const SceneView& sv, const RenderParams& P, const WavefrontState& W, uint32_t queue, int grid, cudaStream_t s) {
@@ -1455,10 +1459,13 @@ void launch_world_hit_surface(const SceneView& sv, const rt_ray* d_rays, const d
 // rt_shade: the step of ray_color after world.hit (camera.rs:288-321) for a batch of rt_hit_records, one row per thread, the
 // general instantiation of the render's step (shade_hit<SC_OTHER> + end_segment) with the draws philox(seed; pixel = i,
 // sample = 0, segment, slot).  contribute() adds to radiance + 3 i.  Defined after the render kernels, as the world-hit family.
+// IDS (rt_shade_ids): the draws and the depth cut of row i are those of ids[i] = (pixel, sample, segment), `segment` is not read;
+// a row at segment >= max_depth ends with RT_PATH_ERROR and nothing else of it is touched, a survivor's ids[i].segment goes up by one.
+template <bool IDS>
 __global__ void __launch_bounds__(SHADE_BLOCK, shade_blocks(SC_OTHER, false))
     k_shade_records(SceneView sv, RenderParams P, const rt_hit_record* __restrict__ records, uint64_t n, uint32_t n_materials, uint32_t segment,
                     rt_ray* __restrict__ rays, double* __restrict__ beta, double* __restrict__ radiance, uint8_t* __restrict__ state,
-                    unsigned long long* n_errors) {
+                    unsigned long long* n_errors, rt_path_id* __restrict__ ids) {
     // contribute() and end_segment() count errors at &W.counters->errors: that is this thread's own word of s_errors (address
     // arithmetic on integers, as tests/device_kat.cu does), so that a row knows whether its segment added one
     __shared__ unsigned long long s_errors[SHADE_BLOCK];
@@ -1468,8 +1475,18 @@ __global__ void __launch_bounds__(SHADE_BLOCK, shade_blocks(SC_OTHER, false))
     unsigned long long errors = 0;
     for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
         if (!(state[i] & RT_PATH_ALIVE)) continue;  // an inactive row: nothing else of it is read or written
+        uint32_t pixel = (uint32_t)i, sample = 0u, seg = segment;
+        if (IDS) {
+            pixel = ids[i].pixel, sample = ids[i].sample, seg = ids[i].segment;
+            if (seg >= P.cam.max_depth) {  // the reference never runs that segment
+                state[i] = (uint8_t)RT_PATH_ERROR;
+                errors++;
+                continue;
+            }
+            // contribute() adds to W.accum + 3 pixel, and the row's own radiance is radiance + 3 i (address arithmetic on integers)
+            W.accum = reinterpret_cast<double*>(reinterpret_cast<uintptr_t>(radiance + 3 * i) - (uintptr_t)pixel * (3 * sizeof(double)));
+        }
         s_errors[threadIdx.x] = 0;
-        const uint32_t pixel = (uint32_t)i;
         const double* rp = reinterpret_cast<const double*>(rays + i);
         RayD r;
         r.o = D3{rp[0], rp[1], rp[2]};
@@ -1501,9 +1518,9 @@ __global__ void __launch_bounds__(SHADE_BLOCK, shade_blocks(SC_OTHER, false))
             // through the rest of the chain (scaling and rotating keep an inf or NaN component), and a chain of finite steps ends
             // finite, so the record's normal tells it exactly.
             const bool hit_ok = rec.inst_id == RT_NONE || finite3(h.normal);
-            shade_hit<SC_OTHER>(sv, P, W, r, b, pixel, 0u, segment, h, hit_ok, nr, nbeta, alive, error, nullptr);
+            shade_hit<SC_OTHER>(sv, P, W, r, b, pixel, sample, seg, h, hit_ok, nr, nbeta, alive, error, nullptr);
         }
-        alive = end_segment(P, W, segment, alive, error, nbeta);
+        alive = end_segment(P, W, seg, alive, error, nbeta);
         const bool err = s_errors[threadIdx.x] != 0;  // a panic, or a NaN contribution contribute() dropped
         errors += err ? 1u : 0u;
         if (alive) {
@@ -1512,6 +1529,7 @@ __global__ void __launch_bounds__(SHADE_BLOCK, shade_blocks(SC_OTHER, false))
             wp[3] = nr.d.x, wp[4] = nr.d.y, wp[5] = nr.d.z;
             wp[6] = nr.time;
             beta[3 * i + 0] = nbeta.x, beta[3 * i + 1] = nbeta.y, beta[3 * i + 2] = nbeta.z;
+            if (IDS) ids[i].segment = seg + 1;
         }
         state[i] = (uint8_t)((alive ? RT_PATH_ALIVE : 0u) | (err ? RT_PATH_ERROR : 0u));
     }
@@ -1520,7 +1538,8 @@ __global__ void __launch_bounds__(SHADE_BLOCK, shade_blocks(SC_OTHER, false))
 void launch_shade_records(const SceneView& sv, const RenderParams& P, const rt_hit_record* d_records, uint64_t n, uint32_t n_materials,
                           uint32_t segment, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, unsigned long long* d_errors,
                           int grid, cudaStream_t s) {
-    k_shade_records<<<grid, SHADE_BLOCK, 0, s>>>(sv, P, d_records, n, n_materials, segment, d_rays, d_beta, d_radiance, d_state, d_errors);
+    k_shade_records<false><<<grid, SHADE_BLOCK, 0, s>>>(sv, P, d_records, n, n_materials, segment, d_rays, d_beta, d_radiance, d_state, d_errors,
+                                                        nullptr);
 }
 
 // rt_camera_rays: Camera::get_ray of stratum `sample` through every pixel, k_generate's camera_ray, in the render's pixel order
@@ -1536,6 +1555,41 @@ __global__ void __launch_bounds__(256) k_camera_rays(rt_camera cam, uint64_t see
 }
 void launch_camera_rays(const rt_camera& cam, uint64_t seed, uint32_t sample, uint64_t n, rt_ray* d_out, int grid, cudaStream_t s) {
     k_camera_rays<<<grid, 256, 0, s>>>(cam, seed, sample, n, d_out);
+}
+
+// The path-id forms of the three kernels above (rt_world_hit_ids, rt_shade_ids, rt_camera_rays_ids): the draws of row i are
+// addressed by ids[i] instead of (i, sample, segment).  Instantiated here, after the render kernels, as their twins.
+void launch_world_hit_record_ids(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin,
+                                 double tmax, uint64_t seed, const rt_path_id* d_ids, bool count, const HitRec* d_surface, rt_hit_record* d_out,
+                                 unsigned long long* d_counters, int grid, cudaStream_t s) {
+    SceneView mv = sv;  // global-memory nodes only, as launch_world_hit_record
+    mv.n_cached_nodes = 0;
+    const size_t media_smem = generic ? (size_t)sv.media_stack_entries * MEDIA_BLOCK * sizeof(uint32_t) : 0;  // <= 64 KB, opted in by kernel_setup
+    const bool xf = sv.media_xform != 0;
+    auto k = generic ? (count ? (xf ? k_world_hit_record<true, true, true, true> : k_world_hit_record<true, true, false, true>)
+                              : (xf ? k_world_hit_record<false, true, true, true> : k_world_hit_record<false, true, false, true>))
+                     : (count ? (xf ? k_world_hit_record<true, false, true, true> : k_world_hit_record<true, false, false, true>)
+                              : (xf ? k_world_hit_record<false, false, true, true> : k_world_hit_record<false, false, false, true>));
+    k<<<grid, MEDIA_BLOCK, media_smem, s>>>(mv, d_rays, d_tmax_per_ray, n, tmin, tmax, seed, 0u, d_surface, d_out, d_counters, d_ids);
+}
+void launch_shade_records_ids(const SceneView& sv, const RenderParams& P, const rt_hit_record* d_records, uint64_t n, uint32_t n_materials,
+                              rt_path_id* d_ids, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, unsigned long long* d_errors,
+                              int grid, cudaStream_t s) {
+    k_shade_records<true><<<grid, SHADE_BLOCK, 0, s>>>(sv, P, d_records, n, n_materials, 0u, d_rays, d_beta, d_radiance, d_state, d_errors, d_ids);
+}
+__global__ void __launch_bounds__(256) k_camera_rays_ids(rt_camera cam, uint64_t seed, const rt_path_id* __restrict__ ids, uint64_t n,
+                                                          rt_ray* __restrict__ out) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        RayD r;
+        camera_ray(cam, seed, ids[i].pixel, ids[i].sample, r);
+        double* wp = reinterpret_cast<double*>(out + i);
+        wp[0] = r.o.x, wp[1] = r.o.y, wp[2] = r.o.z;
+        wp[3] = r.d.x, wp[4] = r.d.y, wp[5] = r.d.z;
+        wp[6] = r.time;
+    }
+}
+void launch_camera_rays_ids(const rt_camera& cam, uint64_t seed, const rt_path_id* d_ids, uint64_t n, rt_ray* d_out, int grid, cudaStream_t s) {
+    k_camera_rays_ids<<<grid, 256, 0, s>>>(cam, seed, d_ids, n, d_out);
 }
 
 int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks_per_sm, int* walk_blocks_per_sm) {
@@ -1560,8 +1614,10 @@ int kernel_setup(size_t smem_bytes, int* extend_blocks_per_sm, int* shade_blocks
                                 (const void*)k_media<true, 2, false, false>, (const void*)k_media<true, 2, true, false>,
                                 (const void*)k_transmittance<false, true, false>, (const void*)k_transmittance<false, true, true>,
                                 (const void*)k_transmittance<true, true, false>, (const void*)k_transmittance<true, true, true>,
-                                (const void*)k_world_hit_record<false, true, false>, (const void*)k_world_hit_record<false, true, true>,
-                                (const void*)k_world_hit_record<true, true, false>, (const void*)k_world_hit_record<true, true, true>};
+                                (const void*)k_world_hit_record<false, true, false, false>, (const void*)k_world_hit_record<false, true, true, false>,
+                                (const void*)k_world_hit_record<true, true, false, false>, (const void*)k_world_hit_record<true, true, true, false>,
+                                (const void*)k_world_hit_record<false, true, false, true>, (const void*)k_world_hit_record<false, true, true, true>,
+                                (const void*)k_world_hit_record<true, true, false, true>, (const void*)k_world_hit_record<true, true, true, true>};
     for (const void* f : media_smem)
         if ((e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, TRAVERSAL_STACK * MEDIA_BLOCK * (int)sizeof(uint32_t))) != cudaSuccess) return (int)e;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(extend_blocks_per_sm, k_extend<false, false, 0, 0>, EXTEND_BLOCK, smem_bytes);

@@ -163,6 +163,16 @@ void launch_shade_records(const SceneView& sv, const RenderParams& P, const rt_h
                           int grid, cudaStream_t s);
 // rt_camera_rays: d_out[pixel] = Camera::get_ray of stratum `sample` (k_generate's camera_ray), `grid` CTAs of 256 threads
 void launch_camera_rays(const rt_camera& cam, uint64_t seed, uint32_t sample, uint64_t n, rt_ray* d_out, int grid, cudaStream_t s);
+// The path-id forms (rt_world_hit_ids, rt_shade_ids, rt_camera_rays_ids): as the three above, with the draws of row i addressed by
+// d_ids[i] = (pixel, sample, segment).  launch_shade_records_ids takes each row's segment from d_ids (a row at segment >= max_depth
+// ends with RT_PATH_ERROR) and adds one to it on the rows that go on.  launch_camera_rays_ids writes d_out[i] for i < n.
+void launch_world_hit_record_ids(const SceneView& sv, bool generic, const rt_ray* d_rays, const double* d_tmax_per_ray, uint32_t n, double tmin,
+                                 double tmax, uint64_t seed, const rt_path_id* d_ids, bool count, const HitRec* d_surface, rt_hit_record* d_out,
+                                 unsigned long long* d_counters, int grid, cudaStream_t s);
+void launch_shade_records_ids(const SceneView& sv, const RenderParams& P, const rt_hit_record* d_records, uint64_t n, uint32_t n_materials,
+                              rt_path_id* d_ids, rt_ray* d_rays, double* d_beta, double* d_radiance, uint8_t* d_state, unsigned long long* d_errors,
+                              int grid, cudaStream_t s);
+void launch_camera_rays_ids(const rt_camera& cam, uint64_t seed, const rt_path_id* d_ids, uint64_t n, rt_ray* d_out, int grid, cudaStream_t s);
 void launch_init(const WavefrontState& W, const RenderParams& P, int grid, cudaStream_t s);
 void launch_generate(const SceneView& sv, const RenderParams& P, const WavefrontState& W, int grid, cudaStream_t s);
 void launch_extend(const SceneView& sv, const RenderParams& P, const WavefrontState& W, bool count, int grid, size_t smem_bytes, cudaStream_t s);

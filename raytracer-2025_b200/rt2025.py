@@ -27,7 +27,8 @@ RT_PATH_ALIVE, RT_PATH_ERROR = 1, 2  # rt_shade path state bits
 ABI_SYMBOLS = [
     "rt_scene_create", "rt_scene_destroy", "rt_closest_hit", "rt_closest_hit_device", "rt_occluded", "rt_occluded_device", "rt_transmittance",
     "rt_transmittance_device", "rt_world_hit", "rt_world_hit_device", "rt_shade", "rt_shade_device",
-    "rt_camera_rays", "rt_camera_rays_device", "rt_render",
+    "rt_camera_rays", "rt_camera_rays_device", "rt_camera_rays_ids", "rt_camera_rays_ids_device", "rt_world_hit_ids",
+    "rt_world_hit_ids_device", "rt_shade_ids", "rt_shade_ids_device", "rt_render",
     "rt_render_device", "rt_render_rgb8", "rt_render_multi", "rt_render_multi_rgb8", "rt_tonemap", "rt_tonemap_device", "rt_scene_get_info", "rt_scene_get_ranks", "rt_last_error",
     "rt_abi_version", "rt_device_count",
 ]
@@ -130,6 +131,9 @@ assert rt_ray_dtype.itemsize == 56 and rt_hit_dtype.itemsize == 24 and rt_object
 rt_hit_record_dtype = np.dtype([("t", "<f8"), ("p", "<f8", (3,)), ("normal", "<f8", (3,)), ("u", "<f8"), ("v", "<f8"), ("kind", "<u4"),
                                 ("front_face", "<u4"), ("prim_id", "<u4"), ("inst_id", "<u4"), ("material", "<u4"), ("reserved", "<u4")])
 assert rt_hit_record_dtype.itemsize == 96
+# the address of a row's draws in the path-id entries: (pixel j * W + i, stratum, segment); `reserved` is never read or written
+rt_path_id_dtype = np.dtype([("pixel", "<u4"), ("sample", "<u4"), ("segment", "<u4"), ("reserved", "<u4")])
+assert rt_path_id_dtype.itemsize == 16
 
 
 def build_native(targets=("product", "host")):
@@ -243,6 +247,17 @@ def product_lib(required=True):
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
             L.rt_camera_rays.argtypes = [C.POINTER(rt_camera), C.c_uint64, C.c_uint32, C.c_void_p]
             L.rt_camera_rays_device.argtypes = [C.POINTER(rt_camera), C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p]
+        if hasattr(L, "rt_shade_ids"):  # absent from older builds selected with RT2025_LIB for A/B runs
+            L.rt_camera_rays_ids.argtypes = [C.POINTER(rt_camera), C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p]
+            L.rt_camera_rays_ids_device.argtypes = [C.POINTER(rt_camera), C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+            L.rt_world_hit_ids.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double, C.c_uint64,
+                                           C.c_uint32, C.c_void_p, C.POINTER(rt_stats)]
+            L.rt_world_hit_ids_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, C.c_double,
+                                                  C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+            L.rt_shade_ids.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
+                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
+            L.rt_shade_ids_device.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(rt_stats)]
         L.rt_render.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
                                 C.POINTER(rt_stats)]
         L.rt_render_device.argtypes = [C.c_void_p, C.POINTER(rt_camera), C.POINTER(rt_render_opts), C.c_void_p,
@@ -563,6 +578,59 @@ class Scene:
                                       d_state_ptr, stream, C.byref(st)), self.L)
         return st
 
+    def world_hit_ids(self, rays, ids, t_min=1e-8, t_max=float("inf"), seed=0, flags=0):
+        """rt_world_hit_ids: world_hit with the draws of ray i addressed by ids[i] (rt_path_id_dtype: pixel, sample, segment) instead
+        of (i, 0, segment).  Returns (rt_hit_record_dtype array, stats)."""
+        rays = np.ascontiguousarray(rays, dtype=rt_ray_dtype)
+        ids = np.ascontiguousarray(ids, dtype=rt_path_id_dtype)
+        if ids.shape != (len(rays),):
+            raise ValueError(f"ids has shape {ids.shape}; {len(rays)} path ids expected")
+        out = np.empty(len(rays), dtype=rt_hit_record_dtype)
+        per_ray = None
+        if np.ndim(t_max) != 0:
+            per_ray = np.ascontiguousarray(t_max, dtype=np.float64)
+            if per_ray.shape != (len(rays),):
+                raise ValueError(f"t_max has shape {per_ray.shape}; a scalar or {len(rays)} values expected")
+            t_max = float("inf")
+        st = rt_stats()
+        _check(self.L.rt_world_hit_ids(self.h, rays.ctypes.data, ids.ctypes.data, None if per_ray is None else per_ray.ctypes.data, len(rays),
+                                       t_min, t_max, seed, flags, out.ctypes.data, C.byref(st)), self.L)
+        return out, st
+
+    def world_hit_ids_device(self, d_rays_ptr, d_ids_ptr, n, d_out_ptr, d_t_max_ptr=None, t_min=1e-8, t_max=float("inf"), seed=0, flags=0,
+                             stream=None):
+        """rt_world_hit_ids_device: the same on device buffers (n rays, n 16-byte path ids, n records out)."""
+        st = rt_stats()
+        _check(self.L.rt_world_hit_ids_device(self.h, d_rays_ptr, d_ids_ptr, d_t_max_ptr, n, t_min, t_max, seed, flags, d_out_ptr, stream,
+                                              C.byref(st)), self.L)
+        return st
+
+    def shade_ids(self, records, ids, rays, beta, radiance, state, seed=0, camera=None, flags=0):
+        """rt_shade_ids: shade with the draws and the segment of row i taken from ids[i] (rt_path_id_dtype).  Updates ids in place
+        with rays, beta, radiance and state: the rows that go on get ids["segment"] + 1.  radiance is still per row.  Returns the
+        stats."""
+        cam = camera if camera is not None else self.host.camera
+        records = np.ascontiguousarray(records, dtype=rt_hit_record_dtype)
+        n = len(records)
+        for name, a, dt, shape in (("ids", ids, rt_path_id_dtype, (n,)), ("rays", rays, rt_ray_dtype, (n,)), ("beta", beta, np.float64, (n, 3)),
+                                   ("radiance", radiance, np.float64, (n, 3)), ("state", state, np.uint8, (n,))):
+            if not (isinstance(a, np.ndarray) and a.dtype == dt and a.shape == shape and a.flags.c_contiguous and a.flags.writeable):
+                raise ValueError(f"{name}: a writeable C-contiguous {np.dtype(dt)} array of shape {shape} is updated in place")
+        st = rt_stats()
+        _check(self.L.rt_shade_ids(self.h, C.byref(cam), records.ctypes.data, ids.ctypes.data, n, seed, flags, rays.ctypes.data,
+                                   beta.ctypes.data, radiance.ctypes.data, state.ctypes.data, C.byref(st)), self.L)
+        return st
+
+    def shade_ids_device(self, d_records_ptr, d_ids_ptr, n, d_rays_ptr, d_beta_ptr, d_radiance_ptr, d_state_ptr, seed=0, camera=None, flags=0,
+                         stream=None):
+        """rt_shade_ids_device: the same on device buffers (n records, n path ids, n rays, n x 3 beta and radiance doubles, n state
+        bytes)."""
+        cam = camera if camera is not None else self.host.camera
+        st = rt_stats()
+        _check(self.L.rt_shade_ids_device(self.h, C.byref(cam), d_records_ptr, d_ids_ptr, n, seed, flags, d_rays_ptr, d_beta_ptr,
+                                          d_radiance_ptr, d_state_ptr, stream, C.byref(st)), self.L)
+        return st
+
     def render_opts(self, seed=1, accum_type=RT_ACCUM_F64, part_index=0, part_count=1, sample_begin=0, sample_end=0,
                     flags=0, max_paths_in_flight=0, no_binning=False, classic_media_order=False):
         o = rt_render_opts()
@@ -640,6 +708,21 @@ def camera_rays_device(camera, seed, sample, d_out_ptr, stream=None):
     """rt_camera_rays_device: the same into image_width * image_height rays at d_out_ptr on the current device."""
     L = product_lib()
     _check(L.rt_camera_rays_device(C.byref(camera), seed, sample, d_out_ptr, stream), L)
+
+
+def camera_rays_ids(camera, seed, ids):
+    """rt_camera_rays_ids: out[i] = Camera::get_ray of pixel ids[i]["pixel"] (j * image_width + i) and stratum ids[i]["sample"]."""
+    L = product_lib()
+    ids = np.ascontiguousarray(ids, dtype=rt_path_id_dtype)
+    out = np.empty(len(ids), dtype=rt_ray_dtype)
+    _check(L.rt_camera_rays_ids(C.byref(camera), seed, ids.ctypes.data, len(ids), out.ctypes.data), L)
+    return out
+
+
+def camera_rays_ids_device(camera, seed, d_ids_ptr, n, d_out_ptr, stream=None):
+    """rt_camera_rays_ids_device: the same from n path ids at d_ids_ptr into n rays at d_out_ptr on the current device."""
+    L = product_lib()
+    _check(L.rt_camera_rays_ids_device(C.byref(camera), seed, d_ids_ptr, n, d_out_ptr, stream), L)
 
 
 def tonemap_device(d_accum_ptr, n_pixels, d_rgb_ptr, toon_map=0, accum_type=RT_ACCUM_F32, stream=None):

@@ -116,6 +116,8 @@ pub struct rt_hit_record {
     pub t: f64, pub p: [f64; 3], pub normal: [f64; 3], pub u: f64, pub v: f64,
     pub kind: u32, pub front_face: u32, pub prim_id: u32, pub inst_id: u32, pub material: u32, pub reserved: u32,
 }
+#[repr(C)] #[derive(Clone, Copy, Default)]
+pub struct rt_path_id { pub pixel: u32, pub sample: u32, pub segment: u32, pub reserved: u32 }
 #[repr(C)] pub struct rt_scene { _private: [u8; 0] }
 
 extern "C" {
@@ -132,6 +134,12 @@ extern "C" {
     pub fn rt_shade_device(scene: *const rt_scene, cam: *const rt_camera, d_records: *const rt_hit_record, n: u64, seed: u64, segment: u32, flags: u32, d_rays: *mut rt_ray, d_beta: *mut f64, d_radiance: *mut f64, d_state: *mut u8, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_camera_rays(cam: *const rt_camera, seed: u64, sample: u32, out: *mut rt_ray) -> i32;
     pub fn rt_camera_rays_device(cam: *const rt_camera, seed: u64, sample: u32, d_out: *mut rt_ray, stream: *mut c_void) -> i32;
+    pub fn rt_camera_rays_ids(cam: *const rt_camera, seed: u64, ids: *const rt_path_id, n: u64, out: *mut rt_ray) -> i32;
+    pub fn rt_camera_rays_ids_device(cam: *const rt_camera, seed: u64, d_ids: *const rt_path_id, n: u64, d_out: *mut rt_ray, stream: *mut c_void) -> i32;
+    pub fn rt_world_hit_ids(scene: *const rt_scene, rays: *const rt_ray, ids: *const rt_path_id, t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, seed: u64, flags: u32, out: *mut rt_hit_record, stats: *mut rt_stats) -> i32;
+    pub fn rt_world_hit_ids_device(scene: *const rt_scene, d_rays: *const rt_ray, d_ids: *const rt_path_id, d_t_max_per_ray: *const f64, n: u64, t_min: f64, t_max: f64, seed: u64, flags: u32, d_out: *mut rt_hit_record, stream: *mut c_void, stats: *mut rt_stats) -> i32;
+    pub fn rt_shade_ids(scene: *const rt_scene, cam: *const rt_camera, records: *const rt_hit_record, ids: *mut rt_path_id, n: u64, seed: u64, flags: u32, rays: *mut rt_ray, beta: *mut f64, radiance: *mut f64, state: *mut u8, stats: *mut rt_stats) -> i32;
+    pub fn rt_shade_ids_device(scene: *const rt_scene, cam: *const rt_camera, d_records: *const rt_hit_record, d_ids: *mut rt_path_id, n: u64, seed: u64, flags: u32, d_rays: *mut rt_ray, d_beta: *mut f64, d_radiance: *mut f64, d_state: *mut u8, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, accum: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_device(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, d_accum: *mut c_void, stream: *mut c_void, stats: *mut rt_stats) -> i32;
     pub fn rt_render_rgb8(scene: *const rt_scene, cam: *const rt_camera, opts: *const rt_render_opts, rgb: *mut u8, stats: *mut rt_stats) -> i32;
